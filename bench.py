@@ -24,6 +24,13 @@ N > 1 (torchrun): weak scaling by sample range — every rank sweeps its own
 max all-reduce over the [channels x angles] peak table.
 
 `--impl reference` runs only the reference CPU arm with the same JSON shape.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller -
+the combined peak table of phaserot_peaks, [channels x 180 * subsample] float32:
+index 0 the raw input peak, index i the peak at i / subsample degrees - as
+DIR/peaks.npy.  The inputs are generated from fixed seeds, so two builds run
+with the same arguments can be compared table for table.  Only the GPU arm has
+this output.
 """
 import argparse
 import ctypes
@@ -532,10 +539,11 @@ class SweepBench:
         w0 = time.perf_counter()
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         self.barrier()
         w = time.perf_counter() - w0
+        self.last_output = out
         ms = e0.elapsed_time(e1)
         # the table read-back is a host sync inside the step; wall and event time agree, keep the larger
         t = torch.tensor([max(ms / 1e3, w if wall else 0.0)], device=self.dev, dtype=torch.float64)
@@ -630,6 +638,18 @@ class SweepBench:
         del self.x
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, peaks):
+    """The table the last timed step returned to its caller (phaserot_peaks), as out_dir/peaks.npy."""
+    peaks = np.asarray(peaks, np.float32)
+    if peaks.nbytes > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: the table's {peaks.nbytes} bytes exceed {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "peaks.npy"), peaks)
+
+
 def shard_range(capi, wl, total_frames, rank, world, local):
     """Frames [f0, f1) of rank `rank` when one stream of total_frames is cut on the FFT segment grid."""
     with capi.Phaserot(mode=capi.MODE_CLI, n_channels=wl["C"], blksiz=wl["blksiz"], subsample=wl["S"], device=local) as h:
@@ -716,6 +736,8 @@ def gpu_main(args):
     A = sb.A
     sampler = ClockSampler(local) if rank == 0 else None
     t_dev, st, clocks = sb.run_device(args.steps, args.warmup, sampler, args.wall)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sb.last_output)
     launches = torch.tensor([st["kernel_launches"]], device=dev, dtype=torch.int64)
     if world > 1:
         dist.all_reduce(launches)
@@ -939,7 +961,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the render / plugin / true-peak secondary legs")
     ap.add_argument("--wall", action="store_true", help="use max(wall, events) as the step time")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="GPU arm only: write the peak table of the last timed step as DIR/peaks.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.impl == "reference":
         # under torchrun only rank 0 works; the other ranks exit quietly
         if int(os.environ.get("RANK", "0")) != 0:

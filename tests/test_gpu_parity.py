@@ -568,12 +568,15 @@ def test_lv2_plugin_binary_through_host_harness(golden):
     for inplace in (False, True):
         y, lat, _ = O.lv2_render(so, x, 48000, 256, ang[:, None], inplace=inplace)
         assert np.max(np.abs(y[0] - g["r48000_b256_y"])) <= AUDIO_TOL * float(np.abs(g["r48000_b256_y"]).max())
-    if O.have_ref():  # live comparison against the reference binary on a long noise render (config 2 style, shortened)
-        xm = O.pink_noise(48000 * 5, 42)
-        ncalls = (len(xm) + 1023) // 1024
-        a90 = np.full((ncalls, 1), 90.0, np.float32)
+    # a long noise render (config 2 style, shortened, last call partial) against the oracle's plugin loop
+    xm = O.pink_noise(48000 * 5, 42)
+    ncalls = (len(xm) + 1023) // 1024
+    a90 = np.full((ncalls, 1), 90.0, np.float32)
+    yg, _, _ = O.lv2_render(so, xm, 48000, 1024, a90)
+    yo = O.oracle_plugin_run(xm, 48000, 1024, a90[:, 0].copy())
+    assert np.max(np.abs(yg[0] - yo)) <= AUDIO_TOL * float(np.abs(yo).max())
+    if O.have_ref():  # and against the reference binary itself, where it is built
         yr, _, _ = O.lv2_render(os.path.join(O.REF_DIR, "phaserotate_ref.so"), xm, 48000, 1024, a90)
-        yg, _, _ = O.lv2_render(so, xm, 48000, 1024, a90)
         assert np.max(np.abs(yg - yr)) <= AUDIO_TOL * float(np.abs(yr).max())
 
 
@@ -594,9 +597,40 @@ def test_cli_search_output_matches_reference_text(golden, tmp_path):
         r = _cli(*argv, wav)
         assert r.returncode == 0, r.stderr
         assert r.stdout == str(g[key]), key
+    # verbose tables (-vv): every peak printed is the oracle's at the printed angle, within print precision
+    our = _cli("-vv", "-s", "12", wav)
+    assert our.returncode == 0, our.stderr
+    blk = [int(l.split()[-1]) for l in our.stderr.splitlines() if l.startswith("Process block-size")]
+    assert len(blk) == 1, our.stderr
+    po = O.oracle_analyze(g["x"], blk[0])
+
+    def db(p):
+        return 20.0 * np.log10(p) if p >= 1e-15 else -np.inf
+
+    rows = 0
+    for line in our.stdout.splitlines():
+        if line.startswith("#"):
+            continue
+        tok = [float(t) for t in line.split()]
+        a = int(round(tok[0] * 2)) % 360
+        chans = tok[2:]
+        assert len(chans) == po.shape[0], line
+        for c, v in enumerate(chans):
+            if v != -np.inf:     # -inf: a channel the refine pass leaves out (mask)
+                assert abs(v - db(po[c, a])) <= 2e-4, (line, c)
+        if -np.inf not in chans:
+            assert abs(tok[1] - db(po[:, a].max())) <= 2e-4, line
+        rows += 1
+    assert rows >= 30 + 2 * 13, our.stdout    # coarse table (every 6 deg) and at least two refine windows
+    considered = 0
+    for line in our.stderr.splitlines():
+        if line.startswith("Consider min:"):  # "Consider min: p (< thr) chn: c @ deg deg", c counted from 0
+            p, c, deg = float(line.split()[2]), int(line.split("chn:")[1].split()[0]), float(line.split("@")[1].split()[0])
+            assert abs(p - po[c, int(round(deg * 2)) % 360]) <= 1e-5 * p + 1e-6, line
+            considered += 1
+    assert considered >= 2
     if O.have_ref():  # verbose tables: same lines, numbers within print precision
         ref = subprocess.run([os.path.join(O.REF_DIR, "phase-rotate"), "-vv", "-s", "12", wav], capture_output=True, text=True)
-        our = _cli("-vv", "-s", "12", wav)
         assert our.stderr == ref.stderr
         assert len(our.stdout.splitlines()) == len(ref.stdout.splitlines())
         for a, b in zip(our.stdout.splitlines(), ref.stdout.splitlines()):
