@@ -217,6 +217,51 @@ PHASEROT_API int phaserot_sweep_shard (phaserot_t* h, const void* data, int form
 
 PHASEROT_API uint32_t phaserot_shard_align (const phaserot_t* h);
 
+/* ---- per-section analysis and render ------------------------------------ */
+
+/* Extends phaserot_sweep() / phaserot_sweep_pcm() (one analyze_file() pass, cli:565-587) with one min-peak
+ * table per section of the stream, for material whose best angle changes along the file (an album or a
+ * mix as one file, a broadcast, a film stem).  Same arguments, first-block and flush rules as
+ * phaserot_sweep(); `data` is host memory in `format` = PHASEROT_PCM_*.  The stream is cut into sections
+ * of section_frames frames, a positive multiple of phaserot_shard_align(h); the last section is the
+ * remainder and the zero flush block belongs to it: ceil(n_frames / section_frames) sections.
+ * The table of section k equals, bit for bit, the table phaserot_sweep_shard_device() gives for frames
+ * [k S, (k+1) S) with the blksiz frames before them as history, first = (k == 0), last = (k == last
+ * section); the element-wise max over the sections is the table of phaserot_sweep() bit for bit.  Grid
+ * index 0 is the raw input peak of the section (cli:413-414).
+ * One FFT pass over the whole stream, whose rows are (section, channel) pairs, each with its own filter
+ * radius and survivor list: the launches do not grow with the number of sections.  A section whose list
+ * overflows (few-tone material) is repeated through the shard path with dense mode
+ * (phaserot_stats_t.dense_repeats counts these repeats).
+ * At most 65535 (section, channel) rows per call (one hour of 48 kHz stereo in sections down to 0.11 s);
+ * more is PHASEROT_E_INVAL with a phaserot_last_error() text, as is a section length off the alignment.
+ * The handle's own peak table is not touched; every call starts from zeros.  Synchronous.
+ * PHASEROT_E_STATE for plugin handles, PHASEROT_E_UNSUPPORTED for true-peak handles (oversample > 1). */
+PHASEROT_API int phaserot_sweep_sections (phaserot_t* h, const void* data, int format, uint64_t n_frames, uint64_t section_frames,
+                                          int ang_start, int ang_end, int ang_stride, int chn);
+/* The same over audio resident in device memory (interleaved float32). */
+PHASEROT_API int phaserot_sweep_sections_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, uint64_t section_frames,
+                                                 int ang_start, int ang_end, int ang_stride, int chn);
+/* Tables of the last sections sweep: out[n_sections][n_channels][180 * subsample] (NULL: only
+ * *n_sections is returned; 0 before the first sections sweep).  Extends phaserot_peaks(). */
+PHASEROT_API int phaserot_section_peaks (phaserot_t* h, int* n_sections, float* out);
+
+/* Extends phaserot_render() / phaserot_render_device() (PhaseRotate::apply over the stream, cli:467-485)
+ * with one angle per section and channel: angles[k * n_channels + c], in grid steps on the FULL circle
+ * (a + 2 * 180 * subsample renders the same output as a; a + 180 * subsample renders its negation).
+ * Unlike phaserot_render(), the angles are not wrapped (cli:463).  Output sample t of section k is
+ * rendered at angle a[k][c], except the first blksiz frames of every section k > 0, where the angle moves
+ * linearly from a[k-1][c] to a[k][c]: at sample j of that ramp the angle is
+ *     phi = a[k-1] + (a[k] - a[k-1]) * (j + 1) / blksiz grid steps
+ * and (sa, ca) = sincos of phi times the SinCosLut constant (cli:41-72).  Outside the ramps every sample
+ * equals phaserot_render() at that section's angle bit for bit.  Sections are those of
+ * phaserot_sweep_sections() (same section_frames rule and row limit); flush_blocks and the output layout
+ * are those of phaserot_render(); the apply() stream state is not changed.  Synchronous. */
+PHASEROT_API int phaserot_render_sections (phaserot_t* h, const float* interleaved, uint64_t n_frames, uint64_t section_frames,
+                                           const int* angles, int flush_blocks, float* out);
+PHASEROT_API int phaserot_render_sections_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, uint64_t section_frames,
+                                                  const int* angles, int flush_blocks, float* d_out);
+
 /* ---- several GPUs in one process ---------------------------------------- */
 
 /* A group of handles, one per device, that analyses ONE stream: the file is cut

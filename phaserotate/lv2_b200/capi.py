@@ -26,6 +26,8 @@ SYMBOLS = [
     "phaserot_process", "phaserot_process_levels", "phaserot_latency",
     "phaserot_sweep_shard_device", "phaserot_sweep_shard", "phaserot_shard_align", "phaserot_plugin_angle",
     "phaserot_sweep_shard_boot_device", "phaserot_sweep_shard_resume",
+    "phaserot_sweep_sections", "phaserot_sweep_sections_device", "phaserot_section_peaks",
+    "phaserot_render_sections", "phaserot_render_sections_device",
     "phaserot_group_create", "phaserot_group_destroy", "phaserot_group_size", "phaserot_group_handle", "phaserot_group_sweep",
     "phaserot_group_peaks", "phaserot_group_reset", "phaserot_pending_table", "phaserot_set_profiling", "phaserot_get_kernel_times",
     "phaserot_sync", "phaserot_get_stats", "phaserot_reset_stats",
@@ -103,6 +105,11 @@ def load():
     lib.phaserot_plugin_angle.argtypes = [vp, vp]
     lib.phaserot_sweep_shard_boot_device.argtypes = [vp, vp, C.c_uint64, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
     lib.phaserot_sweep_shard_resume.argtypes = [vp]
+    lib.phaserot_sweep_sections.argtypes = [vp, vp, C.c_int, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.phaserot_sweep_sections_device.argtypes = [vp, vp, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.phaserot_section_peaks.argtypes = [vp, C.POINTER(C.c_int), vp]
+    lib.phaserot_render_sections.argtypes = [vp, vp, C.c_uint64, C.c_uint64, vp, C.c_int, vp]
+    lib.phaserot_render_sections_device.argtypes = [vp, vp, C.c_uint64, C.c_uint64, vp, C.c_int, vp]
     lib.phaserot_group_create.argtypes = [C.POINTER(vp), C.POINTER(Cfg), vp, C.c_int]
     lib.phaserot_group_destroy.argtypes = [vp]
     lib.phaserot_group_destroy.restype = None
@@ -302,6 +309,47 @@ class Phaserot:
 
     def sync(self):
         self._ck(self._lib.phaserot_sync(self._h), "phaserot_sync")
+
+    # -- per-section analysis and render ------------------------------------
+    def sweep_sections(self, x, section_frames, ang_start=0, ang_end=None, stride=1, chn=-1):
+        """x: host array [frames, channels] of float32, int16 or int32 (PCM_S32), or packed 24-bit uint8 bytes."""
+        if ang_end is None:
+            ang_end = self.maxsample
+        x = np.ascontiguousarray(x)
+        fmt = {np.dtype(np.float32): PCM_F32, np.dtype(np.int16): PCM_S16, np.dtype(np.int32): PCM_S32, np.dtype(np.uint8): PCM_S24}[x.dtype]
+        n = x.size // self.n_channels // (3 if fmt == PCM_S24 else 1)
+        self._ck(self._lib.phaserot_sweep_sections(self._h, _ptr(x), fmt, n, section_frames, ang_start, ang_end, stride, chn),
+                 "phaserot_sweep_sections")
+
+    def sweep_sections_device(self, dev_ptr, n_frames, section_frames, ang_start=0, ang_end=None, stride=1, chn=-1):
+        if ang_end is None:
+            ang_end = self.maxsample
+        self._ck(self._lib.phaserot_sweep_sections_device(self._h, C.c_void_p(dev_ptr), n_frames, section_frames, ang_start, ang_end, stride, chn),
+                 "phaserot_sweep_sections_device")
+
+    def section_peaks(self):
+        """Tables of the last sections sweep: [n_sections, channels, 180 * subsample]."""
+        n = C.c_int()
+        self._ck(self._lib.phaserot_section_peaks(self._h, C.byref(n), None), "phaserot_section_peaks")
+        out = np.zeros((n.value, self.n_channels, self.maxsample), np.float32)
+        self._ck(self._lib.phaserot_section_peaks(self._h, C.byref(n), _ptr(out)), "phaserot_section_peaks")
+        return out
+
+    def render_sections(self, x, section_frames, angles, flush_blocks=1):
+        """angles: [n_sections, channels] grid steps on the full circle."""
+        x = np.ascontiguousarray(x, np.float32).reshape(-1, self.n_channels)
+        n = x.shape[0]
+        nblk = (n + self.blksiz - 1) // self.blksiz + flush_blocks
+        out = np.zeros((nblk * self.blksiz, self.n_channels), np.float32)
+        ang = np.ascontiguousarray(angles, np.int32)
+        self._ck(self._lib.phaserot_render_sections(self._h, _ptr(x), n, section_frames, _ptr(ang), flush_blocks, _ptr(out)),
+                 "phaserot_render_sections")
+        return out
+
+    def render_sections_device(self, d_in, n_frames, section_frames, angles, flush_blocks, d_out):
+        ang = np.ascontiguousarray(angles, np.int32)
+        self._ck(self._lib.phaserot_render_sections_device(self._h, C.c_void_p(d_in), n_frames, section_frames, _ptr(ang), flush_blocks,
+                                                           C.c_void_p(d_out)), "phaserot_render_sections_device")
 
     # -- CLI render --------------------------------------------------------
     def apply(self, buf, angles):

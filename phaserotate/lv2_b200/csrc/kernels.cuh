@@ -42,7 +42,12 @@ constexpr int kTidOff    = kXchFloats + 4 + kRedFloats;               // lane id
 constexpr int kSmemBytes = kM * (int)sizeof (float2) + (kTidOff + 48) * (int)sizeof (float);
 static_assert (kSmemBytes + 1024 <= 132 * 1024, "fftconv_kernel must fit the 132 KB carve-out");
 
-enum { EPI_POINTS = 0, EPI_RENDER = 1, EPI_HILBERT = 2 };
+// EPI_SECT_*: the same epilogues with rows by section (phaserot_sweep_sections, phaserot_render_sections):
+// the row of a segment is section * nchan + channel, see ConvParams::sect_segs
+enum { EPI_POINTS = 0, EPI_RENDER = 1, EPI_HILBERT = 2, EPI_SECT_POINTS = 3, EPI_SECT_RENDER = 4 };
+__host__ __device__ constexpr bool epi_points (int e) { return e == EPI_POINTS || e == EPI_SECT_POINTS; }
+__host__ __device__ constexpr bool epi_render (int e) { return e == EPI_RENDER || e == EPI_SECT_RENDER; }
+__host__ __device__ constexpr bool epi_sect (int e) { return e == EPI_SECT_POINTS || e == EPI_SECT_RENDER; }
 
 enum { SRC_PLANE = 0, SRC_INTER = 1 };
 
@@ -102,6 +107,16 @@ struct ConvParams {
 	long long     out_frames;
 	int           out_compact;  // EPI_HILBERT: segment j of the launch writes its V outputs at out[8 + j V ..) (true-peak staging)
 	int           prefetch;     // > 0: L2 prefetch distance in segments (experiments; 0 = off, the default)
+	// EPI_SECT_*: segment seg lies in section min (seg / sect_segs, n_sect - 1) (sections start on segment
+	// boundaries; the last one takes the remainder); thr2, list, count, overflow, rawpeak and r2max are
+	// indexed by row = section * nchan + (channel - chan0) instead of by channel
+	long long     sect_segs;
+	int           n_sect;
+	int           sect_boot;    // EPI_SECT_POINTS bootstrap launch: segment si of the launch samples section si / sect_boot
+	const float2* sect_cs;      // EPI_SECT_RENDER: [n_sect][C] steady-state (ca, sa)
+	const int*    sect_ang;     // EPI_SECT_RENDER: [n_sect][C] angles in grid steps; the first hist_frames samples of a
+	                            // section k > 0 ramp linearly from the angle of section k - 1
+	float         ang_mp;       // EPI_SECT_RENDER: radians per grid step (the SinCosLut constant)
 };
 
 // Segment input loaders: z[n0 + idx] for the first forward pass and the direct
@@ -253,7 +268,20 @@ struct EpiCtx {
 	int       c, i_hi, i_skip, i_zero;
 	long long mbase, obase; // complex stream index / output index of local index 0
 	float     rawmax;
+	int       row;          // EPI_SECT_*: row of the segment
+	long long t_sect;       // EPI_SECT_RENDER: first output sample of the segment's section
 };
+
+// (ca, sa) of sample j of the ramp into the section of row `row` (EPI_SECT_RENDER):
+// phi = a[k-1] + (a[k] - a[k-1]) (j + 1) / L grid steps
+__device__ __forceinline__ float2 sect_ramp_cs (const ConvParams& p, int row, long long j)
+{
+	const int   a0  = p.sect_ang[row - p.nchan], a1 = p.sect_ang[row];
+	const float phi = (float)a0 + (float)(a1 - a0) * (float)(j + 1) / (float)p.hist_frames;
+	float       s, c;
+	sincosf (phi * p.ang_mp, &s, &c);
+	return make_float2 (c, s);
+}
 
 // Epilogue straight from the registers of the last inverse pass: thread e holds
 // the outputs w[k] of local index i = e + 512 k; valid ones have i in [Lh, i_hi),
@@ -366,9 +394,11 @@ __device__ __forceinline__ void epilogue (const float2 (&w)[32], float* xch, uin
 	const int dl    = p.dl;
 	const int warp  = tid >> 5;
 	const int xbase = warp ? (warp - 1) * 32 : 15 * 32 - 1;
-	if (EPI == EPI_POINTS) {
-		float          thr2   = xch[kXchFloats + 4 + kRedThr]; // parked in shared memory by the kernel prologue
-		const ListDst  dst    = { p.list + (long long)cx.c * p.list_stride, p.count + cx.c, p.list_cap, p.overflow };
+	if (epi_points (EPI)) {
+		// (sections: the radius, list and flags of the segment's row)
+		const int      row    = epi_sect (EPI) ? cx.row : cx.c;
+		float          thr2   = epi_sect (EPI) ? __ldg (p.thr2 + row) : xch[kXchFloats + 4 + kRedThr]; // parked in shared memory by the kernel prologue
+		const ListDst  dst    = { p.list + (long long)row * p.list_stride, p.count + row, p.list_cap, epi_sect (EPI) ? p.overflow + row : p.overflow };
 		const unsigned lt     = lanemask_lt ();
 		float          rawmax = cx.rawmax;
 		if (p.boot_beta > 0.f) {
@@ -388,7 +418,7 @@ __device__ __forceinline__ void epilogue (const float2 (&w)[32], float* xch, uin
 			if (tid == 0) {
 				float m = red[0];
 				for (int i = 1; i < kConvThreads / 32; ++i) m = fmaxf (m, red[i]);
-				const unsigned old = atomicMax (p.r2max + cx.c, __float_as_uint (m));
+				const unsigned old = atomicMax (p.r2max + row, __float_as_uint (m));
 				red[kConvThreads / 32] = fmaxf (m, __uint_as_float (old));
 			}
 			__syncthreads ();
@@ -437,7 +467,7 @@ __device__ __forceinline__ void epilogue (const float2 (&w)[32], float* xch, uin
 		cx.rawmax = rawmax;
 	} else {
 		float2*      outc = p.out + (cx.obase + (long long)cx.c * p.out_stride);
-		const float2 cs   = (EPI == EPI_RENDER) ? p.cs[cx.c] : make_float2 (0.f, 1.f);
+		const float2 cs   = (EPI == EPI_RENDER) ? p.cs[cx.c] : (EPI == EPI_SECT_RENDER) ? p.sect_cs[cx.row] : make_float2 (0.f, 1.f);
 		const int    rlen = (EPI == EPI_RENDER && p.ramp_len) ? p.ramp_len[cx.c] : 0;
 #pragma unroll
 		for (int kb = 0; kb < 32; kb += 4) {
@@ -450,7 +480,7 @@ __device__ __forceinline__ void epilogue (const float2 (&w)[32], float* xch, uin
 				ok[kk]      = i >= p.Lh && i < cx.i_hi;
 				zd[kk]      = make_float2 (0.f, 0.f);
 			}
-			if (EPI == EPI_RENDER) load_direct (zd, ok, tid, kb, dl, tb, ld);
+			if (epi_render (EPI)) load_direct (zd, ok, tid, kb, dl, tb, ld);
 #pragma unroll
 			for (int kk = 0; kk < 4; ++kk) {
 				const int k  = kb + kk;
@@ -461,8 +491,12 @@ __device__ __forceinline__ void epilogue (const float2 (&w)[32], float* xch, uin
 					float2          y  = make_float2 (pv, w[k].x);
 					const long long t0 = 2 * (cx.mbase + i);
 					if (EPI == EPI_HILBERT) cx.rawmax = fmaxf (cx.rawmax, fmaxf (fabsf (pv), fabsf (w[k].x))); // bootstrap gate of the true-peak sweep
-					if (EPI == EPI_RENDER) {
+					if (epi_render (EPI)) {
 						float2 cs0 = cs, cs1 = cs;
+						if (EPI == EPI_SECT_RENDER && cx.t_sect > 0 && t0 - cx.t_sect < p.hist_frames) { // ramp (rare: sincosf per sample)
+							cs0 = sect_ramp_cs (p, cx.row, t0 - cx.t_sect);
+							if (t0 + 1 - cx.t_sect < p.hist_frames) cs1 = sect_ramp_cs (p, cx.row, t0 + 1 - cx.t_sect);
+						}
 						if (t0 < rlen) {
 							const float2* r = p.ramp + (long long)cx.c * p.ramp_stride + t0;
 							cs0             = r[0];
@@ -472,7 +506,7 @@ __device__ __forceinline__ void epilogue (const float2 (&w)[32], float* xch, uin
 						y.x = __fadd_rn (__fmul_rn (cs0.x, zd[kk].x), __fmul_rn (cs0.y, pv));
 						y.y = __fadd_rn (__fmul_rn (cs1.x, zd[kk].y), __fmul_rn (cs1.y, w[k].x));
 					}
-					if (EPI == EPI_RENDER && p.out_inter) {
+					if (epi_render (EPI) && p.out_inter) {
 						// straight into the interleaved frames (plain stores: the CTAs of the
 						// other channels fill the rest of each sector side by side, L2 merges them)
 						float* o = p.out_inter + t0 * p.C + cx.c;
@@ -554,6 +588,23 @@ __device__ __noinline__ void spectrum_only (float2* sm, const float* xch, const 
 // channels of one stretch of interleaved input run at the same time and share
 // it through L2.  NP = number of tap partitions (2 only for FIR length 32768).
 // ---------------------------------------------------------------------------
+__device__ __forceinline__ void flush_rawmax (unsigned* dst, float r, int lane)
+{
+	for (int o = 16; o; o >>= 1) r = fmaxf (r, __shfl_xor_sync (0xffffffffu, r, o));
+	if (lane == 0) atomicMax (dst, __float_as_uint (r));
+}
+
+// Bootstrap wave of a sections sweep: segment si of the launch samples section k = si / sect_boot; the
+// sect_boot samples of a section are spread over it, each at a pseudo-random offset inside its share.
+__device__ __forceinline__ long long sect_boot_seg (const ConvParams& p, int si)
+{
+	const long long k    = si / p.sect_boot, j = si % p.sect_boot;
+	const long long nall = (p.m_end + p.V - 1) / p.V;
+	const long long n    = k == p.n_sect - 1 ? nall - k * p.sect_segs : p.sect_segs; // the last section takes the remainder
+	const long long w    = max (1LL, n / p.sect_boot);
+	return k * p.sect_segs + min (n - 1, j * n / p.sect_boot + (long long)(((unsigned)si * 2654435761u >> 8) % (unsigned)w));
+}
+
 template <int EPI, int SRC, int NP>
 __global__ void __launch_bounds__ (kConvThreads, 1) fftconv_kernel (const ConvParams p)
 {
@@ -620,9 +671,22 @@ __global__ void __launch_bounds__ (kConvThreads, 1) fftconv_kernel (const ConvPa
 	const int s_begin = jb * run, s_end = min ((int)p.nseg, s_begin + run);
 	const int c = p.chan0 + ci;
 	bool prev_inside = false;
+	cx.row = -1;
 	for (int si = s_begin; si < s_end; ++si) {
 
-		const long long seg = p.seg0 + si * p.seg_stride + (p.seg_jitter ? (long long)(((unsigned)si * 2654435761u >> 8) % (unsigned)p.seg_stride) : 0);
+		long long seg = p.seg0 + si * p.seg_stride + (p.seg_jitter ? (long long)(((unsigned)si * 2654435761u >> 8) % (unsigned)p.seg_stride) : 0);
+		if (EPI == EPI_SECT_POINTS && p.sect_boot) seg = sect_boot_seg (p, si);
+		if (epi_sect (EPI)) {
+			const long long k   = min (seg / p.sect_segs, (long long)p.n_sect - 1);
+			const int       row = (int)k * p.nchan + ci;
+			if (EPI == EPI_SECT_POINTS && row != cx.row && cx.row >= 0) {
+				// a run crossing a section boundary: the raw peak so far belongs to the previous row
+				flush_rawmax (p.rawpeak + cx.row, cx.rawmax, lane);
+				cx.rawmax = 0.f;
+			}
+			cx.row    = row;
+			cx.t_sect = k * p.sect_segs * 2 * p.V;
+		}
 		const long long n0  = seg * p.V - p.Lh; // complex stream index of local index 0
 		if (NP == 2 && (si == s_begin || p.seg_stride != 1)) {
 			// the scratch does not hold the spectrum of segment seg - 1 yet
@@ -680,6 +744,7 @@ __global__ void __launch_bounds__ (kConvThreads, 1) fftconv_kernel (const ConvPa
 		for (int o = 16; o; o >>= 1) r = fmaxf (r, __shfl_xor_sync (0xffffffffu, r, o));
 		if (lane == 0) atomicMax (p.rawpeak + c, __float_as_uint (r));
 	}
+	if (EPI == EPI_SECT_POINTS && s_begin < s_end) flush_rawmax (p.rawpeak + cx.row, cx.rawmax, lane);
 	if (EPI == EPI_HILBERT && p.r2max && s_begin < s_end) {
 		// largest H^2 of the launch: truepeak_kernel gates its bootstrap wave on it
 		float r = cx.rawmax;

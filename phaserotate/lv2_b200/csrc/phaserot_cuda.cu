@@ -225,6 +225,16 @@ struct phaserot {
 	PinBuf h_stage[2], h_res, h_io, h_cs;
 	long long plane_stride = 0, out_stride = 0, list_stride = 0;
 
+	// per-section analysis (phaserot_sweep_sections): device table [rows][A] | raw peaks [rows], row = section * (c1 - c0) + c - c0;
+	// d_sect_aux: evaluated points (u64) | thr2 [rows] | count [rows] | overflow flags [rows] | bootstrap flags [rows] | r2max [rows]
+	DevBuf                 d_sect, d_sect_aux, d_sect_rt;
+	long long              sect_n = 0;
+	int                    sect_A = 0, sect_c0 = 0, sect_c1 = 0;
+	bool                   sect_raw = false;
+	std::vector<int>       sect_idx;
+	std::vector<long long> sect_redo_k; // sections whose list overflowed: their tables come from the shard path
+	std::vector<float>     sect_redo;   // [redone section][C][MS]
+
 	// pending (asynchronous) sweep result
 	bool             pending = false;
 	std::vector<int> pend_idx;
@@ -451,7 +461,7 @@ launch_conv_np (phaserot* h, const ConvParams& p)
 		return PHASEROT_OK;
 	}
 	const int grid = (int)std::min<long long> (total, h->n_sm);
-	ProfScope ps (h, EPI == EPI_POINTS ? 0 : EPI == EPI_HILBERT ? 6 : 3);
+	ProfScope ps (h, epi_points (EPI) ? 0 : EPI == EPI_HILBERT ? 6 : 3);
 	fftconv_kernel<EPI, SRC, NP><<<grid, kConvThreads, kSmemBytes, h->stream>>> (p);
 	CK (cudaGetLastError ());
 	++h->stats.kernel_launches;
@@ -737,6 +747,82 @@ angle_schedule (phaserot* h, int ang_start, int ang_end, int ang_stride, std::ve
 		if (angle >= ang_end) {
 			break;
 		}
+	}
+	return PHASEROT_OK;
+}
+
+// H2D of a host stream into d_inter (allocated by the caller) in chunks on the copy stream, integer PCM
+// widened there; the compute stream waits for each chunk, and `landed (frames)` runs after every chunk
+// but the last, so that the caller can start on the frames that have landed.
+template <class Landed>
+int
+upload_chunks (phaserot* h, const void* src, int pcm_bytes, long long n_frames, Landed&& landed)
+{
+	int rc = PHASEROT_OK;
+	const long long chunk_frames = std::max<long long> (4, ((8LL << 20) / h->C) & ~3LL); // ~32 MB of floats per chunk; a multiple of 4 frames keeps every chunk 4-byte aligned at 3 bytes per sample
+	const size_t    bps          = pcm_bytes ? (size_t)pcm_bytes : sizeof (float);      // bytes per sample on the host side
+	cudaPointerAttributes at;
+	const bool pinned = (cudaPointerGetAttributes (&at, src) == cudaSuccess) && (at.type == cudaMemoryTypeHost);
+	cudaGetLastError ();
+	if (!pinned) {
+		for (int b = 0; b < 2; ++b) {
+			rc = h->h_stage[b].ensure (bps * (size_t)std::min (chunk_frames, std::max<long long> (n_frames, 4)) * h->C); // short files: small staging (pinned allocation costs ~0.3 ms per MB)
+			if (rc) return rc;
+		}
+	}
+	if (pcm_bytes) {
+		// integer PCM: raw chunk -> device staging -> pcm_to_float_kernel on the copy
+		// stream -> the float copy of the file; staging buffer b is reused two chunks
+		// later on the same stream, i.e. after the kernel that read it
+		for (int b = 0; b < 2; ++b) {
+			rc = h->d_stage[b].ensure (bps * (size_t)std::min (chunk_frames, std::max<long long> (n_frames, 4)) * h->C);
+			if (rc) return rc;
+		}
+	}
+	// the previous pass may still be reading d_inter on the compute stream
+	CK (cudaEventRecord (h->ev_done[0], h->stream));
+	CK (cudaStreamWaitEvent (h->copy_stream, h->ev_done[0], 0));
+	int       b  = 0;
+	long long f0 = 0;
+	bool      used[2] = { false, false };
+	while (f0 < n_frames) {
+		const long long nf    = std::min (chunk_frames, n_frames - f0);
+		const size_t    bytes = bps * (size_t)nf * h->C;
+		const void*     hsrc  = (const char*)src + bps * (size_t)f0 * h->C;
+		if (!pinned) {
+			if (used[b]) {
+				CK (cudaEventSynchronize (h->ev_copy[b])); // staging buffer free again
+			}
+			memcpy (h->h_stage[b].p, hsrc, bytes);
+			hsrc = h->h_stage[b].p;
+		}
+		float* d_chunk = (float*)h->d_inter.p + (size_t)f0 * h->C;
+		if (pcm_bytes) {
+			CK (cudaMemcpyAsync (h->d_stage[b].p, hsrc, bytes, cudaMemcpyHostToDevice, h->copy_stream));
+			const long long ns = nf * h->C;
+			const unsigned  nb = (unsigned)((ns + 1023) / 1024);
+			if (pcm_bytes == 2) {
+				pcm_to_float_kernel<int16_t><<<nb, 256, 0, h->copy_stream>>> ((const int16_t*)h->d_stage[b].p, d_chunk, ns);
+			} else if (pcm_bytes == 3) {
+				pcm24_to_float_kernel<<<nb, 256, 0, h->copy_stream>>> ((const uint8_t*)h->d_stage[b].p, d_chunk, ns);
+			} else {
+				pcm_to_float_kernel<int32_t><<<nb, 256, 0, h->copy_stream>>> ((const int32_t*)h->d_stage[b].p, d_chunk, ns);
+			}
+			CK (cudaGetLastError ());
+			++h->stats.kernel_launches;
+		} else {
+			CK (cudaMemcpyAsync (d_chunk, hsrc, bytes, cudaMemcpyHostToDevice, h->copy_stream));
+		}
+		CK (cudaEventRecord (h->ev_copy[b], h->copy_stream));
+		CK (cudaStreamWaitEvent (h->stream, h->ev_copy[b], 0));
+		h->stats.h2d_bytes += bytes;
+		used[b] = true;
+		f0 += nf;
+		if (f0 < n_frames) {
+			rc = landed (f0);
+			if (rc) return rc;
+		}
+		b ^= 1;
 	}
 	return PHASEROT_OK;
 }
@@ -1164,72 +1250,11 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		p.inter = (const float*)h->d_inter.p;
 		rc      = tp_head ();
 		if (rc) return rc;
-		const long long chunk_frames = std::max<long long> (4, ((8LL << 20) / h->C) & ~3LL); // ~32 MB of floats per chunk; a multiple of 4 frames keeps every chunk 4-byte aligned at 3 bytes per sample
-		const size_t    bps          = pcm_bytes ? (size_t)pcm_bytes : sizeof (float);      // bytes per sample on the host side
-		cudaPointerAttributes at;
-		const bool pinned = (cudaPointerGetAttributes (&at, src) == cudaSuccess) && (at.type == cudaMemoryTypeHost);
-		cudaGetLastError ();
-		if (!pinned) {
-			for (int b = 0; b < 2; ++b) {
-				rc = h->h_stage[b].ensure (bps * (size_t)std::min (chunk_frames, std::max<long long> (n_frames, 4)) * h->C); // short files: small staging (pinned allocation costs ~0.3 ms per MB)
-				if (rc) return rc;
-			}
-		}
-		if (pcm_bytes) {
-			// integer PCM: raw chunk -> device staging -> pcm_to_float_kernel on the copy
-			// stream -> the float copy of the file; staging buffer b is reused two chunks
-			// later on the same stream, i.e. after the kernel that read it
-			for (int b = 0; b < 2; ++b) {
-				rc = h->d_stage[b].ensure (bps * (size_t)std::min (chunk_frames, std::max<long long> (n_frames, 4)) * h->C);
-				if (rc) return rc;
-			}
-		}
-		// the previous pass may still be reading d_inter on the compute stream
-		CK (cudaEventRecord (h->ev_done[0], h->stream));
-		CK (cudaStreamWaitEvent (h->copy_stream, h->ev_done[0], 0));
-		int       b  = 0;
-		long long f0 = 0;
-		bool      used[2] = { false, false };
-		while (f0 < n_frames) {
-			const long long nf    = std::min (chunk_frames, n_frames - f0);
-			const size_t    bytes = bps * (size_t)nf * h->C;
-			const void*     hsrc  = (const char*)src + bps * (size_t)f0 * h->C;
-			if (!pinned) {
-				if (used[b]) {
-					CK (cudaEventSynchronize (h->ev_copy[b])); // staging buffer free again
-				}
-				memcpy (h->h_stage[b].p, hsrc, bytes);
-				hsrc = h->h_stage[b].p;
-			}
-			float* d_chunk = (float*)h->d_inter.p + (size_t)f0 * h->C;
-			if (pcm_bytes) {
-				CK (cudaMemcpyAsync (h->d_stage[b].p, hsrc, bytes, cudaMemcpyHostToDevice, h->copy_stream));
-				const long long ns = nf * h->C;
-				const unsigned  nb = (unsigned)((ns + 1023) / 1024);
-				if (pcm_bytes == 2) {
-					pcm_to_float_kernel<int16_t><<<nb, 256, 0, h->copy_stream>>> ((const int16_t*)h->d_stage[b].p, d_chunk, ns);
-				} else if (pcm_bytes == 3) {
-					pcm24_to_float_kernel<<<nb, 256, 0, h->copy_stream>>> ((const uint8_t*)h->d_stage[b].p, d_chunk, ns);
-				} else {
-					pcm_to_float_kernel<int32_t><<<nb, 256, 0, h->copy_stream>>> ((const int32_t*)h->d_stage[b].p, d_chunk, ns);
-				}
-				CK (cudaGetLastError ());
-				++h->stats.kernel_launches;
-			} else {
-				CK (cudaMemcpyAsync (d_chunk, hsrc, bytes, cudaMemcpyHostToDevice, h->copy_stream));
-			}
-			CK (cudaEventRecord (h->ev_copy[b], h->copy_stream));
-			CK (cudaStreamWaitEvent (h->stream, h->ev_copy[b], 0));
-			h->stats.h2d_bytes += bytes;
-			used[b] = true;
-			f0 += nf;
-			frames_ready = f0;
-			if (f0 < n_frames) {
-				rc = process_ready (false);
-				if (rc) return rc;
-			}
-			b ^= 1;
-		}
+		rc = upload_chunks (h, src, pcm_bytes, n_frames, [&] (long long f) {
+			frames_ready = f;
+			return process_ready (false);
+		});
+		if (rc) return rc;
 		rc = process_ready (true);
 		if (rc) return rc;
 	}
@@ -1251,6 +1276,325 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		h->redo.chn         = chn;
 	}
 	h->pending = true;
+	return PHASEROT_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Per-section analysis: the rows of the sweep are (section, channel) pairs.
+// ---------------------------------------------------------------------------
+
+// sweep_kernel walks the rows with grid.z: at most 65535 (section, channel) rows per call,
+// e.g. one hour of 48 kHz stereo in 0.11 s sections or of 8 channels in 0.44 s sections
+constexpr long long kMaxSectionRows = 65535;
+
+// The section instantiations are loaded on first use only, like the kernels of set_device_attrs().
+int
+ensure_sect_attrs (phaserot* h)
+{
+	std::lock_guard<std::mutex> lk (g_create_lock);
+	static std::vector<int>     done;
+	if (done.size () <= (size_t)h->dev) done.resize ((size_t)h->dev + 1, 0);
+	if (done[(size_t)h->dev] & h->NP) return PHASEROT_OK;
+	int rc;
+	if (h->NP == 2) {
+		if ((rc = set_conv_attr<EPI_SECT_POINTS, SRC_INTER, 2> ())) return rc;
+		if ((rc = set_conv_attr<EPI_SECT_RENDER, SRC_INTER, 2> ())) return rc;
+	} else {
+		if ((rc = set_conv_attr<EPI_SECT_POINTS, SRC_INTER, 1> ())) return rc;
+		if ((rc = set_conv_attr<EPI_SECT_RENDER, SRC_INTER, 1> ())) return rc;
+	}
+	done[(size_t)h->dev] |= h->NP;
+	return PHASEROT_OK;
+}
+
+int
+check_sections (phaserot* h, long long n_frames, long long S, int nchan, long long* n_sect)
+{
+	const long long align = (long long)phaserot_shard_align (h);
+	if (n_frames <= 0 || S <= 0 || S % align) {
+		snprintf (g_last_error, sizeof (g_last_error), "section length %lld is not a positive multiple of %lld frames", S, align);
+		return PHASEROT_E_INVAL;
+	}
+	*n_sect = (n_frames + S - 1) / S;
+	if (*n_sect * nchan > kMaxSectionRows) {
+		snprintf (g_last_error, sizeof (g_last_error), "%lld sections x %d channels exceed the limit of %lld section rows", *n_sect, nchan, kMaxSectionRows);
+		return PHASEROT_E_INVAL;
+	}
+	return PHASEROT_OK;
+}
+
+/*
+ * One analysis pass over a whole stream (the arguments of phaserot_sweep) with a table per section of
+ * S frames.  The FFT pass is the one of sweep_core - the same continuous input and segment grid - and
+ * only the epilogue's destination follows the section (EPI_SECT_POINTS): every row has its own filter
+ * radius, survivor list and table.  Normal mode only: a row whose list overflows is flagged, and its
+ * section is repeated afterwards through sweep_core as a shard with history (which has dense mode).
+ * Synchronous.
+ */
+int
+sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt, long long n_frames, long long S, int ang_start, int ang_end,
+                     int ang_stride, int chn)
+{
+	const int pcm_bytes = fmt == PHASEROT_PCM_S16 ? 2 : fmt == PHASEROT_PCM_S32 ? 4 : fmt == PHASEROT_PCM_S24 ? 3 : 0;
+	if (chn >= h->C) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->OS > 1) {
+		return PHASEROT_E_UNSUPPORTED;
+	}
+	const int c0    = chn < 0 ? 0 : chn;
+	const int c1    = chn < 0 ? h->C : chn + 1;
+	const int nchan = c1 - c0;
+	long long n_sect;
+	int       rc = check_sections (h, n_frames, S, nchan, &n_sect);
+	if (rc) return rc;
+	std::vector<int> idx;
+	bool             raw = false;
+	rc                   = angle_schedule (h, ang_start, ang_end, ang_stride, idx, raw);
+	if (rc) return rc;
+	rc = finish_pending (h); // a pending sweep of the handle's own table completes first
+	if (rc) return rc;
+	rc = ensure_sect_attrs (h);
+	if (rc) return rc;
+	h->sect_n = 0;
+	h->sect_redo_k.clear ();
+	h->sect_redo.clear ();
+
+	const int       A     = (int)idx.size ();
+	const long long R     = n_sect * nchan;
+	const long long B     = (n_frames + h->L - 1) / h->L;
+	const long long t_end = (B + 1) * h->L; // B blocks + the zero flush block, like phaserot_sweep
+	const long long m_end = (t_end + 1) / 2;
+	const long long nseg  = (m_end + h->V - 1) / h->V;
+	const long long sps   = S / (2 * (long long)h->V); // segments per section
+	const long long last_segs = nseg - (n_sect - 1) * sps;
+
+	// survivor lists, pooled: 1/32 of the points of a row (the largest one: the last section takes the remainder
+	// and the flush block), at least 8 K points.  Rows only ever receive points of their own section, so a row's
+	// list needs nothing like the 1 M floor of a whole channel.
+	const long long cap = std::max<long long> (8192, 2 * (long long)h->V * std::max (sps, last_segs) / 32);
+	rc = h->d_list.ensure ((size_t)(R * cap) * sizeof (float2));
+	if (rc) return rc;
+	rc = h->d_sect.ensure (sizeof (unsigned) * (size_t)(R * std::max (A, 1) + R));
+	if (rc) return rc;
+	rc = h->d_sect_aux.ensure (sizeof (unsigned long long) + sizeof (unsigned) * 5 * (size_t)R);
+	if (rc) return rc;
+	unsigned*           table = (unsigned*)h->d_sect.p;
+	unsigned*           rawpk = table + (size_t)R * A;
+	unsigned long long* n_ev  = (unsigned long long*)h->d_sect_aux.p;
+	float*              thr2  = (float*)(n_ev + 1);
+	unsigned*           count = (unsigned*)(thr2 + R);
+	unsigned*           ovf   = count + R;
+	unsigned*           ovf_b = ovf + R;
+	unsigned*           r2max = ovf_b + R;
+	CK (cudaMemsetAsync (h->d_sect.p, 0, sizeof (unsigned) * (size_t)(R * std::max (A, 1) + R), h->stream));
+	CK (cudaMemsetAsync (h->d_sect_aux.p, 0, sizeof (unsigned long long) + sizeof (unsigned) * 5 * (size_t)R, h->stream));
+	if (A > 0) {
+		rc = h->d_cs.ensure (sizeof (float2) * (size_t)A);
+		if (rc) return rc;
+		rc = h->h_cs.ensure (sizeof (float2) * (size_t)A);
+		if (rc) return rc;
+		float2* cs = (float2*)h->h_cs.p;
+		for (int k = 0; k < A; ++k) cs[k] = make_float2 (h->lut_c[(size_t)idx[(size_t)k]], h->lut_s[(size_t)idx[(size_t)k]]);
+		CK (cudaMemcpyAsync (h->d_cs.p, cs, sizeof (float2) * (size_t)A, cudaMemcpyHostToDevice, h->stream));
+	}
+
+	const float* d_src = src;
+	if (!src_is_device) {
+		// the bootstrap wave samples every section, so the pass starts once the whole stream has landed
+		rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)n_frames * h->C, 16));
+		if (rc) return rc;
+		rc = upload_chunks (h, src, pcm_bytes, n_frames, [] (long long) { return PHASEROT_OK; });
+		if (rc) return rc;
+		d_src = (const float*)h->d_inter.p;
+	}
+
+	const bool no_prune = (h->cfg.flags & PHASEROT_FLAG_NO_PRUNE) != 0;
+	const int  thr_mode = A == 0 ? 2 : no_prune ? 0 : 1;
+	ConvParams p;
+	fill_conv_common (h, p);
+	p.inter       = d_src;
+	p.n_frames    = n_frames;
+	p.C           = h->C;
+	p.chan0       = c0;
+	p.nchan       = nchan;
+	p.m_end       = m_end;
+	p.m_skip      = !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK) ? h->Lh / 2 : 0;
+	p.m_zero      = !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK) ? h->Lh : 0;
+	p.list        = (float2*)h->d_list.p;
+	p.list_stride = cap;
+	p.list_cap    = (unsigned)cap;
+	p.count       = count;
+	p.thr2        = thr2;
+	p.rawpeak     = rawpk;
+	p.r2max       = r2max;
+	p.sect_segs   = sps;
+	p.n_sect      = (int)n_sect;
+
+	// new radius of every row from its running peaks; zeroes the list counters
+	auto thresholds = [&] () -> int {
+		ProfScope ps (h, 5);
+		threshold_kernel<<<(unsigned)R, 256, 0, h->stream>>> (table, A, A, 0, thr2, count, 1, thr_mode);
+		CK (cudaGetLastError ());
+		++h->stats.kernel_launches;
+		return PHASEROT_OK;
+	};
+	auto sweep = [&] (bool boot) -> int {
+		if (A == 0) return PHASEROT_OK;
+		const SweepCfg sc = pick_sweep_cfg (A);
+		const int      gx = std::max<long long> (1, (h->n_sm * 8) / std::max<long long> (1, sc.gy * R));
+		const dim3     grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)R);
+		const float2*  lst = (const float2*)h->d_list.p;
+		const float2*  cs  = (const float2*)h->d_cs.p;
+		const int      so  = boot ? 0 : 1; // a flagged row is redone: do not brute-force its full list
+		ProfScope      ps (h, 1);
+		switch (sc.R) {
+			case 1: sweep_kernel<1><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
+			case 2: sweep_kernel<2><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
+			case 4: sweep_kernel<4><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
+			default: sweep_kernel<8><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
+		}
+		CK (cudaGetLastError ());
+		++h->stats.kernel_launches;
+		return PHASEROT_OK;
+	};
+	auto conv = [&] () -> int { return h->NP == 2 ? launch_conv_np<EPI_SECT_POINTS, SRC_INTER, 2> (h, p) : launch_conv_np<EPI_SECT_POINTS, SRC_INTER, 1> (h, p); };
+
+	if (thr_mode == 1) {
+		// Bootstrap: a quarter of the segments of every section (at least one; more when there are fewer
+		// sections than a wave has segments), gated like sweep_core's wave on the largest radius the row
+		// has seen.  A whole-stream sweep refreshes its radius between launches; a row is usually done
+		// within one contiguous launch, so its radius has to be close to final before it starts (one
+		// segment per 10 s section left 40 % of the programme's samples on the lists).  Any subset is
+		// valid: the contiguous passes visit these segments again.
+		const long long wave = std::max<long long> (1, (h->n_sm + nchan - 1) / nchan);
+		rc = thresholds ();
+		if (rc) return rc;
+		p.sect_boot  = (int)std::min<long long> (std::max ((wave + n_sect - 1) / n_sect, (sps + 3) / 4), sps);
+		p.seg0       = 0;
+		p.seg_stride = 2; // sparse: no stash reuse between consecutive segments of a CTA
+		p.nseg       = n_sect * p.sect_boot;
+		p.boot_beta  = kBootBeta;
+		p.overflow   = ovf_b; // nobody reads it
+		rc = conv ();
+		if (rc) return rc;
+		rc = sweep (true);
+		if (rc) return rc;
+	}
+	// contiguous launches sized like sweep_core's device-resident ones (8 segments per CTA, then 16 x that)
+	p.sect_boot  = 0;
+	p.seg_stride = 1;
+	p.boot_beta  = 0.f;
+	p.overflow   = ovf;
+	const long long segs_first = std::max<long long> (1, ((long long)h->n_sm * 8) / nchan);
+	long long       seg_done   = 0;
+	for (int n_main = 0; seg_done < nseg; ++n_main) {
+		const bool      short_rest = nseg - seg_done <= 2 * segs_first;
+		const long long n          = std::min ((n_main == 0 && !short_rest) ? segs_first : 16 * segs_first, nseg - seg_done);
+		rc = thresholds ();
+		if (rc) return rc;
+		p.seg0 = seg_done;
+		p.nseg = n;
+		rc = conv ();
+		if (rc) return rc;
+		rc = sweep (false);
+		if (rc) return rc;
+		seg_done += n;
+	}
+
+	// flagged rows -> sections to repeat
+	std::vector<unsigned> flags ((size_t)R);
+	unsigned long long    evaluated = 0;
+	CK (cudaMemcpyAsync (flags.data (), ovf, sizeof (unsigned) * (size_t)R, cudaMemcpyDeviceToHost, h->stream));
+	CK (cudaMemcpyAsync (&evaluated, n_ev, sizeof (evaluated), cudaMemcpyDeviceToHost, h->stream));
+	CK (cudaStreamSynchronize (h->stream));
+	prof_resolve (h);
+	h->stats.points_total += (uint64_t)nchan * (uint64_t)(2 * (m_end - p.m_skip));
+	h->stats.points_evaluated += evaluated;
+	h->sect_n   = n_sect;
+	h->sect_A   = A;
+	h->sect_c0  = c0;
+	h->sect_c1  = c1;
+	h->sect_raw = raw;
+	h->sect_idx = idx;
+	for (long long k = 0; k < n_sect; ++k) {
+		bool any = false;
+		for (int ci = 0; ci < nchan; ++ci) any = any || flags[(size_t)(k * nchan + ci)] != 0;
+		if (!any) continue;
+		// The shard path with history, in dense mode from the start (its launches are sized to the list), on a
+		// zeroed handle table; the handle's own table and mode are restored afterwards.
+		const std::vector<float> keep  = h->table;
+		const bool               dense = h->dense_mode;
+		std::fill (h->table.begin (), h->table.end (), 0.f);
+		h->dense_mode       = true;
+		const long long f0  = k * S;
+		const long long F   = std::min (S, n_frames - f0);
+		const long long Bk  = (F + h->L - 1) / h->L;
+		const bool      lst = k == n_sect - 1;
+		rc = sweep_core (h, d_src + (size_t)f0 * h->C, true, F, lst ? (Bk + 1) * h->L : F, k == 0, k ? d_src + (size_t)(f0 - h->L) * h->C : nullptr, ang_start, ang_end,
+		                 ang_stride, chn);
+		if (!rc) rc = finish_pending (h);
+		if (!rc) {
+			h->sect_redo_k.push_back (k);
+			h->sect_redo.insert (h->sect_redo.end (), h->table.begin (), h->table.end ());
+			++h->stats.dense_repeats;
+		}
+		h->table      = keep;
+		h->dense_mode = dense;
+		if (rc) {
+			h->sect_n = 0;
+			return rc;
+		}
+	}
+	return PHASEROT_OK;
+}
+
+/*
+ * Render with one angle per (section, channel): the fused CLI render of render_core (interleaved in,
+ * interleaved out, t_end frames) with EPI_SECT_RENDER, which forms (ca, sa) per sample from the
+ * [n_sect][C] angle table.  angles: host [n_sect][C], full circle.
+ */
+int
+render_sections_core (phaserot* h, const float* d_src, long long n_frames, long long t_end, long long S, long long n_sect, const int* angles, float* d_dst)
+{
+	int rc = ensure_sect_attrs (h);
+	if (rc) return rc;
+	const size_t        nrow = (size_t)(n_sect * h->C);
+	std::vector<float2> cs (nrow);
+	for (size_t r = 0; r < nrow; ++r) {
+		// a + MS renders the negation of a: LUT pair of a mod MS, negated for odd half turns
+		const long long a  = angles[r];
+		const long long q  = (a >= 0 ? a : a - h->MS + 1) / h->MS;
+		const size_t    i  = (size_t)(a - q * h->MS);
+		const float     sg = (q & 1) ? -1.f : 1.f;
+		cs[r]              = make_float2 (sg * h->lut_c[i], sg * h->lut_s[i]);
+	}
+	rc = h->d_sect_rt.ensure ((sizeof (float2) + sizeof (int)) * nrow);
+	if (rc) return rc;
+	float2* d_cs  = (float2*)h->d_sect_rt.p;
+	int*    d_ang = (int*)(d_cs + nrow);
+	CK (cudaMemcpyAsync (d_cs, cs.data (), sizeof (float2) * nrow, cudaMemcpyHostToDevice, h->stream));
+	CK (cudaMemcpyAsync (d_ang, angles, sizeof (int) * nrow, cudaMemcpyHostToDevice, h->stream));
+	ConvParams p;
+	fill_conv_common (h, p);
+	p.chan0      = 0;
+	p.nchan      = h->C;
+	p.seg0       = 0;
+	p.m_end      = (t_end + 1) / 2;
+	p.nseg       = (p.m_end + h->V - 1) / h->V;
+	p.inter      = d_src;
+	p.n_frames   = n_frames;
+	p.C          = h->C;
+	p.out_inter  = d_dst;
+	p.out_frames = t_end;
+	p.sect_segs  = S / (2 * (long long)h->V);
+	p.n_sect     = (int)n_sect;
+	p.sect_cs    = d_cs;
+	p.sect_ang   = d_ang;
+	p.ang_mp     = (float)(2.f * M_PI / h->S / -360.0); // build_lut()
+	rc = h->NP == 2 ? launch_conv_np<EPI_SECT_RENDER, SRC_INTER, 2> (h, p) : launch_conv_np<EPI_SECT_RENDER, SRC_INTER, 1> (h, p);
+	if (rc) return rc;
+	CK (cudaStreamSynchronize (h->stream)); // the host tables above are about to go
 	return PHASEROT_OK;
 }
 
@@ -1653,7 +1997,8 @@ phaserot_destroy (phaserot_t* h)
 	if (h->own_stream) cudaStreamSynchronize (h->own_stream);
 	if (h->copy_stream) cudaStreamSynchronize (h->copy_stream);
 	for (DevBuf* b : { &h->d_G, &h->d_G1, &h->d_scratch, &h->d_tw, &h->d_g, &h->d_plane, &h->d_out, &h->d_list, &h->d_stage[0], &h->d_stage[1], &h->d_io, &h->d_inter, &h->d_hist, &h->d_small,
-	                   &h->d_cs, &h->d_peaks, &h->d_ramp, &h->d_chancs, &h->d_tpH, &h->d_ring, &h->d_slot, &h->d_sec, &h->d_wide }) {
+	                   &h->d_cs, &h->d_peaks, &h->d_ramp, &h->d_chancs, &h->d_tpH, &h->d_ring, &h->d_slot, &h->d_sec, &h->d_wide,
+	                   &h->d_sect, &h->d_sect_aux, &h->d_sect_rt }) {
 		b->release ();
 	}
 	for (PinBuf* b : { &h->h_stage[0], &h->h_stage[1], &h->h_res, &h->h_io, &h->h_cs, &h->h_slot }) {
@@ -2079,6 +2424,127 @@ int
 phaserot_render_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, const int* angles, int flush_blocks, float* d_out)
 {
 	return render_bulk (h, d_interleaved, true, n_frames, angles, flush_blocks, d_out, true);
+}
+
+int
+phaserot_sweep_sections (phaserot_t* h, const void* data, int format, uint64_t n_frames, uint64_t section_frames, int ang_start, int ang_end, int ang_stride,
+                         int chn)
+{
+	if (!h || (!data && n_frames) || format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->plugin) {
+		return PHASEROT_E_STATE;
+	}
+	DevGuard guard (h->dev);
+	return sweep_sections_core (h, (const float*)data, false, format, (long long)n_frames, (long long)section_frames, ang_start, ang_end, ang_stride, chn);
+}
+
+int
+phaserot_sweep_sections_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, uint64_t section_frames, int ang_start, int ang_end,
+                                int ang_stride, int chn)
+{
+	if (!h || (!d_interleaved && n_frames)) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->plugin) {
+		return PHASEROT_E_STATE;
+	}
+	DevGuard guard (h->dev);
+	return sweep_sections_core (h, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, (long long)section_frames, ang_start, ang_end, ang_stride, chn);
+}
+
+int
+phaserot_section_peaks (phaserot_t* h, int* n_sections, float* out)
+{
+	if (!h || !n_sections) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->plugin) {
+		return PHASEROT_E_STATE;
+	}
+	*n_sections = (int)h->sect_n;
+	if (!out || h->sect_n == 0) {
+		return PHASEROT_OK;
+	}
+	DevGuard            guard (h->dev);
+	const int           A = h->sect_A, nchan = h->sect_c1 - h->sect_c0;
+	const size_t        R = (size_t)h->sect_n * nchan;
+	std::vector<float>  res (R * A + R);
+	CK (cudaMemcpyAsync (res.data (), h->d_sect.p, sizeof (float) * res.size (), cudaMemcpyDeviceToHost, h->stream));
+	CK (cudaStreamSynchronize (h->stream));
+	h->stats.d2h_bytes += sizeof (float) * res.size ();
+	const size_t per = (size_t)h->C * h->MS;
+	std::fill (out, out + (size_t)h->sect_n * per, 0.f);
+	for (size_t r = 0; r < R; ++r) {
+		// the same merge as finish_pending(): grid index 0 holds the raw peak unless the angle set maps onto it too
+		float* row = out + (r / nchan) * per + (size_t)(h->sect_c0 + (int)(r % nchan)) * h->MS;
+		for (int k = 0; k < A; ++k) {
+			const int a = h->sect_idx[(size_t)k];
+			row[a]      = std::max (row[a], res[r * A + (size_t)k]);
+		}
+		if (h->sect_raw) row[0] = std::max (row[0], res[R * A + r]);
+	}
+	for (size_t i = 0; i < h->sect_redo_k.size (); ++i) {
+		memcpy (out + (size_t)h->sect_redo_k[i] * per, h->sect_redo.data () + i * per, sizeof (float) * per);
+	}
+	return PHASEROT_OK;
+}
+
+static int
+render_sections_bulk (phaserot* h, const float* src, bool dev_in, uint64_t n_frames, uint64_t section_frames, const int* angles, int flush_blocks, float* dst,
+                      bool dev_out)
+{
+	if (!h || (!src && n_frames) || !angles || !dst || flush_blocks < 0) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->plugin) {
+		return PHASEROT_E_STATE;
+	}
+	DevGuard        guard (h->dev);
+	const long long F = (long long)n_frames;
+	long long       n_sect;
+	int             rc = check_sections (h, F, (long long)section_frames, h->C, &n_sect);
+	if (rc) return rc;
+	const long long B     = (F + h->L - 1) / h->L;
+	const long long t_end = (B + flush_blocks) * h->L;
+	const size_t    bytes = sizeof (float) * (size_t)t_end * h->C;
+	const float*    d_src = src;
+	if (!dev_in) {
+		const size_t in_bytes = sizeof (float) * (size_t)F * h->C;
+		rc                    = h->d_io.ensure (in_bytes);
+		if (rc) return rc;
+		CK (cudaMemcpyAsync (h->d_io.p, src, in_bytes, cudaMemcpyHostToDevice, h->stream));
+		h->stats.h2d_bytes += in_bytes;
+		d_src = (const float*)h->d_io.p;
+	}
+	float* d_dst = dst;
+	if (!dev_out) {
+		rc = h->d_stage[0].ensure (bytes);
+		if (rc) return rc;
+		d_dst = (float*)h->d_stage[0].p;
+	}
+	rc = render_sections_core (h, d_src, F, t_end, (long long)section_frames, n_sect, angles, d_dst);
+	if (rc) return rc;
+	if (!dev_out) {
+		CK (cudaMemcpyAsync (dst, d_dst, bytes, cudaMemcpyDeviceToHost, h->stream));
+		CK (cudaStreamSynchronize (h->stream));
+		h->stats.d2h_bytes += bytes;
+	}
+	return PHASEROT_OK;
+}
+
+int
+phaserot_render_sections (phaserot_t* h, const float* interleaved, uint64_t n_frames, uint64_t section_frames, const int* angles, int flush_blocks, float* out)
+{
+	return render_sections_bulk (h, interleaved, false, n_frames, section_frames, angles, flush_blocks, out, false);
+}
+
+int
+phaserot_render_sections_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, uint64_t section_frames, const int* angles, int flush_blocks,
+                                 float* d_out)
+{
+	return render_sections_bulk (h, d_interleaved, true, n_frames, section_frames, angles, flush_blocks, d_out, true);
 }
 
 uint32_t

@@ -62,6 +62,7 @@ struct Options {
 	int          subsample   = 2;     // --subsample N: 1/N degree grid (BASELINE configs 3 and 5 use 10 and 100)
 	int          gpus        = 1;     // --gpus N: sample-range shards over N devices (0 = all)
 	bool         fixed_write = false; // --fixed-write: write loop without the reference's two quirks (cli:985, cli:973)
+	double       sections    = 0;     // --sections SECONDS: one angle per section of the file (0 = one for the whole file)
 };
 
 // PHASEROT_CLI_TIMING=1: wall-clock breakdown of the process on stderr (file read, CUDA
@@ -172,6 +173,7 @@ parse_options (int argc, char** argv)
 		{ "subsample", required_argument, 0, 1001 },
 		{ "gpus", required_argument, 0, 1002 },
 		{ "fixed-write", no_argument, 0, 1003 },
+		{ "sections", required_argument, 0, 1004 },
 		{ 0, 0, 0, 0 },
 	};
 	int c;
@@ -209,8 +211,19 @@ parse_options (int argc, char** argv)
 				}
 				break;
 			case 1003: o.fixed_write = true; break;
+			case 1004: {
+				char* ep    = nullptr;
+				o.sections = strtod (optarg, &ep);
+				if (*ep != '\0' || !(o.sections > 0) || !std::isfinite (o.sections)) {
+					die ("Error: --sections takes a section length in seconds > 0.\n");
+				}
+				break;
+			}
 			default: die ("Error: unrecognized option. See --help for usage information.\n");
 		}
+	}
+	if (o.sections > 0 && (o.angles_arg || o.oversample || o.gpus != 1)) {
+		die ("Error: --sections cannot be combined with -a, --true-peak or --gpus.\n");
 	}
 	kSubsample = o.subsample;
 	kMaxSample = 180 * kSubsample;
@@ -329,6 +342,152 @@ struct PeakTable {
 		return mask[(size_t)c] ? one (c, a) : 0.f;
 	}
 };
+
+// Angle search on one peak table: the coarse pass over every `stride`-th angle, then the refine pass
+// around its local minima, replayed on the table (cli:815-929).  angle[c] is what the reference applies
+// (channels without a minimum: 0, p_min = +inf).
+struct MinResult {
+	std::vector<int>   angle;
+	std::vector<float> p_min, r_zro, r_min;
+};
+
+MinResult
+find_min_angles (const PeakTable& tab, const Options& opt, FILE* vfd)
+{
+const int               C      = tab.channels;
+const int               stride = opt.stride;
+const std::vector<bool> all ((size_t)C, true);
+
+	if (opt.verbose > 1) { // gnuplot table of the coarse pass (cli:800-813)
+		printf ("# Angle mono-peak");
+		for (int c = 0; c < C; ++c) {
+			printf (" chn-%d", c + 1);
+		}
+		printf ("\n");
+		for (int a = 0; a < kMaxSample; a += stride) {
+			printf ("%.2f %.4f", a / (float)kSubsample, to_dB (tab.peak (-1, a, all)));
+			for (int c = 0; c < C; ++c) {
+				printf (" %.4f", to_dB (tab.peak (c, a, all)));
+			}
+			printf ("\n");
+		}
+	}
+
+	const float inf = std::numeric_limits<float>::infinity ();
+	std::map<int, std::vector<int>> mins; // coarse angle -> channels to refine there
+	std::vector<int>   min_angle ((size_t)C, 0);
+	// The reference leaves p_min / min_angle uninitialised for a channel whose
+	// coarse peaks are all equal (cli:835-839); +inf / 0 is the evident intent.
+	std::vector<float> p_min ((size_t)C, inf), r_zro ((size_t)C, 0.f), r_min ((size_t)C, 0.f);
+
+	for (int c = 0; c < C; ++c) {
+		const int pc   = opt.link ? -1 : c;
+		float     cmin = inf, cmax = 0;
+		r_zro[(size_t)c] = tab.peak (c, 0, all);
+		for (int a = 0; a < kMaxSample; a += stride) {
+			cmin = std::min (cmin, tab.peak (pc, a, all));
+			cmax = std::max (cmax, tab.peak (pc, a, all));
+		}
+		float range = cmax - cmin;
+		if (range == 0) {
+			mins[0].push_back (c);
+			continue;
+		}
+		if (stride > 1) {
+			range *= .07;
+			p_min[(size_t)c] = inf;
+		} else {
+			range            = 0;
+			p_min[(size_t)c] = cmin;
+		}
+		for (int a = 0; a < kMaxSample; a += stride) {
+			const float p = tab.peak (pc, a, all);
+			if (p <= cmin + range) {
+				mins[a].push_back (c);
+				if (opt.verbose > 1) {
+					fprintf (vfd, "Consider min: %f (< %f) chn: %d @ %.2f deg\n", p, cmin + range, c, a / (float)kSubsample);
+				}
+			}
+		}
+	}
+
+	if (stride == 1) {
+		for (auto& mp : mins) { // ascending: the largest angle wins (cli:859-865)
+			for (int cn : mp.second) {
+				min_angle[(size_t)cn] = mp.first;
+				r_min[(size_t)cn]     = tab.peak (cn, mp.first, all);
+			}
+		}
+	} else {
+		const int s2 = (stride + 1) / 2;
+		for (auto& mp : mins) {
+			// which channels the reference's refine pass analyses (cli:880)
+			std::vector<bool> mask ((size_t)C, mp.second.size () > 1);
+			if (mp.second.size () == 1) {
+				mask[(size_t)mp.second.front ()] = true;
+			}
+			const int ma = mp.first;
+			for (int cn : mp.second) {
+				for (int a = ma - s2; a < ma + s2 + 1; ++a) {
+					const float p = tab.peak (opt.link ? -1 : cn, a, mask);
+					if (p <= p_min[(size_t)cn]) { // ties: the later angle wins (cli:885)
+						p_min[(size_t)cn]     = p;
+						r_min[(size_t)cn]     = tab.peak (cn, a, mask);
+						min_angle[(size_t)cn] = (a + kMaxSample) % kMaxSample;
+					}
+					if (opt.verbose > 1) {
+						printf ("%.2f %.4f", ((a + kMaxSample) % kMaxSample) / (float)kSubsample, to_dB (tab.peak (-1, a, mask)));
+						for (int c = 0; c < C; ++c) {
+							printf (" %.4f", to_dB (tab.peak (c, a, mask)));
+						}
+						printf ("\n");
+					}
+				}
+			}
+		}
+	}
+
+	// minimise the channel phase distance (cli:905-929)
+	float avg_rotate = 0;
+	int   avg_count  = 0;
+	for (int c = 0; c < C; ++c) {
+		if (p_min[(size_t)c] != inf) {
+			avg_rotate += min_angle[(size_t)c];
+			++avg_count;
+		}
+	}
+	avg_rotate /= avg_count;
+	const float avg_dist = kMaxSample / (float)avg_count;
+	for (int c = 0; c < C; ++c) {
+		if (p_min[(size_t)c] == inf) {
+			continue;
+		}
+		if (min_angle[(size_t)c] > 90 * kSubsample && fabsf (min_angle[(size_t)c] - avg_rotate) > avg_dist) {
+			min_angle[(size_t)c] -= kMaxSample;
+		} else if (avg_rotate > 90 * kSubsample) {
+			min_angle[(size_t)c] -= kMaxSample;
+		}
+	}
+	return MinResult { min_angle, p_min, r_zro, r_min };
+}
+
+// the per-channel result lines of the report (cli:931-947)
+void
+report_channels (const MinResult& r, FILE* vfd)
+{
+	const float inf = std::numeric_limits<float>::infinity ();
+	for (size_t c = 0; c < r.angle.size (); ++c) {
+		if (r.p_min[c] == inf) {
+			fprintf (vfd, "Channel: %2d Phase:   0 deg # cannot find min.\n", (int)c + 1);
+			continue;
+		}
+		fprintf (vfd, "Channel: %2d Phase: %5.2f deg", (int)c + 1, r.angle[c] / (float)kSubsample);
+		if (r.angle[c] != 0) {
+			fprintf (vfd, ", gain: %5.2f dB (att. %4.2f to %4.2f dBFS)", to_dB (r.r_zro[c]) - to_dB (r.r_min[c]), to_dB (r.r_zro[c]), to_dB (r.r_min[c]));
+		}
+		fprintf (vfd, "\n");
+	}
+}
 
 } // namespace
 
@@ -491,7 +650,47 @@ main (int argc, char** argv)
 	}
 	timer.mark ("phaserot_create (tables, kernels)");
 
-	if (find_min) {
+	uint64_t         sect_len = 0; // --sections: frames per section
+	std::vector<int> sect_angles;  // --sections: [section][channel] in grid steps on the full circle
+	if (find_min && opt.sections > 0) {
+		// one sweep, one table per section; the search of the whole-file analysis runs on each of them
+		const uint64_t al = phaserot_shard_align (pr);
+		sect_len          = std::max<uint64_t> (1, (uint64_t)ceil (ceil (opt.sections * nfo.samplerate) / (double)al)) * al; // rounded up
+		if (opt.verbose) {
+			fprintf (vfd, "Section length  : %.3f s (%llu frames)\n", sect_len / (double)nfo.samplerate, (unsigned long long)sect_len);
+		}
+		check (phaserot_sweep_sections (pr, audio, pcm_fmt, F, sect_len, 0, kMaxSample, 1, -1), "analysis failed");
+		int ns = 0;
+		check (phaserot_section_peaks (pr, &ns, nullptr), "analysis failed");
+		const size_t       per = (size_t)C * kMaxSample;
+		std::vector<float> tables ((size_t)ns * per);
+		check (phaserot_section_peaks (pr, &ns, tables.data ()), "analysis failed");
+		timer.mark ("analysis (upload + sweep)");
+		if (!outfile || opt.verbose) {
+			fprintf (vfd, "# Result -- Minimize digital peak\n");
+		}
+		PeakTable tab;
+		tab.channels = C;
+		for (int k = 0; k < ns; ++k) {
+			tab.t.assign (tables.begin () + (std::ptrdiff_t)(k * per), tables.begin () + (std::ptrdiff_t)((k + 1) * per));
+			const MinResult r = find_min_angles (tab, opt, vfd);
+			if (!outfile || opt.verbose) {
+				fprintf (vfd, "# Section %d: %.3f - %.3f s\n", k + 1, (double)k * sect_len / nfo.samplerate,
+				         (double)std::min<uint64_t> (F, (uint64_t)(k + 1) * sect_len) / nfo.samplerate);
+				report_channels (r, vfd);
+			}
+			for (int c = 0; c < C; ++c) {
+				// section 0 renders at the index the whole-file render uses (cli:463); every following section
+				// at whichever of a, a - 180 deg (the same peak) is nearer to the angle before it: a ramp
+				// between sections never turns more than 90 degrees
+				int a = ((r.angle[(size_t)c] % kMaxSample) + kMaxSample) % kMaxSample;
+				if (k > 0) {
+					a += kMaxSample * (int)lround ((sect_angles[(size_t)(k - 1) * C + c] - a) / (double)kMaxSample);
+				}
+				sect_angles.push_back (a);
+			}
+		}
+	} else if (find_min) {
 		const int stride = opt.stride;
 		if (opt.verbose > 1) {
 			fprintf (vfd, "Analyzing using %d process threads, stride = %d\n", C, stride);
@@ -509,136 +708,11 @@ main (int argc, char** argv)
 		tab.t.resize ((size_t)C * kMaxSample);
 		check (phaserot_peaks (pr, tab.t.data ()), "analysis failed");
 		timer.mark ("analysis (upload + sweep)");
-		const std::vector<bool> all ((size_t)C, true);
-
-		if (opt.verbose > 1) { // gnuplot table of the coarse pass (cli:800-813)
-			printf ("# Angle mono-peak");
-			for (int c = 0; c < C; ++c) {
-				printf (" chn-%d", c + 1);
-			}
-			printf ("\n");
-			for (int a = 0; a < kMaxSample; a += stride) {
-				printf ("%.2f %.4f", a / (float)kSubsample, to_dB (tab.peak (-1, a, all)));
-				for (int c = 0; c < C; ++c) {
-					printf (" %.4f", to_dB (tab.peak (c, a, all)));
-				}
-				printf ("\n");
-			}
-		}
-
-		const float inf = std::numeric_limits<float>::infinity ();
-		std::map<int, std::vector<int>> mins; // coarse angle -> channels to refine there
-		std::vector<int>   min_angle ((size_t)C, 0);
-		// The reference leaves p_min / min_angle uninitialised for a channel whose
-		// coarse peaks are all equal (cli:835-839); +inf / 0 is the evident intent.
-		std::vector<float> p_min ((size_t)C, inf), r_zro ((size_t)C, 0.f), r_min ((size_t)C, 0.f);
-
-		for (int c = 0; c < C; ++c) {
-			const int pc   = opt.link ? -1 : c;
-			float     cmin = inf, cmax = 0;
-			r_zro[(size_t)c] = tab.peak (c, 0, all);
-			for (int a = 0; a < kMaxSample; a += stride) {
-				cmin = std::min (cmin, tab.peak (pc, a, all));
-				cmax = std::max (cmax, tab.peak (pc, a, all));
-			}
-			float range = cmax - cmin;
-			if (range == 0) {
-				mins[0].push_back (c);
-				continue;
-			}
-			if (stride > 1) {
-				range *= .07;
-				p_min[(size_t)c] = inf;
-			} else {
-				range            = 0;
-				p_min[(size_t)c] = cmin;
-			}
-			for (int a = 0; a < kMaxSample; a += stride) {
-				const float p = tab.peak (pc, a, all);
-				if (p <= cmin + range) {
-					mins[a].push_back (c);
-					if (opt.verbose > 1) {
-						fprintf (vfd, "Consider min: %f (< %f) chn: %d @ %.2f deg\n", p, cmin + range, c, a / (float)kSubsample);
-					}
-				}
-			}
-		}
-
-		if (stride == 1) {
-			for (auto& mp : mins) { // ascending: the largest angle wins (cli:859-865)
-				for (int cn : mp.second) {
-					min_angle[(size_t)cn] = mp.first;
-					r_min[(size_t)cn]     = tab.peak (cn, mp.first, all);
-				}
-			}
-		} else {
-			const int s2 = (stride + 1) / 2;
-			for (auto& mp : mins) {
-				// which channels the reference's refine pass analyses (cli:880)
-				std::vector<bool> mask ((size_t)C, mp.second.size () > 1);
-				if (mp.second.size () == 1) {
-					mask[(size_t)mp.second.front ()] = true;
-				}
-				const int ma = mp.first;
-				for (int cn : mp.second) {
-					for (int a = ma - s2; a < ma + s2 + 1; ++a) {
-						const float p = tab.peak (opt.link ? -1 : cn, a, mask);
-						if (p <= p_min[(size_t)cn]) { // ties: the later angle wins (cli:885)
-							p_min[(size_t)cn]     = p;
-							r_min[(size_t)cn]     = tab.peak (cn, a, mask);
-							min_angle[(size_t)cn] = (a + kMaxSample) % kMaxSample;
-						}
-						if (opt.verbose > 1) {
-							printf ("%.2f %.4f", ((a + kMaxSample) % kMaxSample) / (float)kSubsample, to_dB (tab.peak (-1, a, mask)));
-							for (int c = 0; c < C; ++c) {
-								printf (" %.4f", to_dB (tab.peak (c, a, mask)));
-							}
-							printf ("\n");
-						}
-					}
-				}
-			}
-		}
-
-		// minimise the channel phase distance (cli:905-929)
-		float avg_rotate = 0;
-		int   avg_count  = 0;
-		for (int c = 0; c < C; ++c) {
-			if (p_min[(size_t)c] != inf) {
-				avg_rotate += min_angle[(size_t)c];
-				++avg_count;
-			}
-		}
-		avg_rotate /= avg_count;
-		const float avg_dist = kMaxSample / (float)avg_count;
-		angles.clear ();
-		for (int c = 0; c < C; ++c) {
-			if (p_min[(size_t)c] == inf) {
-				angles.push_back (0);
-				continue;
-			}
-			if (min_angle[(size_t)c] > 90 * kSubsample && fabsf (min_angle[(size_t)c] - avg_rotate) > avg_dist) {
-				min_angle[(size_t)c] -= kMaxSample;
-			} else if (avg_rotate > 90 * kSubsample) {
-				min_angle[(size_t)c] -= kMaxSample;
-			}
-			angles.push_back (min_angle[(size_t)c]);
-		}
-
+		const MinResult r = find_min_angles (tab, opt, vfd);
+		angles            = r.angle;
 		if (!outfile || opt.verbose) { // report (cli:931-947)
 			fprintf (vfd, "# Result -- Minimize digital peak\n");
-			for (int c = 0; c < C; ++c) {
-				if (p_min[(size_t)c] == inf) {
-					fprintf (vfd, "Channel: %2d Phase:   0 deg # cannot find min.\n", c + 1);
-					continue;
-				}
-				fprintf (vfd, "Channel: %2d Phase: %5.2f deg", c + 1, min_angle[(size_t)c] / (float)kSubsample);
-				if (min_angle[(size_t)c] != 0) {
-					fprintf (vfd, ", gain: %5.2f dB (att. %4.2f to %4.2f dBFS)", to_dB (r_zro[(size_t)c]) - to_dB (r_min[(size_t)c]),
-					         to_dB (r_zro[(size_t)c]), to_dB (r_min[(size_t)c]));
-				}
-				fprintf (vfd, "\n");
-			}
+			report_channels (r, vfd);
 		}
 	}
 
@@ -667,7 +741,7 @@ main (int argc, char** argv)
 		};
 
 		std::vector<float> last_out (bs, 0.f); // processed block the reference would still hold in `buf`
-		if (opt.fixed_write) {
+		if (opt.fixed_write || sect_len) {
 			// --fixed-write: the latency-compensated render y[t + L/2], t in [0, F), as the
 			// write loop intends it: the trim counts FRAMES (the reference offsets the
 			// interleaved buffer by `latency` floats, cli:985: channels > 1 start at frame
@@ -682,7 +756,11 @@ main (int argc, char** argv)
 			if (!y) {
 				die ("Out of memory\n");
 			}
-			check (phaserot_render (pr, audio, F, angles.data (), 1, y), "render failed");
+			if (sect_len) { // --sections: always written this way
+				check (phaserot_render_sections (pr, audio, F, sect_len, sect_angles.data (), 1, y), "render failed");
+			} else {
+				check (phaserot_render (pr, audio, F, angles.data (), 1, y), "render failed");
+			}
 			if ((sf_count_t)F != sf_writef_float (outfile, y + (size_t)latency * (size_t)C, (sf_count_t)F)) {
 				fprintf (stderr, "Error writing to output file.\n");
 			}
