@@ -262,6 +262,38 @@ PHASEROT_API int phaserot_render_sections (phaserot_t* h, const float* interleav
 PHASEROT_API int phaserot_render_sections_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, uint64_t section_frames,
                                                   const int* angles, int flush_blocks, float* d_out);
 
+/* ---- integrated loudness of the rotated output ----------------------------- */
+
+/* Extends the report of analyze_file (cli:931-947), which gives the peak before and after rotation, with the
+ * integrated loudness of ITU-R BS.1770-4 before and after: the peak-to-loudness ratio a loudness target with a
+ * true-peak ceiling (EBU R128: -23 LUFS / -1 dBTP) is met with, and a check that rotation kept the loudness.
+ * For each of n_sets angle sets, lufs[k] is the integrated loudness of the output phaserot_render() writes after
+ * the latency trim at those angles (the --fixed-write render):
+ *     out[t] = ca[c] x[t] + sa[c] H'[t],   t in [0, n_frames),   H' = Hilbert branch aligned to x
+ * with (sa, ca) the SinCosLut pair (cli:41-72) of angles[k * n_channels + c], in grid steps on the FULL circle as
+ * in phaserot_render_sections() (a + 180 * subsample is the negation of a, which measures the same).  Set 0 at
+ * angle 0 is the input itself.  No first-block rule applies: that rule belongs to the analysis only.
+ *   K-weighting : the two biquads of BS.1770-4 (high shelf, then high pass), coefficients for any rate derived
+ *                 as libebur128 does - at 48 kHz they are those of Tables 1 and 2
+ *   gating      : sub-blocks of step = floor(sample_rate / 10 + 0.5) frames; 400 ms blocks of 4 sub-blocks,
+ *                 hop 1 sub-block, complete blocks only; l_j = -0.691 + 10 log10 sum_c G_c z_cj; absolute gate
+ *                 -70 LUFS, then the relative gate -10 LU; lufs = -0.691 + 10 log10 (gated mean)
+ *                 -INFINITY when no block passes or the stream is shorter than 400 ms
+ *   weights     : G_c per channel (NULL = 1.0 each; BS.1770 5.1 in WAV order: 1, 1, 1, 0, 1.41, 1.41)
+ * Rotation and K-weighting are linear, so every 100 ms sub-block's mean square is a quadratic form in (ca, sa);
+ * one pass gives its three sums and any number of angle sets costs only the gate.
+ * `data` and `format` as phaserot_sweep_pcm() / PHASEROT_PCM_F32, with the same widening; host memory.
+ * Synchronous; deterministic (the same doubles on every call, and from the host and device forms on the same
+ * float input).  The peak table, section tables and apply() stream state are not changed (the host form
+ * completes a pending device sweep first, as phaserot_peaks() would).  Valid for true-peak handles too.
+ * PHASEROT_E_STATE for plugin handles; PHASEROT_E_INVAL with a phaserot_last_error() text for n_sets < 1, NULL
+ * angles or lufs, a negative or non-finite weight, n_frames == 0 or a sample_rate outside [8000, 768000]. */
+PHASEROT_API int phaserot_loudness (phaserot_t* h, const void* data, int format, uint64_t n_frames, double sample_rate,
+                                    const float* weights, const int* angles, int n_sets, double* lufs);
+/* The same over audio resident in device memory (interleaved float32, n_frames * n_channels). */
+PHASEROT_API int phaserot_loudness_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, double sample_rate,
+                                           const float* weights, const int* angles, int n_sets, double* lufs);
+
 /* ---- several GPUs in one process ---------------------------------------- */
 
 /* A group of handles, one per device, that analyses ONE stream: the file is cut

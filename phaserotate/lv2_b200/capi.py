@@ -28,6 +28,7 @@ SYMBOLS = [
     "phaserot_sweep_shard_boot_device", "phaserot_sweep_shard_resume",
     "phaserot_sweep_sections", "phaserot_sweep_sections_device", "phaserot_section_peaks",
     "phaserot_render_sections", "phaserot_render_sections_device",
+    "phaserot_loudness", "phaserot_loudness_device",
     "phaserot_group_create", "phaserot_group_destroy", "phaserot_group_size", "phaserot_group_handle", "phaserot_group_sweep",
     "phaserot_group_peaks", "phaserot_group_reset", "phaserot_pending_table", "phaserot_set_profiling", "phaserot_get_kernel_times",
     "phaserot_sync", "phaserot_get_stats", "phaserot_reset_stats",
@@ -110,6 +111,8 @@ def load():
     lib.phaserot_section_peaks.argtypes = [vp, C.POINTER(C.c_int), vp]
     lib.phaserot_render_sections.argtypes = [vp, vp, C.c_uint64, C.c_uint64, vp, C.c_int, vp]
     lib.phaserot_render_sections_device.argtypes = [vp, vp, C.c_uint64, C.c_uint64, vp, C.c_int, vp]
+    lib.phaserot_loudness.argtypes = [vp, vp, C.c_int, C.c_uint64, C.c_double, vp, vp, C.c_int, vp]
+    lib.phaserot_loudness_device.argtypes = [vp, vp, C.c_uint64, C.c_double, vp, vp, C.c_int, vp]
     lib.phaserot_group_create.argtypes = [C.POINTER(vp), C.POINTER(Cfg), vp, C.c_int]
     lib.phaserot_group_destroy.argtypes = [vp]
     lib.phaserot_group_destroy.restype = None
@@ -350,6 +353,31 @@ class Phaserot:
         ang = np.ascontiguousarray(angles, np.int32)
         self._ck(self._lib.phaserot_render_sections_device(self._h, C.c_void_p(d_in), n_frames, section_frames, _ptr(ang), flush_blocks,
                                                            C.c_void_p(d_out)), "phaserot_render_sections_device")
+
+    # -- integrated loudness -------------------------------------------------
+    def _loudness_args(self, angle_sets, weights):
+        ang = np.ascontiguousarray(angle_sets, np.int32).reshape(-1, self.n_channels)
+        w = None if weights is None else np.ascontiguousarray(weights, np.float32).reshape(self.n_channels)
+        return ang, w, np.zeros(ang.shape[0], np.float64)
+
+    def loudness(self, x, angle_sets, sample_rate, weights=None):
+        """BS.1770-4 integrated loudness (LUFS) of the trimmed render at each angle set.
+        x: host array [frames, channels] of float32, int16 or int32 (PCM_S32), or packed 24-bit uint8 bytes;
+        angle_sets: [n_sets, channels] grid steps on the full circle; weights: [channels] or None (1.0)."""
+        x = np.ascontiguousarray(x)
+        fmt = {np.dtype(np.float32): PCM_F32, np.dtype(np.int16): PCM_S16, np.dtype(np.int32): PCM_S32, np.dtype(np.uint8): PCM_S24}[x.dtype]
+        n = x.size // self.n_channels // (3 if fmt == PCM_S24 else 1)
+        ang, w, out = self._loudness_args(angle_sets, weights)
+        self._ck(self._lib.phaserot_loudness(self._h, _ptr(x), fmt, n, float(sample_rate), None if w is None else _ptr(w), _ptr(ang),
+                                             ang.shape[0], _ptr(out)), "phaserot_loudness")
+        return out
+
+    def loudness_device(self, ptr, n_frames, angle_sets, sample_rate, weights=None):
+        """The same over interleaved float32 audio in device memory."""
+        ang, w, out = self._loudness_args(angle_sets, weights)
+        self._ck(self._lib.phaserot_loudness_device(self._h, C.c_void_p(ptr), n_frames, float(sample_rate), None if w is None else _ptr(w),
+                                                    _ptr(ang), ang.shape[0], _ptr(out)), "phaserot_loudness_device")
+        return out
 
     # -- CLI render --------------------------------------------------------
     def apply(self, buf, angles):

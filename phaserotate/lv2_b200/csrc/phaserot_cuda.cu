@@ -9,6 +9,7 @@
 // launch, and create() refuses to hand out a handle without an sm_100 device.
 #include "../../../include/phaserot_cuda.h"
 #include "kernels.cuh"
+#include "loudness.cuh"
 #include "fft16k_tables.h"
 
 #include <algorithm>
@@ -16,6 +17,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <mutex>
 #include <new>
 #include <string>
@@ -234,6 +236,10 @@ struct phaserot {
 	std::vector<int>       sect_idx;
 	std::vector<long long> sect_redo_k; // sections whose list overflowed: their tables come from the shard path
 	std::vector<float>     sect_redo;   // [redone section][C][MS]
+
+	// integrated loudness (phaserot_loudness): K(x) [frames][C] floats | Hilbert branch of one FFT launch [C][stride]
+	// floats | fp64 work: sub-block sums, head correction, chunk states, A powers, weights, results | angle sets
+	DevBuf d_kx, d_lH, d_lwork, d_lset;
 
 	// pending (asynchronous) sweep result
 	bool             pending = false;
@@ -1598,6 +1604,256 @@ render_sections_core (phaserot* h, const float* d_src, long long n_frames, long 
 	return PHASEROT_OK;
 }
 
+// ---------------------------------------------------------------------------
+// Integrated loudness of the rotated output (phaserot_loudness*, loudness.cuh)
+// ---------------------------------------------------------------------------
+
+// K-weighting at any rate, derived like libebur128 does; at 48 kHz these are the
+// coefficients of BS.1770-4 Tables 1 and 2
+KwCoef
+kweight_coef (double fs)
+{
+	KwCoef       k {};
+	double       K  = std::tan (M_PI * 1681.974450955533 / fs);
+	const double Qs = 0.7071752369554196;
+	const double Vh = std::pow (10.0, 3.999843853973347 / 20.0);
+	const double Vb = std::pow (Vh, 0.4996667741545416);
+	double       a0 = 1.0 + K / Qs + K * K;
+	k.b[0][0]       = (Vh + Vb * K / Qs + K * K) / a0;
+	k.b[0][1]       = 2.0 * (K * K - Vh) / a0;
+	k.b[0][2]       = (Vh - Vb * K / Qs + K * K) / a0;
+	k.a[0][0]       = 1.0;
+	k.a[0][1]       = 2.0 * (K * K - 1.0) / a0;
+	k.a[0][2]       = (1.0 - K / Qs + K * K) / a0;
+	K               = std::tan (M_PI * 38.13547087602444 / fs);
+	const double Qh = 0.5003270373238773;
+	a0              = 1.0 + K / Qh + K * K;
+	k.b[1][0]       = 1.0;
+	k.b[1][1]       = -2.0;
+	k.b[1][2]       = 1.0;
+	k.a[1][0]       = 1.0;
+	k.a[1][1]       = 2.0 * (K * K - 1.0) / a0;
+	k.a[1][2]       = (1.0 - K / Qh + K * K) / a0;
+	return k;
+}
+
+// P[m - 1] = A^(m N), m = 1 .. 32: A is the zero-input state transition of the K cascade (kw_step)
+std::vector<double>
+kweight_powers (const KwCoef& k, long long N)
+{
+	using M4 = std::vector<double>;
+	auto mul = [] (const M4& a, const M4& b) {
+		M4 r (16, 0.0);
+		for (int i = 0; i < 4; ++i)
+			for (int j = 0; j < 4; ++j)
+				for (int q = 0; q < 4; ++q) r[4 * i + j] += a[4 * i + q] * b[4 * q + j];
+		return r;
+	};
+	M4 A (16, 0.0);
+	for (int j = 0; j < 4; ++j) { // column j = one zero-input step from unit state j
+		double s[4] = { 0., 0., 0., 0. };
+		s[j]            = 1.0;
+		const double y1 = s[0];
+		const double n0 = -k.a[0][1] * y1 + s[1], n1 = -k.a[0][2] * y1;
+		const double y2 = k.b[1][0] * y1 + s[2];
+		const double n2 = k.b[1][1] * y1 - k.a[1][1] * y2 + s[3], n3 = k.b[1][2] * y1 - k.a[1][2] * y2;
+		A[0 + j] = n0, A[4 + j] = n1, A[8 + j] = n2, A[12 + j] = n3;
+	}
+	M4 AN (16, 0.0);
+	for (int i = 0; i < 4; ++i) AN[5 * i] = 1.0;
+	for (long long e = N; e; e >>= 1, A = mul (A, A)) {
+		if (e & 1) AN = mul (AN, A);
+	}
+	std::vector<double> P;
+	M4                  Am = AN;
+	for (int m = 1; m <= 32; ++m, Am = mul (Am, AN)) P.insert (P.end (), Am.begin (), Am.end ());
+	return P;
+}
+
+// The Hilbert instantiation is loaded with the true-peak handles; loudness needs it on every CLI handle.
+int
+ensure_hilbert_attrs (phaserot* h)
+{
+	std::lock_guard<std::mutex> lk (g_create_lock);
+	return set_device_attrs (h->dev, false, h->NP, 2);
+}
+
+constexpr long long kKwChunk = 4096; // frames per thread of kweight_kernel
+
+/*
+ * phaserot_loudness over F frames of interleaved float32 audio on the device.
+ *   weights : host [C] or null (1.0)      angles : host [n_sets][C], full circle
+ */
+int
+loudness_core (phaserot* h, const float* d_x, long long F, double fs, const float* weights, const int* angles, int n_sets, double* lufs)
+{
+	const int       C     = h->C;
+	const long long step  = (long long)std::floor (fs / 10.0 + 0.5); // 100 ms sub-block
+	const long long n_sub = F / step;
+	if (n_sub < 4) { // no complete 400 ms block
+		std::fill (lufs, lufs + n_sets, -std::numeric_limits<double>::infinity ());
+		return PHASEROT_OK;
+	}
+	int rc = ensure_hilbert_attrs (h);
+	if (rc) return rc;
+	const long long Fu       = n_sub * step;                  // samples that lie in a sub-block
+	const int       D        = h->L / 2;                      // latency of the render
+	const long long T        = Fu + D;                        // K(x) frames the Hilbert branch of t < Fu reads
+	const long long n_chunk  = (T + kKwChunk - 1) / kKwChunk;
+	const int       nz       = (int)std::min (Fu, step);      // samples of the head correction
+	const long long V2       = 2LL * h->V;                    // samples per FFT segment
+	const long long nseg     = (T + V2 - 1) / V2;
+	const long long segs     = std::min (nseg, std::max<long long> (1, (long long)h->n_sm * 16 / C)); // per FFT launch
+	const long long h_stride = (kTpCarry + segs * V2 + 3) & ~3LL;
+	const KwCoef    kc       = kweight_coef (fs);
+
+	// fp64 work area
+	const size_t n_sums = (size_t)n_sub * C * 3, n_zc = (size_t)C * nz, n_st = (size_t)n_chunk * C * 4;
+	rc = h->d_kx.ensure (sizeof (float) * (size_t)T * C);
+	if (rc) return rc;
+	rc = h->d_lH.ensure (sizeof (float) * (size_t)h_stride * C);
+	if (rc) return rc;
+	rc = h->d_lwork.ensure (sizeof (double) * (n_sums + n_zc + n_st + 32 * 16 + C + (size_t)n_sets));
+	if (rc) return rc;
+	rc = h->d_lset.ensure (sizeof (float2) * (size_t)n_sets * C);
+	if (rc) return rc;
+	double*  d_sums = (double*)h->d_lwork.p;
+	double*  d_zc   = d_sums + n_sums;
+	KwState* d_st   = (KwState*)(d_zc + n_zc);
+	double*  d_P    = d_zc + n_zc + n_st;
+	double*  d_G    = d_P + 32 * 16;
+	double*  d_lufs = d_G + C;
+	float*   d_kx   = (float*)h->d_kx.p;
+	float*   d_H    = (float*)h->d_lH.p;
+
+	// rotations of every set, as phaserot_render_sections forms them: a + MS is the negation of a
+	std::vector<float2> cs ((size_t)n_sets * C);
+	for (size_t r = 0; r < cs.size (); ++r) {
+		const long long a  = angles[r];
+		const long long q  = (a >= 0 ? a : a - h->MS + 1) / h->MS;
+		const size_t    i  = (size_t)(a - q * h->MS);
+		const float     sg = (q & 1) ? -1.f : 1.f;
+		cs[r]              = make_float2 (sg * h->lut_c[i], sg * h->lut_s[i]);
+	}
+	std::vector<double> G ((size_t)C, 1.0);
+	if (weights) {
+		for (int c = 0; c < C; ++c) G[(size_t)c] = weights[c];
+	}
+	const std::vector<double> P = kweight_powers (kc, kKwChunk);
+	CK (cudaMemcpyAsync (h->d_lset.p, cs.data (), sizeof (float2) * cs.size (), cudaMemcpyHostToDevice, h->stream));
+	CK (cudaMemcpyAsync (d_P, P.data (), sizeof (double) * P.size (), cudaMemcpyHostToDevice, h->stream));
+	CK (cudaMemcpyAsync (d_G, G.data (), sizeof (double) * G.size (), cudaMemcpyHostToDevice, h->stream));
+	CK (cudaMemsetAsync (d_sums, 0, sizeof (double) * n_sums, h->stream));
+
+	ConvParams p;
+	fill_conv_common (h, p);
+	p.C           = C;
+	p.chan0       = 0;
+	p.nchan       = C;
+	p.seg_stride  = 1;
+	p.out         = (float2*)d_H;
+	p.out_stride  = h_stride / 2;
+	p.out_compact = 1;
+
+	// head correction: the Hilbert branch of x itself over its first segment (2 V >= D samples)
+	p.inter    = d_x;
+	p.n_frames = F;
+	p.m_end    = (T + 1) / 2;
+	p.seg0     = 0;
+	p.nseg     = 1;
+	rc         = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
+	if (rc) return rc;
+	{
+		ProfScope ps (h, 5);
+		loudness_head_kernel<<<C, 32, 0, h->stream>>> (d_H, h_stride, D, kc, d_zc, nz);
+	}
+	CK (cudaGetLastError ());
+	++h->stats.kernel_launches;
+
+	// K(x) over [0, T): zero-state chunks, carry, re-run from the carried states
+	{
+		ProfScope      ps (h, 5);
+		const unsigned nb = (unsigned)((n_chunk * C + 255) / 256);
+		kweight_kernel<false><<<nb, 256, 0, h->stream>>> (d_x, F, T, C, kKwChunk, kc, d_st, nullptr);
+		kweight_carry_kernel<<<C, 32, 0, h->stream>>> (d_st, n_chunk, C, d_P);
+		kweight_kernel<true><<<nb, 256, 0, h->stream>>> (d_x, F, T, C, kKwChunk, kc, d_st, d_kx);
+	}
+	CK (cudaGetLastError ());
+	h->stats.kernel_launches += 3;
+
+	// Hilbert branch of K(x), one launch of segments at a time, each consumed by the sums
+	p.inter    = d_kx;
+	p.n_frames = T;
+	for (long long s0 = 0; s0 < nseg; s0 += segs) {
+		p.seg0 = s0;
+		p.nseg = std::min (segs, nseg - s0);
+		rc     = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
+		if (rc) return rc;
+		const long long u0 = s0 * V2, lo = std::max (0LL, u0 - D), hi = std::min (Fu, u0 + p.nseg * V2 - D);
+		if (lo >= hi) continue;
+		const long long j0 = lo / step, j1 = (hi - 1) / step;
+		{
+			ProfScope ps (h, 5);
+			loudness_stats_kernel<<<dim3 ((unsigned)(j1 - j0 + 1), (unsigned)C), 256, 0, h->stream>>> (d_kx, C, d_H, h_stride, u0, D, step, j0, lo, hi, d_zc, nz,
+			                                                                                           d_sums);
+		}
+		CK (cudaGetLastError ());
+		++h->stats.kernel_launches;
+	}
+
+	{
+		ProfScope ps (h, 5);
+		loudness_gate_kernel<<<(unsigned)n_sets, 256, 0, h->stream>>> (d_sums, C, n_sub - 3, step, (const float2*)h->d_lset.p, d_G, d_lufs);
+	}
+	CK (cudaGetLastError ());
+	++h->stats.kernel_launches;
+	CK (cudaMemcpyAsync (lufs, d_lufs, sizeof (double) * (size_t)n_sets, cudaMemcpyDeviceToHost, h->stream));
+	CK (cudaStreamSynchronize (h->stream));
+	h->stats.d2h_bytes += sizeof (double) * (size_t)n_sets;
+	prof_resolve (h);
+	return PHASEROT_OK;
+}
+
+int
+loudness_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t n_frames, double fs, const float* weights, const int* angles, int n_sets,
+                double* lufs)
+{
+	if (!h) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->plugin) {
+		return PHASEROT_E_STATE;
+	}
+	const char* bad = nullptr;
+	if (!src) bad = "NULL audio";
+	else if (format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) bad = "unknown sample format";
+	else if (n_frames == 0) bad = "n_frames is 0";
+	else if (!(fs >= 8000.0 && fs <= 768000.0)) bad = "sample_rate outside [8000, 768000]";
+	else if (n_sets < 1) bad = "n_sets < 1";
+	else if (!angles || !lufs) bad = "NULL angles or lufs";
+	for (int c = 0; !bad && weights && c < h->C; ++c) {
+		if (!std::isfinite (weights[c]) || weights[c] < 0.f) bad = "a channel weight is negative or not finite";
+	}
+	if (bad) {
+		snprintf (g_last_error, sizeof (g_last_error), "phaserot_loudness: %s", bad);
+		return PHASEROT_E_INVAL;
+	}
+	DevGuard     guard (h->dev);
+	const float* d_x = (const float*)src;
+	if (!dev_in) {
+		// d_inter may still be the source of the pending sweep's dense-mode repeat: complete that sweep first
+		int rc = finish_pending (h);
+		if (rc) return rc;
+		const int pcm_bytes = format == PHASEROT_PCM_S16 ? 2 : format == PHASEROT_PCM_S32 ? 4 : format == PHASEROT_PCM_S24 ? 3 : 0;
+		rc                  = h->d_inter.ensure (sizeof (float) * (size_t)n_frames * h->C);
+		if (rc) return rc;
+		rc = upload_chunks (h, src, pcm_bytes, (long long)n_frames, [] (long long) { return PHASEROT_OK; });
+		if (rc) return rc;
+		d_x = (const float*)h->d_inter.p;
+	}
+	return loudness_core (h, d_x, (long long)n_frames, fs, weights, angles, n_sets, lufs);
+}
+
 /*
  * Render stream: y[t] = ca x[t - L/2] + sa H[t] for t in [0, t_end).
  *   d_dst_inter == nullptr   planar result left in d_out (float2 per two samples; plugin bulk path)
@@ -1998,7 +2254,7 @@ phaserot_destroy (phaserot_t* h)
 	if (h->copy_stream) cudaStreamSynchronize (h->copy_stream);
 	for (DevBuf* b : { &h->d_G, &h->d_G1, &h->d_scratch, &h->d_tw, &h->d_g, &h->d_plane, &h->d_out, &h->d_list, &h->d_stage[0], &h->d_stage[1], &h->d_io, &h->d_inter, &h->d_hist, &h->d_small,
 	                   &h->d_cs, &h->d_peaks, &h->d_ramp, &h->d_chancs, &h->d_tpH, &h->d_ring, &h->d_slot, &h->d_sec, &h->d_wide,
-	                   &h->d_sect, &h->d_sect_aux, &h->d_sect_rt }) {
+	                   &h->d_sect, &h->d_sect_aux, &h->d_sect_rt, &h->d_kx, &h->d_lH, &h->d_lwork, &h->d_lset }) {
 		b->release ();
 	}
 	for (PinBuf* b : { &h->h_stage[0], &h->h_stage[1], &h->h_res, &h->h_io, &h->h_cs, &h->h_slot }) {
@@ -2545,6 +2801,20 @@ phaserot_render_sections_device (phaserot_t* h, const float* d_interleaved, uint
                                  float* d_out)
 {
 	return render_sections_bulk (h, d_interleaved, true, n_frames, section_frames, angles, flush_blocks, d_out, true);
+}
+
+int
+phaserot_loudness (phaserot_t* h, const void* data, int format, uint64_t n_frames, double sample_rate, const float* weights, const int* angles, int n_sets,
+                   double* lufs)
+{
+	return loudness_entry (h, data, false, format, n_frames, sample_rate, weights, angles, n_sets, lufs);
+}
+
+int
+phaserot_loudness_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, double sample_rate, const float* weights, const int* angles, int n_sets,
+                          double* lufs)
+{
+	return loudness_entry (h, d_interleaved, true, PHASEROT_PCM_F32, n_frames, sample_rate, weights, angles, n_sets, lufs);
 }
 
 uint32_t

@@ -63,6 +63,7 @@ struct Options {
 	int          gpus        = 1;     // --gpus N: sample-range shards over N devices (0 = all)
 	bool         fixed_write = false; // --fixed-write: write loop without the reference's two quirks (cli:985, cli:973)
 	double       sections    = 0;     // --sections SECONDS: one angle per section of the file (0 = one for the whole file)
+	bool         loudness    = false; // --loudness: BS.1770-4 integrated loudness and PLR of the input and of the output
 };
 
 // PHASEROT_CLI_TIMING=1: wall-clock breakdown of the process on stderr (file read, CUDA
@@ -174,6 +175,7 @@ parse_options (int argc, char** argv)
 		{ "gpus", required_argument, 0, 1002 },
 		{ "fixed-write", no_argument, 0, 1003 },
 		{ "sections", required_argument, 0, 1004 },
+		{ "loudness", no_argument, 0, 1005 },
 		{ 0, 0, 0, 0 },
 	};
 	int c;
@@ -219,11 +221,15 @@ parse_options (int argc, char** argv)
 				}
 				break;
 			}
+			case 1005: o.loudness = true; break;
 			default: die ("Error: unrecognized option. See --help for usage information.\n");
 		}
 	}
 	if (o.sections > 0 && (o.angles_arg || o.oversample || o.gpus != 1)) {
 		die ("Error: --sections cannot be combined with -a, --true-peak or --gpus.\n");
+	}
+	if (o.loudness && (o.angles_arg || o.sections > 0 || o.gpus != 1)) {
+		die ("Error: --loudness cannot be combined with -a, --sections or --gpus.\n");
 	}
 	kSubsample = o.subsample;
 	kMaxSample = 180 * kSubsample;
@@ -650,6 +656,7 @@ main (int argc, char** argv)
 	}
 	timer.mark ("phaserot_create (tables, kernels)");
 
+	MinResult        res;          // whole-file analysis: what the result lines report
 	uint64_t         sect_len = 0; // --sections: frames per section
 	std::vector<int> sect_angles;  // --sections: [section][channel] in grid steps on the full circle
 	if (find_min && opt.sections > 0) {
@@ -708,12 +715,36 @@ main (int argc, char** argv)
 		tab.t.resize ((size_t)C * kMaxSample);
 		check (phaserot_peaks (pr, tab.t.data ()), "analysis failed");
 		timer.mark ("analysis (upload + sweep)");
-		const MinResult r = find_min_angles (tab, opt, vfd);
-		angles            = r.angle;
+		res    = find_min_angles (tab, opt, vfd);
+		angles = res.angle;
 		if (!outfile || opt.verbose) { // report (cli:931-947)
 			fprintf (vfd, "# Result -- Minimize digital peak\n");
-			report_channels (r, vfd);
+			report_channels (res, vfd);
 		}
+	}
+
+	if (opt.loudness) {
+		// BS.1770-4 integrated loudness of the input (set 0: angle 0) and of the --fixed-write render at the
+		// applied angles (set 1), and the peak-to-loudness ratios with the peaks of the result lines
+		std::vector<int> sets ((size_t)2 * C, 0);
+		std::copy (angles.begin (), angles.end (), sets.begin () + C);
+		std::vector<float> w ((size_t)C, 1.f);
+		if (C == 6) {
+			w = { 1.f, 1.f, 1.f, 0.f, 1.41f, 1.41f }; // BS.1770 5.1 weights, WAV order L R C LFE Ls Rs
+		}
+		double lufs[2] = { -std::numeric_limits<double>::infinity (), -std::numeric_limits<double>::infinity () };
+		if (F > 0) {
+			check (phaserot_loudness (pr, audio, pcm_fmt, F, (double)nfo.samplerate, w.data (), sets.data (), 2, lufs), "loudness failed");
+		}
+		float pk_in = 0.f, pk_out = 0.f;
+		for (int c = 0; c < C; ++c) {
+			pk_in  = std::max (pk_in, res.r_zro[(size_t)c]);
+			pk_out = std::max (pk_out, res.p_min[(size_t)c] == std::numeric_limits<float>::infinity () ? res.r_zro[(size_t)c] : res.r_min[(size_t)c]);
+		}
+		printf ("# Loudness -- ITU-R BS.1770-4 integrated\n");
+		printf ("Input : %.2f LUFS, PLR %.2f dB\n", lufs[0], to_dB (pk_in) - lufs[0]);
+		printf ("Output: %.2f LUFS, PLR %.2f dB\n", lufs[1], to_dB (pk_out) - lufs[1]);
+		timer.mark ("loudness");
 	}
 
 	if (outfile) {
