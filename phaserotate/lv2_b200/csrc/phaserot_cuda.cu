@@ -175,6 +175,39 @@ struct PluginChan {
 	float2              last_const   = make_float2 (1.f, 0.f);
 };
 
+// One analysis pass over a stream (sweep_core)
+struct SweepJob {
+	const void*  src         = nullptr;          // interleaved frames (host or device)
+	bool         on_device   = false;            // src is device memory (float32)
+	int          fmt         = PHASEROT_PCM_F32; // host src: PHASEROT_PCM_*
+	long long    n_frames    = 0;                // frames present in src
+	long long    t_end       = 0;                // the pass examines output samples t in [0, t_end)
+	bool         first_block = false;            // apply the first-block rule (cli:418-419) to t < L
+	const float* hist        = nullptr;          // L frames of history preceding src (interleaved) or null
+	int          ang_start = 0, ang_end = 0, ang_stride = 1, chn = -1;
+};
+
+// The pass over F frames that are a whole stream (first and last) or one shard of it: the last shard ends with
+// one zero flush block (analyze_file, cli:572-586), and the first-block rule applies to the first shard
+SweepJob
+shard_job (int L, const void* src, bool on_device, int fmt, long long F, const float* hist, bool first, bool last, int ang_start, int ang_end,
+           int ang_stride, int chn)
+{
+	const long long B = (F + L - 1) / L;
+	return { src, on_device, fmt, F, last ? (B + 1) * L : F, first && B > 0, hist, ang_start, ang_end, ang_stride, chn };
+}
+
+// d_small: per-channel state of the pending sweep and the render
+struct SmallState {
+	unsigned           count[64];
+	float              thr2[64];
+	int                ramp_len[64];
+	unsigned long long stats[3]; // points listed in dense mode, evaluated points, overflow word of bootstrap launches (nobody reads it)
+	unsigned           count_odd[64]; // list counts of odd launches
+	unsigned           r2max[64];
+	unsigned           wide_count[64];
+};
+
 } // namespace
 
 struct phaserot {
@@ -202,21 +235,14 @@ struct phaserot {
 
 	DevBuf d_G, d_G1, d_scratch, d_tw, d_g;
 	DevBuf d_plane, d_out, d_list, d_stage[2], d_io, d_inter, d_hist;
-	DevBuf d_small; // count[C] | thr2[C] | raw[C] | ramp_len[C] | stats[2 x u64]
+	DevBuf d_small; // SmallState
 	DevBuf d_cs, d_peaks, d_ramp, d_chancs;
 	// dense mode (long survivor lists, see sweep_window_kernel): grid index -> slot, sector thresholds, wide list
 	DevBuf d_slot, d_sec, d_wide;
 	PinBuf h_slot;
 	bool      dense_mode  = false; // sticky: the last sweep overflowed its survivor list (few-tone / constant-envelope material)
 	long long list_cap    = 0;     // points per channel the list holds
-	// what the pending sweep ran over, for a dense-mode repeat from finish_pending() (device pointers)
-	struct Redo {
-		const float* src = nullptr;
-		long long    n_frames = 0, t_end = 0;
-		bool         first_block = false;
-		const float* hist = nullptr;
-		int          ang_start = 0, ang_end = 0, ang_stride = 1, chn = -1;
-	} redo;
+	SweepJob  redo;                // the pending sweep in device-resident form, for a dense-mode repeat or a resume
 	uint64_t pend_points = 0; // points examined by the pending sweep (statistics; dense-mode exit test)
 	int      pend_again   = 0;     // PHASEROT_E_AGAIN returned for the pending sweep so far
 	bool     pend_exposed = false; // the pending table was handed out (phaserot_pending_table): the caller combines shards
@@ -296,9 +322,7 @@ struct DevGuard {
 	}
 };
 
-// d_small: count[64] | thr2[64] | raw[64] | ramp_len[64] | stats[2 x u64] | count of odd launches[64] | r2max[64]
-// ... | stats[3 x u64: points listed in dense mode, evaluated points, list overflow flag] | count of odd launches[64] | r2max[64] | wide list count[64]
-constexpr size_t kSmallBytes = 7 * 64 * sizeof (int) + 3 * sizeof (unsigned long long);
+constexpr size_t kSmallBytes = sizeof (SmallState);
 struct ProfScope {
 	phaserot* h;
 	size_t    slot = (size_t)-1;
@@ -339,21 +363,22 @@ prof_resolve (phaserot* h)
 	h->prof_used = 0;
 }
 
-unsigned*           d_count (phaserot* h) { return (unsigned*)h->d_small.p; }
-float*              d_thr2 (phaserot* h) { return (float*)h->d_small.p + 64; }
+SmallState*         d_small (phaserot* h) { return (SmallState*)h->d_small.p; }
+unsigned*           d_count (phaserot* h) { return d_small (h)->count; }
+float*              d_thr2 (phaserot* h) { return d_small (h)->thr2; }
 // raw input peaks [C]: directly behind the [C][A] table of the pending sweep, so that table and
 // raw peaks are one contiguous buffer (one D2H copy, one all-reduce when shards are combined)
 unsigned*           d_raw (phaserot* h) { return (unsigned*)h->d_peaks.p + (size_t)std::max (h->pend_A, 1) * h->C; }
-int*                d_ramplen (phaserot* h) { return (int*)h->d_small.p + 192; }
-unsigned long long* d_stats (phaserot* h) { return (unsigned long long*)((char*)h->d_small.p + 4 * 64 * sizeof (int)); }
+int*                d_ramplen (phaserot* h) { return d_small (h)->ramp_len; }
+unsigned long long* d_stats (phaserot* h) { return d_small (h)->stats; }
 // List-overflow flag of the pending sweep: the word behind the raw peaks, i.e. the LAST element of the
 // device table (bits of 1.0f when set).  It travels with the table through an external max all-reduce, so
 // every rank of a sharded sweep learns that some shard is incomplete without a second collective.
 unsigned*           d_overflow (phaserot* h) { return d_raw (h) + h->C; }
-unsigned*           d_overflow_ignored (phaserot* h) { return (unsigned*)(d_stats (h) + 2); } // bootstrap launches: nobody reads it
-unsigned*           d_count_odd (phaserot* h) { return (unsigned*)((char*)h->d_small.p + 4 * 64 * sizeof (int) + 3 * sizeof (unsigned long long)); }
-unsigned*           d_r2max (phaserot* h) { return d_count_odd (h) + 64; }
-unsigned*           d_wide_count (phaserot* h) { return d_r2max (h) + 64; }
+unsigned*           d_overflow_ignored (phaserot* h) { return (unsigned*)&d_small (h)->stats[2]; }
+unsigned*           d_count_odd (phaserot* h) { return d_small (h)->count_odd; }
+unsigned*           d_r2max (phaserot* h) { return d_small (h)->r2max; }
+unsigned*           d_wide_count (phaserot* h) { return d_small (h)->wide_count; }
 
 int
 upload_tables (phaserot* h)
@@ -429,33 +454,48 @@ set_conv_attr ()
 // Only the kernels a handle of this shape can launch are touched: setting an
 // attribute loads the kernel's code (CUDA loads modules lazily), and a CLI run on
 // a 48 kHz file needs three of the twenty-odd kernels in the library - the rest
-// would only add to the process start-up time.
+// would only add to the process start-up time.  Sections and loudness ask for
+// theirs when they are first called (phaserot_create() does not know whether they
+// will be).
 enum {
-	KA_POINTS = 1 << 0, KA_RENDER_INTER = 1 << 1, KA_RENDER_PLANE = 1 << 2, KA_HILBERT = 1 << 3, // x 2 tap partitions: shifted by 4
+	KA_POINTS = 1 << 0, KA_RENDER_INTER = 1 << 1, KA_RENDER_PLANE = 1 << 2, KA_HILBERT = 1 << 3, KA_SECT_POINTS = 1 << 4, KA_SECT_RENDER = 1 << 5,
 	KA_FIR_STREAM = 1 << 8
 };
+// `want`: KA_* bits; the fftconv_kernel bits (the low byte) stand for the instantiation with the handle's NP.
+// Caller holds g_create_lock and has made `dev` current.
 int
-set_device_attrs (int dev, bool plugin, int NP, int OS) // caller holds g_create_lock and has made `dev` current
+set_device_attrs (int dev, int NP, unsigned want)
 {
-	static std::vector<unsigned> done;
+	static std::vector<unsigned> done; // per device; fftconv_kernel bits of NP = 2 are shifted by 16
 	if (done.size () <= (size_t)dev) done.resize ((size_t)dev + 1, 0u);
-	unsigned want = plugin ? (KA_RENDER_PLANE | KA_FIR_STREAM) : (KA_RENDER_INTER | (OS > 1 ? KA_HILBERT : KA_POINTS));
-	if (NP == 2) want = ((want & 0xf) << 4) | (want & ~0xffu);
+	if (NP == 2) want = ((want & 0xffu) << 16) | (want & ~0xffu);
 	const unsigned todo = want & ~done[(size_t)dev];
 	int rc;
 	if ((todo & KA_POINTS) && (rc = set_conv_attr<EPI_POINTS, SRC_INTER, 1> ())) return rc;
-	if ((todo & (KA_POINTS << 4)) && (rc = set_conv_attr<EPI_POINTS, SRC_INTER, 2> ())) return rc;
+	if ((todo & (KA_POINTS << 16)) && (rc = set_conv_attr<EPI_POINTS, SRC_INTER, 2> ())) return rc;
 	if ((todo & KA_RENDER_INTER) && (rc = set_conv_attr<EPI_RENDER, SRC_INTER, 1> ())) return rc;
-	if ((todo & (KA_RENDER_INTER << 4)) && (rc = set_conv_attr<EPI_RENDER, SRC_INTER, 2> ())) return rc;
+	if ((todo & (KA_RENDER_INTER << 16)) && (rc = set_conv_attr<EPI_RENDER, SRC_INTER, 2> ())) return rc;
 	if ((todo & KA_RENDER_PLANE) && (rc = set_conv_attr<EPI_RENDER, SRC_PLANE, 1> ())) return rc;
-	if ((todo & (KA_RENDER_PLANE << 4)) && (rc = set_conv_attr<EPI_RENDER, SRC_PLANE, 2> ())) return rc;
+	if ((todo & (KA_RENDER_PLANE << 16)) && (rc = set_conv_attr<EPI_RENDER, SRC_PLANE, 2> ())) return rc;
 	if ((todo & KA_HILBERT) && (rc = set_conv_attr<EPI_HILBERT, SRC_INTER, 1> ())) return rc;
-	if ((todo & (KA_HILBERT << 4)) && (rc = set_conv_attr<EPI_HILBERT, SRC_INTER, 2> ())) return rc;
+	if ((todo & (KA_HILBERT << 16)) && (rc = set_conv_attr<EPI_HILBERT, SRC_INTER, 2> ())) return rc;
+	if ((todo & KA_SECT_POINTS) && (rc = set_conv_attr<EPI_SECT_POINTS, SRC_INTER, 1> ())) return rc;
+	if ((todo & (KA_SECT_POINTS << 16)) && (rc = set_conv_attr<EPI_SECT_POINTS, SRC_INTER, 2> ())) return rc;
+	if ((todo & KA_SECT_RENDER) && (rc = set_conv_attr<EPI_SECT_RENDER, SRC_INTER, 1> ())) return rc;
+	if ((todo & (KA_SECT_RENDER << 16)) && (rc = set_conv_attr<EPI_SECT_RENDER, SRC_INTER, 2> ())) return rc;
 	if (todo & KA_FIR_STREAM) {
 		CK (cudaFuncSetAttribute (fir_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
 	}
 	done[(size_t)dev] |= want;
 	return PHASEROT_OK;
+}
+
+// the same from a call that has not taken g_create_lock (sections, loudness: never a plugin run())
+int
+load_kernels (phaserot* h, unsigned want)
+{
+	std::lock_guard<std::mutex> lk (g_create_lock);
+	return set_device_attrs (h->dev, h->NP, want);
 }
 
 template <int EPI, int SRC, int NP>
@@ -570,38 +610,72 @@ pick_sweep_cfg (int A)
 	return best;
 }
 
+// Every angle of d_cs over the survivor lists of `rows` rows from row0 on (list, count: [row]), into
+// table [row][A] with a running max.  A bootstrap list is swept even when its count ran past cap (the
+// excess was dropped); any other flagged row is repeated in dense mode, so its full list is skipped.
 int
-launch_sweep (phaserot* h, int A, int c0, int nchan, const unsigned* count, const float2* lst = nullptr, unsigned cap = 0, bool boot = false)
+launch_sweep (phaserot* h, const float2* lst, long long list_stride, const unsigned* count, unsigned cap, bool boot, int row0, int rows, int A,
+              unsigned* table, unsigned long long* n_eval)
 {
-	const SweepCfg sc = pick_sweep_cfg (A);
-	int gx = (h->n_sm * 8) / std::max (1, sc.gy * nchan);
-	gx     = std::max (gx, 1);
-	const dim3 grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)nchan);
-	if (!lst) lst = (const float2*)h->d_list.p;
-	if (!cap) cap = (unsigned)h->list_cap;
-	const float2*       cs  = (const float2*)h->d_cs.p;
-	unsigned*           pk  = (unsigned*)h->d_peaks.p;
-	unsigned long long* ne  = d_stats (h) + 1;
-	ProfScope           ps (h, 1);
+	if (A == 0) return PHASEROT_OK;
+	const SweepCfg  sc = pick_sweep_cfg (A);
+	const long long gx = std::max<long long> (1, (h->n_sm * 8) / std::max<long long> (1, (long long)sc.gy * rows));
+	const dim3      grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)rows);
+	const float2*   cs = (const float2*)h->d_cs.p;
+	const int       so = boot ? 0 : 1;
+	ProfScope       ps (h, 1);
 	switch (sc.R) {
-		case 1: sweep_kernel<1><<<grid, sc.nt, 0, h->stream>>> (lst, h->list_stride, count, cap, boot ? 0 : 1, c0, cs, A, pk, h->pend_A, ne); break;
-		case 2: sweep_kernel<2><<<grid, sc.nt, 0, h->stream>>> (lst, h->list_stride, count, cap, boot ? 0 : 1, c0, cs, A, pk, h->pend_A, ne); break;
-		case 4: sweep_kernel<4><<<grid, sc.nt, 0, h->stream>>> (lst, h->list_stride, count, cap, boot ? 0 : 1, c0, cs, A, pk, h->pend_A, ne); break;
-		default: sweep_kernel<8><<<grid, sc.nt, 0, h->stream>>> (lst, h->list_stride, count, cap, boot ? 0 : 1, c0, cs, A, pk, h->pend_A, ne); break;
+		case 1: sweep_kernel<1><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
+		case 2: sweep_kernel<2><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
+		case 4: sweep_kernel<4><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
+		default: sweep_kernel<8><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
 	}
 	CK (cudaGetLastError ());
 	++h->stats.kernel_launches;
 	return PHASEROT_OK;
 }
 
-int sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frames, long long t_end, bool first_block, const float* hist,
-                int ang_start, int ang_end, int ang_stride, int chn, int fmt, bool redo, bool boot_only);
+// Contiguous launches of a sweep: the first has PHASEROT_SEGS_FIRST segments per CTA, the following ones up to
+// PHASEROT_SEGS_MULT times that (measurement aids, defaults 8 and 16)
+struct SegsKnobs {
+	int first = getenv ("PHASEROT_SEGS_FIRST") ? std::max (1, atoi (getenv ("PHASEROT_SEGS_FIRST"))) : 8;
+	int mult  = getenv ("PHASEROT_SEGS_MULT") ? std::max (1, atoi (getenv ("PHASEROT_SEGS_MULT"))) : 16;
+};
+
+// Segments per channel of the next contiguous launch (n_main launches so far, seg_done of nseg segments done).
+// The first launch has segs_first as a refresh of the radius - unless what would be left for the second
+// launch is less than that and `merge_short_rest` (short streams, shards of a strong-scaling run): then
+// everything goes into one launch and a launch + sweep round trip (~35 us) is saved.
+long long
+next_launch_segs (int n_main, long long seg_done, long long nseg, long long segs_first, long long segs_max, bool merge_short_rest)
+{
+	const bool short_rest = merge_short_rest && nseg - seg_done <= 2 * segs_first;
+	return (n_main == 0 && !short_rest) ? segs_first : segs_max;
+}
+
+enum class Pass {
+	Fresh,    // a new pass: the pending one is finished first, the device table starts empty, bootstrap included
+	BootOnly, // Fresh, but only the bootstrap wave and its sweep are enqueued (two-phase sharded sweep)
+	Continue, // the pending pass again, on its device table without a bootstrap: dense-mode repeat, or the rest of BootOnly
+};
+int sweep_core (phaserot* h, SweepJob job, Pass pass);
+
+// Repeats the pending sweep in dense mode on top of the table reached so far (a running maximum only
+// grows, and every point evaluated was a real one).  Dense launches are sized to the list, so the repeat
+// cannot overflow.  `evaluated`: points the overflowed attempt evaluated.
+int
+repeat_dense (phaserot* h, unsigned long long evaluated)
+{
+	h->stats.points_evaluated += evaluated;
+	h->dense_mode  = true;
+	h->pend_redone = true;
+	++h->stats.dense_repeats;
+	return sweep_core (h, h->redo, Pass::Continue);
+}
 
 // The pending sweep is complete on the device when this returns: waits for it and,
 // if a survivor list overflowed (material where most samples survive the radius
-// filter), repeats the pass in dense mode on top of the table reached so far (a
-// running maximum only grows, and every point evaluated was a real one).  Dense
-// launches are sized to the list, so the repeat cannot overflow.
+// filter), repeats the pass in dense mode.
 int
 complete_pending (phaserot* h)
 {
@@ -626,15 +700,22 @@ complete_pending (phaserot* h)
 			snprintf (g_last_error, sizeof (g_last_error), "survivor list overflow in dense mode");
 			return PHASEROT_E_CUDA; // cannot happen: dense launches are sized to the list
 		}
-		h->stats.points_evaluated += st[1];
-		h->dense_mode  = true;
-		h->pend_redone = true;
-		++h->stats.dense_repeats;
-		const phaserot::Redo r = h->redo;
-		rc = sweep_core (h, r.src, true, r.n_frames, r.t_end, r.first_block, r.hist, r.ang_start, r.ang_end, r.ang_stride, r.chn, PHASEROT_PCM_F32, true, false);
+		rc = repeat_dense (h, st[1]);
 		if (rc) return rc;
 	}
 	return PHASEROT_OK;
+}
+
+// Running max of one row of a device sweep table (maxima in the order of the angle schedule idx) into a
+// row of the host grid (PhaseRotate::_peak).  Grid index 0 also takes the raw input peak, if any.
+void
+merge_row (float* row, const float* tab, const std::vector<int>& idx, const float* raw)
+{
+	for (size_t k = 0; k < idx.size (); ++k) {
+		const int a = idx[k];
+		row[a]      = std::max (row[a], tab[k]);
+	}
+	if (raw) row[0] = std::max (row[0], *raw);
 }
 
 // merge a finished device sweep into the host table (PhaseRotate::_peak semantics: running max)
@@ -683,28 +764,13 @@ finish_pending (phaserot* h)
 			CK (cudaMemsetAsync (d_overflow (h), 0, sizeof (unsigned), h->stream));
 			return PHASEROT_E_AGAIN;
 		}
-		h->stats.points_evaluated += st[1];
-		h->dense_mode  = true;
-		h->pend_redone = true;
-		++h->stats.dense_repeats;
-		const phaserot::Redo r = h->redo;
-		rc = sweep_core (h, r.src, true, r.n_frames, r.t_end, r.first_block, r.hist, r.ang_start, r.ang_end, r.ang_stride, r.chn, PHASEROT_PCM_F32, true, false);
+		rc = repeat_dense (h, st[1]);
 		if (rc) return rc;
 		return PHASEROT_E_AGAIN;
 	}
+	const float* tab = (const float*)res; // float bits
 	for (int c = h->pend_c0; c < h->pend_c1; ++c) {
-		float* row = h->table.data () + (size_t)c * h->MS;
-		for (int k = 0; k < A; ++k) {
-			float v;
-			memcpy (&v, &res[(size_t)c * A + k], sizeof (float));
-			const int a = h->pend_idx[(size_t)k];
-			row[a]      = std::max (row[a], v);
-		}
-		if (h->pend_raw) {
-			float v;
-			memcpy (&v, &res[(size_t)A * h->C + c], sizeof (float));
-			row[0] = std::max (row[0], v);
-		}
+		merge_row (h->table.data () + (size_t)c * h->MS, tab + (size_t)c * A, h->pend_idx, h->pend_raw ? tab + (size_t)A * h->C + c : nullptr);
 	}
 	h->stats.points_evaluated += st[1];
 	if (getenv ("PHASEROT_DEBUG")) {
@@ -757,16 +823,51 @@ angle_schedule (phaserot* h, int ang_start, int ang_end, int ang_stride, std::ve
 	return PHASEROT_OK;
 }
 
+// bytes per sample of a host stream in PHASEROT_PCM_* format
+size_t
+pcm_bytes (int fmt)
+{
+	return fmt == PHASEROT_PCM_S16 ? 2 : fmt == PHASEROT_PCM_S24 ? 3 : 4;
+}
+
+// (cos, sin) of every angle of the schedule to d_cs, staged through a pinned buffer of the handle: no
+// synchronisation (the caller has waited for the stream's previous pass)
+int
+upload_angle_table (phaserot* h, const std::vector<int>& idx)
+{
+	const size_t n  = std::max<size_t> (idx.size (), 1);
+	int          rc = h->d_cs.ensure (sizeof (float2) * n);
+	if (rc) return rc;
+	rc = h->h_cs.ensure (sizeof (float2) * n);
+	if (rc) return rc;
+	float2* cs = (float2*)h->h_cs.p;
+	for (size_t k = 0; k < idx.size (); ++k) cs[k] = make_float2 (h->lut_c[(size_t)idx[k]], h->lut_s[(size_t)idx[k]]);
+	CK (cudaMemcpyAsync (h->d_cs.p, cs, sizeof (float2) * idx.size (), cudaMemcpyHostToDevice, h->stream));
+	return PHASEROT_OK;
+}
+
+// (cos, sin) of a full-circle angle a: a + MS renders the negation of a, so it is the LUT pair of
+// a mod MS, negated for odd half turns
+float2
+full_circle_cs (const phaserot* h, long long a)
+{
+	const long long q  = (a >= 0 ? a : a - h->MS + 1) / h->MS;
+	const size_t    i  = (size_t)(a - q * h->MS);
+	const float     sg = (q & 1) ? -1.f : 1.f;
+	return make_float2 (sg * h->lut_c[i], sg * h->lut_s[i]);
+}
+
 // H2D of a host stream into d_inter (allocated by the caller) in chunks on the copy stream, integer PCM
 // widened there; the compute stream waits for each chunk, and `landed (frames)` runs after every chunk
 // but the last, so that the caller can start on the frames that have landed.
 template <class Landed>
 int
-upload_chunks (phaserot* h, const void* src, int pcm_bytes, long long n_frames, Landed&& landed)
+upload_chunks (phaserot* h, const void* src, int fmt, long long n_frames, Landed&& landed)
 {
 	int rc = PHASEROT_OK;
 	const long long chunk_frames = std::max<long long> (4, ((8LL << 20) / h->C) & ~3LL); // ~32 MB of floats per chunk; a multiple of 4 frames keeps every chunk 4-byte aligned at 3 bytes per sample
-	const size_t    bps          = pcm_bytes ? (size_t)pcm_bytes : sizeof (float);      // bytes per sample on the host side
+	const size_t    bps          = pcm_bytes (fmt);
+	const bool      widen        = fmt != PHASEROT_PCM_F32; // integer PCM: conversion pass on the copy stream
 	cudaPointerAttributes at;
 	const bool pinned = (cudaPointerGetAttributes (&at, src) == cudaSuccess) && (at.type == cudaMemoryTypeHost);
 	cudaGetLastError ();
@@ -776,7 +877,7 @@ upload_chunks (phaserot* h, const void* src, int pcm_bytes, long long n_frames, 
 			if (rc) return rc;
 		}
 	}
-	if (pcm_bytes) {
+	if (widen) {
 		// integer PCM: raw chunk -> device staging -> pcm_to_float_kernel on the copy
 		// stream -> the float copy of the file; staging buffer b is reused two chunks
 		// later on the same stream, i.e. after the kernel that read it
@@ -803,13 +904,13 @@ upload_chunks (phaserot* h, const void* src, int pcm_bytes, long long n_frames, 
 			hsrc = h->h_stage[b].p;
 		}
 		float* d_chunk = (float*)h->d_inter.p + (size_t)f0 * h->C;
-		if (pcm_bytes) {
+		if (widen) {
 			CK (cudaMemcpyAsync (h->d_stage[b].p, hsrc, bytes, cudaMemcpyHostToDevice, h->copy_stream));
 			const long long ns = nf * h->C;
 			const unsigned  nb = (unsigned)((ns + 1023) / 1024);
-			if (pcm_bytes == 2) {
+			if (fmt == PHASEROT_PCM_S16) {
 				pcm_to_float_kernel<int16_t><<<nb, 256, 0, h->copy_stream>>> ((const int16_t*)h->d_stage[b].p, d_chunk, ns);
-			} else if (pcm_bytes == 3) {
+			} else if (fmt == PHASEROT_PCM_S24) {
 				pcm24_to_float_kernel<<<nb, 256, 0, h->copy_stream>>> ((const uint8_t*)h->d_stage[b].p, d_chunk, ns);
 			} else {
 				pcm_to_float_kernel<int32_t><<<nb, 256, 0, h->copy_stream>>> ((const int32_t*)h->d_stage[b].p, d_chunk, ns);
@@ -833,51 +934,29 @@ upload_chunks (phaserot* h, const void* src, int pcm_bytes, long long n_frames, 
 	return PHASEROT_OK;
 }
 
-/*
- * One analysis pass over a stream.
- *   src          interleaved frames (host or device)
- *   n_frames     frames present in src
- *   t_end        the pass examines output samples t in [0, t_end)
- *   first_block  apply the first-block rule (cli:418-419) to t < L
- *   hist         L frames of history preceding src (host, interleaved) or null
- */
+// One analysis pass over a stream (see SweepJob and Pass).
 int
-sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frames, long long t_end, bool first_block,
-            const float* hist, int ang_start, int ang_end, int ang_stride, int chn, int fmt = PHASEROT_PCM_F32 /* host src: PHASEROT_PCM_* */,
-            bool redo = false /* repeat / continuation of the pending sweep: keep the device table, no bootstrap */,
-            bool boot_only = false /* enqueue the bootstrap wave and its sweep only (two-phase sharded sweep) */)
+sweep_core (phaserot* h, SweepJob job, Pass pass)
 {
-	// bytes per sample on the host side (and on the bus); 0 = float32, no conversion pass
-	const int pcm_bytes = fmt == PHASEROT_PCM_S16 ? 2 : fmt == PHASEROT_PCM_S32 ? 4 : fmt == PHASEROT_PCM_S24 ? 3 : 0;
-	if (chn >= h->C) {
+	const bool redo = pass == Pass::Continue;
+	if (job.chn >= h->C) {
 		return PHASEROT_E_INVAL;
 	}
-	int rc = redo ? PHASEROT_OK : finish_pending (h);
+	int rc = redo ? PHASEROT_OK : finish_pending (h); // (the stream is then idle with respect to the previous pass)
 	if (rc) return rc;
 
 	std::vector<int> idx;
 	bool             raw = false;
-	rc                   = angle_schedule (h, ang_start, ang_end, ang_stride, idx, raw);
+	rc                   = angle_schedule (h, job.ang_start, job.ang_end, job.ang_stride, idx, raw);
 	if (rc) return rc;
 	const int A  = (int)idx.size ();
-	const int c0 = chn < 0 ? 0 : chn;
-	const int c1 = chn < 0 ? h->C : chn + 1;
+	const int c0 = job.chn < 0 ? 0 : job.chn;
+	const int c1 = job.chn < 0 ? h->C : job.chn + 1;
 
-	// angle table
-	std::vector<float2> cs ((size_t)std::max (A, 1));
-	for (int k = 0; k < A; ++k) {
-		cs[(size_t)k] = make_float2 (h->lut_c[(size_t)idx[(size_t)k]], h->lut_s[(size_t)idx[(size_t)k]]);
-	}
-	rc = h->d_cs.ensure (sizeof (float2) * cs.size ());
-	if (rc) return rc;
 	rc = h->d_peaks.ensure (sizeof (unsigned) * ((size_t)std::max (A, 1) * h->C + (size_t)h->C + 1));
 	if (rc) return rc;
-	// staged through a pinned buffer of the handle: no synchronisation (the stream is
-	// idle with respect to the previous pass: finish_pending() above waited for it)
-	rc = h->h_cs.ensure (sizeof (float2) * cs.size ());
+	rc = upload_angle_table (h, idx);
 	if (rc) return rc;
-	memcpy (h->h_cs.p, cs.data (), sizeof (float2) * cs.size ());
-	CK (cudaMemcpyAsync (h->d_cs.p, h->h_cs.p, sizeof (float2) * cs.size (), cudaMemcpyHostToDevice, h->stream));
 	h->pend_A = A; // d_raw() depends on it
 	if (!redo) {
 		CK (cudaMemsetAsync (h->d_peaks.p, 0, sizeof (unsigned) * ((size_t)std::max (A, 1) * h->C + (size_t)h->C + 1), h->stream));
@@ -901,10 +980,10 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		CK (cudaMemcpyAsync (h->d_slot.p, so, sizeof (int) * (size_t)h->MS, cudaMemcpyHostToDevice, h->stream));
 	}
 
-	const long long m_end = (t_end + 1) / 2;
+	const long long m_end = (job.t_end + 1) / 2;
 	const long long nseg  = (m_end + h->V - 1) / h->V;
 	const float*    d_hist = nullptr;
-	if (hist) {
+	if (const float* hist = job.hist) {
 		// frames [-L, 0) of the stream, read by the segments that reach before its start
 		cudaPointerAttributes at;
 		const bool on_device = cudaPointerGetAttributes (&at, hist) == cudaSuccess && at.type == cudaMemoryTypeDevice;
@@ -930,12 +1009,9 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 	// has landed.)
 	const int       OS         = h->OS;
 	const long long ppseg      = (long long)h->V * 2 * (OS > 1 ? OS + 1 : 1); // points a segment can put on the list (true-peak: the sample and OS interpolated points)
-	// (PHASEROT_SEGS_FIRST = segments per CTA of the first contiguous launch, PHASEROT_SEGS_MULT = size of the
-	// following launches in units of it: measurement aids, defaults 8 and 16)
-	static const int k_first = getenv ("PHASEROT_SEGS_FIRST") ? std::max (1, atoi (getenv ("PHASEROT_SEGS_FIRST"))) : 8;
-	static const int k_mult  = getenv ("PHASEROT_SEGS_MULT") ? std::max (1, atoi (getenv ("PHASEROT_SEGS_MULT"))) : 16;
-	long long       segs_first = std::max<long long> (1, ((long long)h->n_sm * k_first) / nchan);
-	long long       segs_max   = !src_is_device ? segs_first : (OS_is_digital (h) ? k_mult : 2) * segs_first;
+	static const SegsKnobs knobs;
+	long long       segs_first = std::max<long long> (1, ((long long)h->n_sm * knobs.first) / nchan);
+	long long       segs_max   = !job.on_device ? segs_first : (OS_is_digital (h) ? knobs.mult : 2) * segs_first;
 	// Survivor list, sized by demand.  Normal mode: 1/32 of the points of the
 	// largest launch (pruning leaves 1e-4 .. 1e-5 of them on programme material), at
 	// least 1 M points per channel; a list that overflows flags the pass and
@@ -983,13 +1059,13 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 	ConvParams p;
 	fill_conv_common (h, p);
 	p.hist     = d_hist;
-	p.n_frames = n_frames;
+	p.n_frames = job.n_frames;
 	p.C        = h->C;
 	p.chan0  = c0;
 	p.nchan  = nchan;
 	p.m_end  = m_end;
-	p.m_skip = (first_block && !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK)) ? h->Lh / 2 : 0;
-	p.m_zero = (first_block && !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK)) ? h->Lh : 0;
+	p.m_skip = (job.first_block && !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK)) ? h->Lh / 2 : 0;
+	p.m_zero = (job.first_block && !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK)) ? h->Lh : 0;
 	p.list        = (float2*)h->d_list.p;
 	p.list_stride = h->list_stride;
 	p.count       = d_count (h);
@@ -1030,7 +1106,7 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		p.out_stride  = h->tp_stride / 2;
 		p.out_compact = 1;
 		tp.hist        = d_hist;
-		tp.n_frames    = n_frames;
+		tp.n_frames    = job.n_frames;
 		tp.C           = h->C;
 		tp.hist_frames = h->L;
 		tp.H           = (const float*)h->d_tpH.p;
@@ -1040,7 +1116,7 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		tp.D           = h->L / 2;
 		tp.t_skip      = 2 * p.m_skip;
 		tp.t_zero      = 2 * p.m_zero;
-		tp.t_end       = t_end;
+		tp.t_end       = job.t_end;
 		tp.os          = OS;
 		tp.list        = p.list;
 		tp.list_stride = p.list_stride;
@@ -1063,17 +1139,20 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 	// every angle over the survivors of one launch.  Normal mode: angles in lanes over the
 	// (short) list.  Dense mode: sector thresholds, then one thread per point over the few
 	// angles it can still raise (sweep_window_kernel); what that leaves goes angles-in-lanes.
+	const float2*       lst    = (const float2*)h->d_list.p;
+	unsigned*           table  = (unsigned*)h->d_peaks.p;
+	unsigned long long* n_eval = d_stats (h) + 1;
 	auto sweep_survivors = [&] (const unsigned* count, unsigned cap, bool boot) -> int {
 		if (A == 0) return PHASEROT_OK;
 		if (!dense || no_prune || (boot && !h->dense_mode)) {
-			return launch_sweep (h, A, c0, nchan, count, nullptr, cap, boot);
+			return launch_sweep (h, lst, h->list_stride, count, cap, boot, c0, nchan, A, table, n_eval);
 		}
 		if (boot) {
 			// Bootstrap list of a dense handle (up to 1 M points per channel, 0.46 ms at every angle): the running
 			// peaks are still zero and every window would be the whole grid, so the head of the list is swept at
 			// every angle - and the whole list then goes through the windows like any other, against that table.
 			static const unsigned kBootBrute = getenv ("PHASEROT_BOOT_BRUTE") ? (unsigned)atoi (getenv ("PHASEROT_BOOT_BRUTE")) : 128u << 10;
-			const int          r          = launch_sweep (h, A, c0, nchan, count, nullptr, std::min (cap, kBootBrute), boot);
+			const int          r          = launch_sweep (h, lst, h->list_stride, count, std::min (cap, kBootBrute), boot, c0, nchan, A, table, n_eval);
 			if (r) return r;
 		}
 		CK (cudaMemsetAsync (d_wide_count (h), 0, sizeof (unsigned) * 64, h->stream));
@@ -1129,7 +1208,7 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		}
 		CK (cudaGetLastError ());
 		h->stats.kernel_launches += 2;
-		return launch_sweep (h, A, c0, nchan, d_wide_count (h), (const float2*)h->d_wide.p, cap);
+		return launch_sweep (h, (const float2*)h->d_wide.p, h->list_stride, d_wide_count (h), cap, false, c0, nchan, A, table, n_eval);
 	};
 
 	// one conv launch + sweep of its survivors + new filter radius
@@ -1222,12 +1301,8 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 			if (r) return r;
 			booted = true;
 		}
-		while (!boot_only && seg_done < seg_ready) {
-			// first contiguous launch: 8 segments per CTA as a refresh of the radius - unless what would be
-			// left for the second launch is less than that (short streams, shards of a strong-scaling run):
-			// then everything goes into one launch and a launch + sweep round trip (~35 us) is saved
-			const bool      short_rest = src_is_device && final && nseg - seg_done <= 2 * segs_first;
-			const long long want       = !booted ? wave : ((n_main == 0 && !short_rest) ? segs_first : segs_max);
+		while (pass != Pass::BootOnly && seg_done < seg_ready) {
+			const long long want = !booted ? wave : next_launch_segs (n_main, seg_done, nseg, segs_first, segs_max, job.on_device && final);
 			const long long n    = std::min (want, seg_ready - seg_done);
 			if (!final && n < want && seg_ready < nseg) {
 				break; // wait for more data to keep launches full
@@ -1241,9 +1316,9 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		return PHASEROT_OK;
 	};
 
-	if (src_is_device) {
-		p.inter      = src;
-		frames_ready = n_frames;
+	if (job.on_device) {
+		p.inter      = (const float*)job.src;
+		frames_ready = job.n_frames;
 		rc           = tp_head ();
 		if (rc) return rc;
 		rc           = process_ready (true);
@@ -1251,12 +1326,12 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 	} else {
 		// H2D in chunks on the copy stream straight into the device copy of the
 		// file; the compute stream starts on a chunk as soon as it has landed
-		rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)n_frames * h->C, 16));
+		rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)job.n_frames * h->C, 16));
 		if (rc) return rc;
 		p.inter = (const float*)h->d_inter.p;
 		rc      = tp_head ();
 		if (rc) return rc;
-		rc = upload_chunks (h, src, pcm_bytes, n_frames, [&] (long long f) {
+		rc = upload_chunks (h, job.src, job.fmt, job.n_frames, [&] (long long f) {
 			frames_ready = f;
 			return process_ready (false);
 		});
@@ -1270,16 +1345,12 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 		h->pend_redone  = false;
 		h->pend_points = (uint64_t)nchan * (uint64_t)(2 * (m_end - p.m_skip)) * (uint64_t)(OS > 1 ? OS + 1 : 1);
 		h->stats.points_total += h->pend_points;
-		// the device-resident form of this pass, should complete_pending() have to repeat it
-		h->redo.src         = p.inter;
-		h->redo.n_frames    = n_frames;
-		h->redo.t_end       = t_end;
-		h->redo.first_block = first_block;
-		h->redo.hist        = d_hist;
-		h->redo.ang_start   = ang_start;
-		h->redo.ang_end     = ang_end;
-		h->redo.ang_stride  = ang_stride;
-		h->redo.chn         = chn;
+		// the device-resident form of this pass, should it have to be repeated or resumed
+		h->redo           = job;
+		h->redo.src       = p.inter;
+		h->redo.on_device = true;
+		h->redo.fmt       = PHASEROT_PCM_F32;
+		h->redo.hist      = d_hist;
 	}
 	h->pending = true;
 	return PHASEROT_OK;
@@ -1292,26 +1363,6 @@ sweep_core (phaserot* h, const float* src, bool src_is_device, long long n_frame
 // sweep_kernel walks the rows with grid.z: at most 65535 (section, channel) rows per call,
 // e.g. one hour of 48 kHz stereo in 0.11 s sections or of 8 channels in 0.44 s sections
 constexpr long long kMaxSectionRows = 65535;
-
-// The section instantiations are loaded on first use only, like the kernels of set_device_attrs().
-int
-ensure_sect_attrs (phaserot* h)
-{
-	std::lock_guard<std::mutex> lk (g_create_lock);
-	static std::vector<int>     done;
-	if (done.size () <= (size_t)h->dev) done.resize ((size_t)h->dev + 1, 0);
-	if (done[(size_t)h->dev] & h->NP) return PHASEROT_OK;
-	int rc;
-	if (h->NP == 2) {
-		if ((rc = set_conv_attr<EPI_SECT_POINTS, SRC_INTER, 2> ())) return rc;
-		if ((rc = set_conv_attr<EPI_SECT_RENDER, SRC_INTER, 2> ())) return rc;
-	} else {
-		if ((rc = set_conv_attr<EPI_SECT_POINTS, SRC_INTER, 1> ())) return rc;
-		if ((rc = set_conv_attr<EPI_SECT_RENDER, SRC_INTER, 1> ())) return rc;
-	}
-	done[(size_t)h->dev] |= h->NP;
-	return PHASEROT_OK;
-}
 
 int
 check_sections (phaserot* h, long long n_frames, long long S, int nchan, long long* n_sect)
@@ -1341,7 +1392,6 @@ int
 sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt, long long n_frames, long long S, int ang_start, int ang_end,
                      int ang_stride, int chn)
 {
-	const int pcm_bytes = fmt == PHASEROT_PCM_S16 ? 2 : fmt == PHASEROT_PCM_S32 ? 4 : fmt == PHASEROT_PCM_S24 ? 3 : 0;
 	if (chn >= h->C) {
 		return PHASEROT_E_INVAL;
 	}
@@ -1360,7 +1410,7 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 	if (rc) return rc;
 	rc = finish_pending (h); // a pending sweep of the handle's own table completes first
 	if (rc) return rc;
-	rc = ensure_sect_attrs (h);
+	rc = load_kernels (h, KA_SECT_POINTS | KA_SECT_RENDER);
 	if (rc) return rc;
 	h->sect_n = 0;
 	h->sect_redo_k.clear ();
@@ -1395,22 +1445,15 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 	unsigned*           r2max = ovf_b + R;
 	CK (cudaMemsetAsync (h->d_sect.p, 0, sizeof (unsigned) * (size_t)(R * std::max (A, 1) + R), h->stream));
 	CK (cudaMemsetAsync (h->d_sect_aux.p, 0, sizeof (unsigned long long) + sizeof (unsigned) * 5 * (size_t)R, h->stream));
-	if (A > 0) {
-		rc = h->d_cs.ensure (sizeof (float2) * (size_t)A);
-		if (rc) return rc;
-		rc = h->h_cs.ensure (sizeof (float2) * (size_t)A);
-		if (rc) return rc;
-		float2* cs = (float2*)h->h_cs.p;
-		for (int k = 0; k < A; ++k) cs[k] = make_float2 (h->lut_c[(size_t)idx[(size_t)k]], h->lut_s[(size_t)idx[(size_t)k]]);
-		CK (cudaMemcpyAsync (h->d_cs.p, cs, sizeof (float2) * (size_t)A, cudaMemcpyHostToDevice, h->stream));
-	}
+	rc = upload_angle_table (h, idx);
+	if (rc) return rc;
 
 	const float* d_src = src;
 	if (!src_is_device) {
 		// the bootstrap wave samples every section, so the pass starts once the whole stream has landed
 		rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)n_frames * h->C, 16));
 		if (rc) return rc;
-		rc = upload_chunks (h, src, pcm_bytes, n_frames, [] (long long) { return PHASEROT_OK; });
+		rc = upload_chunks (h, src, fmt, n_frames, [] (long long) { return PHASEROT_OK; });
 		if (rc) return rc;
 		d_src = (const float*)h->d_inter.p;
 	}
@@ -1445,26 +1488,6 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 		++h->stats.kernel_launches;
 		return PHASEROT_OK;
 	};
-	auto sweep = [&] (bool boot) -> int {
-		if (A == 0) return PHASEROT_OK;
-		const SweepCfg sc = pick_sweep_cfg (A);
-		const int      gx = std::max<long long> (1, (h->n_sm * 8) / std::max<long long> (1, sc.gy * R));
-		const dim3     grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)R);
-		const float2*  lst = (const float2*)h->d_list.p;
-		const float2*  cs  = (const float2*)h->d_cs.p;
-		const int      so  = boot ? 0 : 1; // a flagged row is redone: do not brute-force its full list
-		ProfScope      ps (h, 1);
-		switch (sc.R) {
-			case 1: sweep_kernel<1><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
-			case 2: sweep_kernel<2><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
-			case 4: sweep_kernel<4><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
-			default: sweep_kernel<8><<<grid, sc.nt, 0, h->stream>>> (lst, cap, count, (unsigned)cap, so, 0, cs, A, table, A, n_ev); break;
-		}
-		CK (cudaGetLastError ());
-		++h->stats.kernel_launches;
-		return PHASEROT_OK;
-	};
-	auto conv = [&] () -> int { return h->NP == 2 ? launch_conv_np<EPI_SECT_POINTS, SRC_INTER, 2> (h, p) : launch_conv_np<EPI_SECT_POINTS, SRC_INTER, 1> (h, p); };
 
 	if (thr_mode == 1) {
 		// Bootstrap: a quarter of the segments of every section (at least one; more when there are fewer
@@ -1482,28 +1505,28 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 		p.nseg       = n_sect * p.sect_boot;
 		p.boot_beta  = kBootBeta;
 		p.overflow   = ovf_b; // nobody reads it
-		rc = conv ();
+		rc = launch_conv<EPI_SECT_POINTS, SRC_INTER> (h, p);
 		if (rc) return rc;
-		rc = sweep (true);
+		rc = launch_sweep (h, p.list, cap, count, (unsigned)cap, true, 0, (int)R, A, table, n_ev);
 		if (rc) return rc;
 	}
-	// contiguous launches sized like sweep_core's device-resident ones (8 segments per CTA, then 16 x that)
+	// contiguous launches sized like sweep_core's device-resident ones
 	p.sect_boot  = 0;
 	p.seg_stride = 1;
 	p.boot_beta  = 0.f;
 	p.overflow   = ovf;
-	const long long segs_first = std::max<long long> (1, ((long long)h->n_sm * 8) / nchan);
+	static const SegsKnobs knobs;
+	const long long segs_first = std::max<long long> (1, ((long long)h->n_sm * knobs.first) / nchan);
 	long long       seg_done   = 0;
 	for (int n_main = 0; seg_done < nseg; ++n_main) {
-		const bool      short_rest = nseg - seg_done <= 2 * segs_first;
-		const long long n          = std::min ((n_main == 0 && !short_rest) ? segs_first : 16 * segs_first, nseg - seg_done);
+		const long long n = std::min (next_launch_segs (n_main, seg_done, nseg, segs_first, knobs.mult * segs_first, true), nseg - seg_done);
 		rc = thresholds ();
 		if (rc) return rc;
 		p.seg0 = seg_done;
 		p.nseg = n;
-		rc = conv ();
+		rc = launch_conv<EPI_SECT_POINTS, SRC_INTER> (h, p);
 		if (rc) return rc;
-		rc = sweep (false);
+		rc = launch_sweep (h, p.list, cap, count, (unsigned)cap, false, 0, (int)R, A, table, n_ev); // a flagged row is redone: its full list is skipped
 		if (rc) return rc;
 		seg_done += n;
 	}
@@ -1535,10 +1558,8 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 		h->dense_mode       = true;
 		const long long f0  = k * S;
 		const long long F   = std::min (S, n_frames - f0);
-		const long long Bk  = (F + h->L - 1) / h->L;
-		const bool      lst = k == n_sect - 1;
-		rc = sweep_core (h, d_src + (size_t)f0 * h->C, true, F, lst ? (Bk + 1) * h->L : F, k == 0, k ? d_src + (size_t)(f0 - h->L) * h->C : nullptr, ang_start, ang_end,
-		                 ang_stride, chn);
+		rc = sweep_core (h, shard_job (h->L, d_src + (size_t)f0 * h->C, true, PHASEROT_PCM_F32, F, k ? d_src + (size_t)(f0 - h->L) * h->C : nullptr, k == 0, k == n_sect - 1,
+		                               ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 		if (!rc) rc = finish_pending (h);
 		if (!rc) {
 			h->sect_redo_k.push_back (k);
@@ -1563,18 +1584,11 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 int
 render_sections_core (phaserot* h, const float* d_src, long long n_frames, long long t_end, long long S, long long n_sect, const int* angles, float* d_dst)
 {
-	int rc = ensure_sect_attrs (h);
+	int rc = load_kernels (h, KA_SECT_POINTS | KA_SECT_RENDER);
 	if (rc) return rc;
 	const size_t        nrow = (size_t)(n_sect * h->C);
 	std::vector<float2> cs (nrow);
-	for (size_t r = 0; r < nrow; ++r) {
-		// a + MS renders the negation of a: LUT pair of a mod MS, negated for odd half turns
-		const long long a  = angles[r];
-		const long long q  = (a >= 0 ? a : a - h->MS + 1) / h->MS;
-		const size_t    i  = (size_t)(a - q * h->MS);
-		const float     sg = (q & 1) ? -1.f : 1.f;
-		cs[r]              = make_float2 (sg * h->lut_c[i], sg * h->lut_s[i]);
-	}
+	for (size_t r = 0; r < nrow; ++r) cs[r] = full_circle_cs (h, angles[r]);
 	rc = h->d_sect_rt.ensure ((sizeof (float2) + sizeof (int)) * nrow);
 	if (rc) return rc;
 	float2* d_cs  = (float2*)h->d_sect_rt.p;
@@ -1598,7 +1612,7 @@ render_sections_core (phaserot* h, const float* d_src, long long n_frames, long 
 	p.sect_cs    = d_cs;
 	p.sect_ang   = d_ang;
 	p.ang_mp     = (float)(2.f * M_PI / h->S / -360.0); // build_lut()
-	rc = h->NP == 2 ? launch_conv_np<EPI_SECT_RENDER, SRC_INTER, 2> (h, p) : launch_conv_np<EPI_SECT_RENDER, SRC_INTER, 1> (h, p);
+	rc = launch_conv<EPI_SECT_RENDER, SRC_INTER> (h, p);
 	if (rc) return rc;
 	CK (cudaStreamSynchronize (h->stream)); // the host tables above are about to go
 	return PHASEROT_OK;
@@ -1670,14 +1684,6 @@ kweight_powers (const KwCoef& k, long long N)
 	return P;
 }
 
-// The Hilbert instantiation is loaded with the true-peak handles; loudness needs it on every CLI handle.
-int
-ensure_hilbert_attrs (phaserot* h)
-{
-	std::lock_guard<std::mutex> lk (g_create_lock);
-	return set_device_attrs (h->dev, false, h->NP, 2);
-}
-
 constexpr long long kKwChunk = 4096; // frames per thread of kweight_kernel
 
 /*
@@ -1694,7 +1700,7 @@ loudness_core (phaserot* h, const float* d_x, long long F, double fs, const floa
 		std::fill (lufs, lufs + n_sets, -std::numeric_limits<double>::infinity ());
 		return PHASEROT_OK;
 	}
-	int rc = ensure_hilbert_attrs (h);
+	int rc = load_kernels (h, KA_HILBERT); // phaserot_create() loads it for true-peak handles only
 	if (rc) return rc;
 	const long long Fu       = n_sub * step;                  // samples that lie in a sub-block
 	const int       D        = h->L / 2;                      // latency of the render
@@ -1726,15 +1732,9 @@ loudness_core (phaserot* h, const float* d_x, long long F, double fs, const floa
 	float*   d_kx   = (float*)h->d_kx.p;
 	float*   d_H    = (float*)h->d_lH.p;
 
-	// rotations of every set, as phaserot_render_sections forms them: a + MS is the negation of a
+	// rotations of every set, as phaserot_render_sections forms them
 	std::vector<float2> cs ((size_t)n_sets * C);
-	for (size_t r = 0; r < cs.size (); ++r) {
-		const long long a  = angles[r];
-		const long long q  = (a >= 0 ? a : a - h->MS + 1) / h->MS;
-		const size_t    i  = (size_t)(a - q * h->MS);
-		const float     sg = (q & 1) ? -1.f : 1.f;
-		cs[r]              = make_float2 (sg * h->lut_c[i], sg * h->lut_s[i]);
-	}
+	for (size_t r = 0; r < cs.size (); ++r) cs[r] = full_circle_cs (h, angles[r]);
 	std::vector<double> G ((size_t)C, 1.0);
 	if (weights) {
 		for (int c = 0; c < C; ++c) G[(size_t)c] = weights[c];
@@ -1844,10 +1844,9 @@ loudness_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t 
 		// d_inter may still be the source of the pending sweep's dense-mode repeat: complete that sweep first
 		int rc = finish_pending (h);
 		if (rc) return rc;
-		const int pcm_bytes = format == PHASEROT_PCM_S16 ? 2 : format == PHASEROT_PCM_S32 ? 4 : format == PHASEROT_PCM_S24 ? 3 : 0;
-		rc                  = h->d_inter.ensure (sizeof (float) * (size_t)n_frames * h->C);
+		rc = h->d_inter.ensure (sizeof (float) * (size_t)n_frames * h->C);
 		if (rc) return rc;
-		rc = upload_chunks (h, src, pcm_bytes, (long long)n_frames, [] (long long) { return PHASEROT_OK; });
+		rc = upload_chunks (h, src, format, (long long)n_frames, [] (long long) { return PHASEROT_OK; });
 		if (rc) return rc;
 		d_x = (const float*)h->d_inter.p;
 	}
@@ -1961,8 +1960,9 @@ flush_analyze (phaserot* h)
 		return PHASEROT_OK;
 	}
 	const long long frames = (long long)h->an_blocks * h->L;
-	const int rc = sweep_core (h, h->an_buf.data (), false, frames, frames, h->an_first != 0, h->hist_valid ? h->hist.data () : nullptr,
-	                           h->an_start, h->an_end, h->an_stride, h->an_chn);
+	const SweepJob  job { h->an_buf.data (), false, PHASEROT_PCM_F32, frames, frames, h->an_first != 0, h->hist_valid ? h->hist.data () : nullptr,
+                         h->an_start, h->an_end, h->an_stride, h->an_chn };
+	const int rc = sweep_core (h, job, Pass::Fresh);
 	if (rc) return rc;
 	// keep the last block as history for a continued stream
 	h->hist.assign (h->an_buf.end () - (size_t)h->L * h->C, h->an_buf.end ());
@@ -1971,6 +1971,23 @@ flush_analyze (phaserot* h)
 	h->an_blocks = 0;
 	h->an_first  = 0;
 	return finish_pending (h);
+}
+
+// Argument checks of the sweep entry points: data may be null for an empty stream only, and every
+// shard of a stream but the last is a whole number of blocks
+int
+check_sweep (const phaserot* h, const void* data, uint64_t n_frames, bool last = true)
+{
+	if (!h || (!data && n_frames)) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->plugin) {
+		return PHASEROT_E_STATE;
+	}
+	if (!last && ((long long)n_frames % h->L) != 0) {
+		return PHASEROT_E_INVAL;
+	}
+	return PHASEROT_OK;
 }
 
 // pinned staging of one plugin call of n frames: window [C][wstride] | ramp prefix
@@ -2204,7 +2221,7 @@ phaserot_create (phaserot_t** out, const phaserot_cfg_t* cfg)
 			break;
 		}
 		h->stream = h->own_stream;
-		rc        = set_device_attrs (dev, plugin, h->NP, OS);
+		rc        = set_device_attrs (dev, h->NP, plugin ? (KA_RENDER_PLANE | KA_FIR_STREAM) : (KA_RENDER_INTER | (OS > 1 ? KA_HILBERT : KA_POINTS)));
 		if (rc) break;
 		rc = h->d_small.ensure (kSmallBytes);
 		if (rc) break;
@@ -2314,17 +2331,11 @@ phaserot_reset (phaserot_t* h)
 int
 phaserot_sweep (phaserot_t* h, const float* interleaved, uint64_t n_frames, int ang_start, int ang_end, int ang_stride, int chn)
 {
-	if (!h || (!interleaved && n_frames)) {
-		return PHASEROT_E_INVAL;
-	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
-	DevGuard        guard (h->dev);
-	const long long F = (long long)n_frames;
-	const long long B = (F + h->L - 1) / h->L;
-	// analyze_file: B real blocks + one zero flush block (cli:572-586)
-	int rc = sweep_core (h, interleaved, false, F, (B + 1) * h->L, B > 0, nullptr, ang_start, ang_end, ang_stride, chn);
+	int rc = check_sweep (h, interleaved, n_frames);
+	if (rc) return rc;
+	DevGuard guard (h->dev);
+	rc = sweep_core (h, shard_job (h->L, interleaved, false, PHASEROT_PCM_F32, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn),
+	                 Pass::Fresh);
 	if (rc) return rc;
 	return finish_pending (h);
 }
@@ -2332,16 +2343,13 @@ phaserot_sweep (phaserot_t* h, const float* interleaved, uint64_t n_frames, int 
 int
 phaserot_sweep_pcm (phaserot_t* h, const void* pcm, int format, uint64_t n_frames, int ang_start, int ang_end, int ang_stride, int chn)
 {
-	if (!h || (!pcm && n_frames) || (format != PHASEROT_PCM_S16 && format != PHASEROT_PCM_S32 && format != PHASEROT_PCM_S24)) {
+	if (format != PHASEROT_PCM_S16 && format != PHASEROT_PCM_S32 && format != PHASEROT_PCM_S24) {
 		return PHASEROT_E_INVAL;
 	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
-	DevGuard        guard (h->dev);
-	const long long F = (long long)n_frames;
-	const long long B = (F + h->L - 1) / h->L;
-	int rc = sweep_core (h, (const float*)pcm, false, F, (B + 1) * h->L, B > 0, nullptr, ang_start, ang_end, ang_stride, chn, format);
+	int rc = check_sweep (h, pcm, n_frames);
+	if (rc) return rc;
+	DevGuard guard (h->dev);
+	rc = sweep_core (h, shard_job (h->L, pcm, false, format, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 	if (rc) return rc;
 	return finish_pending (h);
 }
@@ -2349,16 +2357,11 @@ phaserot_sweep_pcm (phaserot_t* h, const void* pcm, int format, uint64_t n_frame
 int
 phaserot_sweep_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, int ang_start, int ang_end, int ang_stride, int chn)
 {
-	if (!h || (!d_interleaved && n_frames)) {
-		return PHASEROT_E_INVAL;
-	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
-	DevGuard        guard (h->dev);
-	const long long F = (long long)n_frames;
-	const long long B = (F + h->L - 1) / h->L;
-	return sweep_core (h, d_interleaved, true, F, (B + 1) * h->L, B > 0, nullptr, ang_start, ang_end, ang_stride, chn);
+	const int rc = check_sweep (h, d_interleaved, n_frames);
+	if (rc) return rc;
+	DevGuard guard (h->dev);
+	return sweep_core (h, shard_job (h->L, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn),
+	                   Pass::Fresh);
 }
 
 int
@@ -2445,40 +2448,22 @@ int
 phaserot_sweep_shard_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, const float* hist, int first, int last,
                              int ang_start, int ang_end, int ang_stride, int chn)
 {
-	if (!h || (!d_interleaved && n_frames)) {
-		return PHASEROT_E_INVAL;
-	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
-	const long long F = (long long)n_frames;
-	if (!last && (F % h->L) != 0) {
-		return PHASEROT_E_INVAL;
-	}
-	DevGuard        guard (h->dev);
-	const long long B     = (F + h->L - 1) / h->L;
-	const long long t_end = last ? (B + 1) * h->L : F;
-	return sweep_core (h, d_interleaved, true, F, t_end, first != 0 && B > 0, hist, ang_start, ang_end, ang_stride, chn);
+	const int rc = check_sweep (h, d_interleaved, n_frames, last != 0);
+	if (rc) return rc;
+	DevGuard guard (h->dev);
+	return sweep_core (h, shard_job (h->L, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn),
+	                   Pass::Fresh);
 }
 
 int
 phaserot_sweep_shard_boot_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, const float* hist, int first, int last,
                                   int ang_start, int ang_end, int ang_stride, int chn)
 {
-	if (!h || (!d_interleaved && n_frames)) {
-		return PHASEROT_E_INVAL;
-	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
-	const long long F = (long long)n_frames;
-	if (!last && (F % h->L) != 0) {
-		return PHASEROT_E_INVAL;
-	}
-	DevGuard        guard (h->dev);
-	const long long B     = (F + h->L - 1) / h->L;
-	const long long t_end = last ? (B + 1) * h->L : F;
-	return sweep_core (h, d_interleaved, true, F, t_end, first != 0 && B > 0, hist, ang_start, ang_end, ang_stride, chn, PHASEROT_PCM_F32, false, true);
+	const int rc = check_sweep (h, d_interleaved, n_frames, last != 0);
+	if (rc) return rc;
+	DevGuard guard (h->dev);
+	return sweep_core (h, shard_job (h->L, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn),
+	                   Pass::BootOnly);
 }
 
 int
@@ -2490,29 +2475,21 @@ phaserot_sweep_shard_resume (phaserot_t* h)
 	if (h->plugin || !h->pending) {
 		return PHASEROT_E_STATE;
 	}
-	DevGuard              guard (h->dev);
-	const phaserot::Redo r = h->redo;
-	return sweep_core (h, r.src, true, r.n_frames, r.t_end, r.first_block, r.hist, r.ang_start, r.ang_end, r.ang_stride, r.chn, PHASEROT_PCM_F32, true, false);
+	DevGuard guard (h->dev);
+	return sweep_core (h, h->redo, Pass::Continue);
 }
 
 int
 phaserot_sweep_shard (phaserot_t* h, const void* data, int format, uint64_t n_frames, const float* hist, int first, int last,
                       int ang_start, int ang_end, int ang_stride, int chn)
 {
-	if (!h || (!data && n_frames) || format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) {
+	if (format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) {
 		return PHASEROT_E_INVAL;
 	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
-	const long long F = (long long)n_frames;
-	if (!last && (F % h->L) != 0) {
-		return PHASEROT_E_INVAL;
-	}
-	DevGuard        guard (h->dev);
-	const long long B     = (F + h->L - 1) / h->L;
-	const long long t_end = last ? (B + 1) * h->L : F;
-	return sweep_core (h, (const float*)data, false, F, t_end, first != 0 && B > 0, hist, ang_start, ang_end, ang_stride, chn, format);
+	const int rc = check_sweep (h, data, n_frames, last != 0);
+	if (rc) return rc;
+	DevGuard guard (h->dev);
+	return sweep_core (h, shard_job (h->L, data, false, format, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 }
 
 int
@@ -2686,12 +2663,11 @@ int
 phaserot_sweep_sections (phaserot_t* h, const void* data, int format, uint64_t n_frames, uint64_t section_frames, int ang_start, int ang_end, int ang_stride,
                          int chn)
 {
-	if (!h || (!data && n_frames) || format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) {
+	if (format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) {
 		return PHASEROT_E_INVAL;
 	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
+	const int rc = check_sweep (h, data, n_frames);
+	if (rc) return rc;
 	DevGuard guard (h->dev);
 	return sweep_sections_core (h, (const float*)data, false, format, (long long)n_frames, (long long)section_frames, ang_start, ang_end, ang_stride, chn);
 }
@@ -2700,12 +2676,8 @@ int
 phaserot_sweep_sections_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, uint64_t section_frames, int ang_start, int ang_end,
                                 int ang_stride, int chn)
 {
-	if (!h || (!d_interleaved && n_frames)) {
-		return PHASEROT_E_INVAL;
-	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
+	const int rc = check_sweep (h, d_interleaved, n_frames);
+	if (rc) return rc;
 	DevGuard guard (h->dev);
 	return sweep_sections_core (h, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, (long long)section_frames, ang_start, ang_end, ang_stride, chn);
 }
@@ -2733,13 +2705,8 @@ phaserot_section_peaks (phaserot_t* h, int* n_sections, float* out)
 	const size_t per = (size_t)h->C * h->MS;
 	std::fill (out, out + (size_t)h->sect_n * per, 0.f);
 	for (size_t r = 0; r < R; ++r) {
-		// the same merge as finish_pending(): grid index 0 holds the raw peak unless the angle set maps onto it too
-		float* row = out + (r / nchan) * per + (size_t)(h->sect_c0 + (int)(r % nchan)) * h->MS;
-		for (int k = 0; k < A; ++k) {
-			const int a = h->sect_idx[(size_t)k];
-			row[a]      = std::max (row[a], res[r * A + (size_t)k]);
-		}
-		if (h->sect_raw) row[0] = std::max (row[0], res[R * A + r]);
+		merge_row (out + (r / nchan) * per + (size_t)(h->sect_c0 + (int)(r % nchan)) * h->MS, res.data () + r * A, h->sect_idx,
+		           h->sect_raw ? res.data () + R * A + r : nullptr);
 	}
 	for (size_t i = 0; i < h->sect_redo_k.size (); ++i) {
 		memcpy (out + (size_t)h->sect_redo_k[i] * per, h->sect_redo.data () + i * per, sizeof (float) * per);
@@ -3259,7 +3226,6 @@ phaserot_group_sweep (phaserot_group_t* g, const void* data, int format, uint64_
 	long long per = (F + n - 1) / n;
 	per           = std::max (align, (per + align - 1) / align * align);
 	const int used = (int)std::max<long long> (1, std::min<long long> (n, (F + per - 1) / per));
-	const size_t bps = format == PHASEROT_PCM_S16 ? 2 : format == PHASEROT_PCM_S24 ? 3 : 4;
 
 	std::vector<int>         rcs ((size_t)used, PHASEROT_OK);
 	std::vector<std::string> errs ((size_t)used);
@@ -3272,11 +3238,9 @@ phaserot_group_sweep (phaserot_group_t* g, const void* data, int format, uint64_
 		if (i > 0) {
 			shard_history (data, format, f0, h->L, h->C, hist);
 		}
-		DevGuard        guard (h->dev);
-		const long long B     = (nf + h->L - 1) / h->L;
-		const long long t_end = lst ? (B + 1) * h->L : nf;
-		int rc = sweep_core (h, (const float*)((const char*)data + bps * (size_t)f0 * h->C), false, nf, t_end, i == 0 && B > 0,
-		                     i > 0 ? hist.data () : nullptr, ang_start, ang_end, ang_stride, chn, format);
+		DevGuard guard (h->dev);
+		int      rc = sweep_core (h, shard_job (h->L, (const char*)data + pcm_bytes (format) * (size_t)f0 * h->C, false, format, nf, i > 0 ? hist.data () : nullptr,
+		                                        i == 0, lst, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 		if (rc == PHASEROT_OK) {
 			rc = complete_pending (h); // a shard whose survivor list overflowed is repeated in dense mode before the tables are combined
 		}
