@@ -294,6 +294,46 @@ PHASEROT_API int phaserot_loudness (phaserot_t* h, const void* data, int format,
 PHASEROT_API int phaserot_loudness_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, double sample_rate,
                                            const float* weights, const int* angles, int n_sets, double* lufs);
 
+/* ---- overs above a ceiling ------------------------------------------------- */
+
+/* Extends the min-peak sweep, which says at which angle the single largest sample is smallest, with how much
+ * of the rotated output a limiter or clipper after a ceiling T (linear, e.g. -1 dBTP) would have to work on:
+ * for every angle, the number of samples above T and by how much, from one pass.
+ *   sample set : exactly the samples and detector points phaserot_sweep() evaluates on the same handle and input
+ *                (first-block rule cli:418-419, the zero flush block, chn, the digital peak or the oversample =
+ *                2 / 4 detector of the true-peak definition above); grid index 0 is the raw input under the
+ *                same detector (cli:413-414)
+ *   digital    : sample t is over at angle a when |y| > T, y = fmaf (ca, x_d, sa * H) - the expression of the
+ *                sweep, so counts[c][a] > 0 exactly when phaserot_sweep()'s peak[c][a] > T, index 0 included
+ *   true-peak  : sample t is over when the largest |y| over its detector points exceeds T; samples are counted,
+ *                not points
+ *   excess     : excess[c][a] = sum over the overs of (v - T), v the value that made the sample over; every term is
+ *                truncated to a multiple of 2^-32 and summed in 64-bit integers, so repeated calls and the host and
+ *                device forms return the same doubles.  The sum of one entry must stay below 2^32 (full scale = 1.0):
+ *                audio within full scale cannot reach it (an hour of 48 kHz audio is 1.7e8 samples, each term a few units at most);
+ *                float input far outside [-1, 1] with a low ceiling can, and its excess is then not defined (the
+ *                counts are)
+ *   output     : full tables counts[n_channels][180 * subsample], excess[n_channels][180 * subsample] (excess may be
+ *                NULL); entries outside the requested angles and channel are 0.  Should the angle loop reach grid
+ *                index 0 both as angle 0 (raw input) and wrapped (a multiple of 180 * subsample), the entry holds
+ *                whichever of the two has more overs.
+ * A point whose radius sqrt(x_d^2 + H^2) is below T cannot be over T at any angle: T is the fixed radius of the
+ * sweep's exact pruning, and PHASEROT_FLAG_NO_PRUNE (radius 0: every examined point listed) gives the same tables.  Low ceilings
+ * put most samples on the survivor lists; an FFT launch whose list overflows is re-run in pieces that fit
+ * (phaserot_stats_t.dense_repeats counts these re-runs) - the tables do not depend on it.
+ * `data` and `format` as phaserot_sweep_pcm() / PHASEROT_PCM_F32, with the same widening; host memory.
+ * Synchronous.  The peak table, section tables and apply() stream state are not changed (the host form completes
+ * a pending device sweep first, as phaserot_peaks() would).  PHASEROT_E_STATE for plugin handles;
+ * PHASEROT_E_INVAL with a phaserot_last_error() text for a ceiling <= 0 or not finite, n_frames == 0, NULL counts,
+ * and the angle and channel arguments phaserot_sweep() rejects. */
+PHASEROT_API int phaserot_overs (phaserot_t* h, const void* data, int format, uint64_t n_frames, float ceiling,
+                                 int ang_start, int ang_end, int ang_stride, int chn,
+                                 uint64_t* counts, double* excess);
+/* The same over audio resident in device memory (interleaved float32, n_frames * n_channels). */
+PHASEROT_API int phaserot_overs_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, float ceiling,
+                                        int ang_start, int ang_end, int ang_stride, int chn,
+                                        uint64_t* counts, double* excess);
+
 /* ---- several GPUs in one process ---------------------------------------- */
 
 /* A group of handles, one per device, that analyses ONE stream: the file is cut

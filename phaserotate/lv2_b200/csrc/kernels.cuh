@@ -12,6 +12,7 @@
 //    threshold_kernel      min over angles of the running peaks -> next filter radius
 //    fir_stream_kernel     small-call plugin path: direct-form FIR + rotate, history in a device ring
 //    truepeak_kernel       oversampled true-peak front end of the sweep
+//    overs_kernel          overs table: per-angle count and excess of survivors above a ceiling
 //
 // Data layout.  A channel's samples x[0..F) are viewed as complex numbers
 // z[n] = x[2n] + i x[2n+1] ("plane", float2, with a zero front pad).  The
@@ -930,6 +931,78 @@ __global__ void __launch_bounds__ (256) sweep_kernel (const float2* __restrict__
 	}
 }
 
+// Overs table (phaserot_overs): the sweep_kernel layout - angles in lanes, R per thread, (ca, sa) from
+// the angle table, tiles of the survivor list broadcast from shared memory - over records of G points
+// (1: a digital sample; 3 / 5: a true-peak sample and its interpolated points).  A record is over at angle
+// a when v = max over its points of |ca x + sa h| (the expression of sweep_kernel) exceeds T; each lane
+// counts its overs and sums (v - T) truncated to multiples of 2^-32 in a 64-bit integer, so the totals
+// do not depend on how records are split over CTAs or launches.  One integer atomicAdd per angle and CTA.
+// count[c] is in points; a channel whose list overflowed is skipped (its launch is re-run in pieces).
+constexpr int kOversTile = 256; // records per tile
+template <int R, int G>
+__global__ void __launch_bounds__ (256) overs_kernel (const float2* __restrict__ list, long long list_stride,
+                                                       const unsigned* __restrict__ count, unsigned cap, int chan0,
+                                                       const float2* __restrict__ cs, int A, float T,
+                                                       unsigned long long* __restrict__ n_over, unsigned long long* __restrict__ excess,
+                                                       unsigned long long* __restrict__ n_eval)
+{
+	__shared__ __align__ (16) float2 tile[kOversTile * G];
+	const int c = chan0 + blockIdx.z;
+	if (count[c] > cap) return;
+	const unsigned n        = count[c] / G; // records
+	const unsigned tile_rec = min ((unsigned)kOversTile, max (32u, (n + gridDim.x - 1) / gridDim.x));
+	if (blockIdx.x * tile_rec >= n) return;
+	const float2* pts = list + (long long)c * list_stride;
+	const int     a0  = blockIdx.y * (blockDim.x * R) + threadIdx.x;
+
+	float              ca[R], sa[R];
+	unsigned           cnt[R];
+	unsigned long long exc[R];
+#pragma unroll
+	for (int r = 0; r < R; ++r) {
+		const int    a = a0 + r * blockDim.x;
+		const float2 v = a < A ? cs[a] : make_float2 (0.f, 0.f);
+		ca[r]          = v.x;
+		sa[r]          = v.y;
+		cnt[r]         = 0;
+		exc[r]         = 0;
+	}
+	const double Td = (double)T;
+
+	for (unsigned base = blockIdx.x * tile_rec; base < n; base += gridDim.x * tile_rec) {
+		const unsigned nr = min (tile_rec, n - base);
+		__syncthreads ();
+		for (unsigned i = threadIdx.x; i < nr * G; i += blockDim.x) tile[i] = pts[(size_t)base * G + i];
+		__syncthreads ();
+#pragma unroll 2
+		for (unsigned i = 0; i < nr; ++i) {
+			float2 q[G];
+#pragma unroll
+			for (int g = 0; g < G; ++g) q[g] = tile[i * G + g]; // broadcast
+#pragma unroll
+			for (int r = 0; r < R; ++r) {
+				float v = 0.f;
+#pragma unroll
+				for (int g = 0; g < G; ++g) v = fmaxf (v, fabsf (fmaf (ca[r], q[g].x, sa[r] * q[g].y)));
+				if (v > T) {
+					++cnt[r];
+					exc[r] += (unsigned long long)(((double)v - Td) * 4294967296.0); // exact difference of two floats, truncated
+				}
+			}
+		}
+		if (n_eval && blockIdx.y == 0 && threadIdx.x == 0) atomicAdd (n_eval, (unsigned long long)nr * G);
+	}
+
+#pragma unroll
+	for (int r = 0; r < R; ++r) {
+		const int a = a0 + r * blockDim.x;
+		if (a < A && cnt[r]) {
+			atomicAdd (n_over + (long long)c * A + a, (unsigned long long)cnt[r]);
+			atomicAdd (excess + (long long)c * A + a, exc[r]);
+		}
+	}
+}
+
 // thr2[c] = (min_a peaks[c][a])^2 * (1 - 1e-5): a point whose radius is below
 // that cannot raise any angle's running maximum (|ca x + sa h| <= sqrt(x^2+h^2)
 // up to a few ulp), so dropping it leaves every peak bit-identical.
@@ -1519,6 +1592,9 @@ __device__ __forceinline__ void tp_append (float2* lst, unsigned* cnt, unsigned 
 	}
 }
 
+// kGroup (phaserot_overs): a sample with any detector point at or above the radius lists ALL of its points,
+// the sample first, as one record of os + 1 points (os = 2: the sample and phases 0 and 2).
+template <bool kGroup = false>
 __global__ void __launch_bounds__ (256, 4) truepeak_kernel (const TpParams p)
 {
 	__shared__ __align__ (16) float sh[kTpTile + kTpHalo], sx[kTpTile + kTpHalo], sq[kTpTile + kTpHalo];
@@ -1586,6 +1662,7 @@ __global__ void __launch_bounds__ (256, 4) truepeak_kernel (const TpParams p)
 				rmax = fmaxf (rmax, fabsf (pt[q].x));
 				if (fmaf (pt[q].x, pt[q].x, pt[q].y * pt[q].y) >= thr2f && (p.os == 4 || !(q == 2 || q == 4))) keep |= 1u << q;
 			}
+			if (kGroup && keep) keep = p.os == 4 ? 0x1fu : 0x0bu;
 			tp_append (lstf, cntf, p.list_cap, p.overflow, keep, pt, lanef);
 		}
 		for (int o = 16; o; o >>= 1) rmax = fmaxf (rmax, __shfl_xor_sync (0xffffffffu, rmax, o));
@@ -1654,10 +1731,48 @@ __global__ void __launch_bounds__ (256, 4) truepeak_kernel (const TpParams p)
 			if (in) rawmax = fmaxf (rawmax, fabsf (xr[q]));
 			if (ex && fmaf (pt[q].x, pt[q].x, pt[q].y * pt[q].y) >= thr2 && (p.os == 4 || !(q == 2 || q == 4))) keep |= 1u << q;
 		}
+		if (kGroup && keep) keep = p.os == 4 ? 0x1fu : 0x0bu;
 		tp_append (lst, cnt, p.list_cap, p.overflow, keep, pt, lane);
 	}
 	for (int o = 16; o; o >>= 1) rawmax = fmaxf (rawmax, __shfl_xor_sync (0xffffffffu, rawmax, o));
 	if (lane == 0 && rawmax > 0.f) atomicMax (p.rawpeak + c, __float_as_uint (rawmax));
+}
+
+// Grid index 0 of the overs table (phaserot_overs): the raw input under the detector of the raw-peak rule
+// (cli:413-414) over frames [0, f_end) - |x[f]| for the digital peak; for os = 2 / 4 the largest of |x[f]|
+// and its interpolated points, formed with the fmaf chain of tp_interp, i.e. the very values truepeak_kernel
+// takes the raw peak of.  Over, count and excess as in overs_kernel.  grid = (frame blocks, channels).
+__global__ void __launch_bounds__ (256) overs_raw_kernel (const float* __restrict__ inter, long long n_frames, int C, int chan0, long long f_end, int os,
+                                                           float T, unsigned long long* __restrict__ n_over, unsigned long long* __restrict__ excess)
+{
+	const int          c   = chan0 + blockIdx.y;
+	unsigned           cnt = 0;
+	unsigned long long exc = 0;
+	for (long long f = (long long)blockIdx.x * blockDim.x + threadIdx.x; f < f_end; f += (long long)gridDim.x * blockDim.x) {
+		float v = f < n_frames ? fabsf (__ldg (inter + f * C + c)) : 0.f;
+		if (os > 1) {
+			float s[16];
+#pragma unroll
+			for (int k = 0; k < 16; ++k) { // s[12 - k] = x[f - k]
+				const long long g = f + k - 12;
+				s[k]              = (k <= 12 && g >= 0 && g < n_frames) ? __ldg (inter + g * C + c) : 0.f;
+			}
+			v = fmaxf (v, fmaxf (fabsf (tp_interp<0> (s, 0)), fabsf (tp_interp<2> (s, 0))));
+			if (os == 4) v = fmaxf (v, fmaxf (fabsf (tp_interp<1> (s, 0)), fabsf (tp_interp<3> (s, 0))));
+		}
+		if (v > T) {
+			++cnt;
+			exc += (unsigned long long)(((double)v - (double)T) * 4294967296.0);
+		}
+	}
+	for (int o = 16; o; o >>= 1) {
+		cnt += __shfl_xor_sync (0xffffffffu, cnt, o);
+		exc += __shfl_xor_sync (0xffffffffu, exc, o);
+	}
+	if ((threadIdx.x & 31) == 0 && cnt) {
+		atomicAdd (n_over + c, (unsigned long long)cnt);
+		atomicAdd (excess + c, exc);
+	}
 }
 
 // last kTpCarry floats of a contiguous launch's H -> front of the buffer, for the next launch

@@ -267,6 +267,10 @@ struct phaserot {
 	// floats | fp64 work: sub-block sums, head correction, chunk states, A powers, weights, results | angle sets
 	DevBuf d_kx, d_lH, d_lwork, d_lset;
 
+	// overs table (phaserot_overs): survivor list | true-peak staging of the Hilbert branch | tables, angle table,
+	// radii and the list counters of every launch; its own buffers, so that a pending device sweep is not disturbed
+	DevBuf d_ovl, d_ovH, d_ovw;
+
 	// pending (asynchronous) sweep result
 	bool             pending = false;
 	std::vector<int> pend_idx;
@@ -653,6 +657,50 @@ next_launch_segs (int n_main, long long seg_done, long long nseg, long long segs
 	return (n_main == 0 && !short_rest) ? segs_first : segs_max;
 }
 
+// Launch sizes and survivor-list capacity of a pass over nseg segments per channel of nchan channels.
+struct ListPlan {
+	long long ppseg;                // points a segment can put on the list (true-peak: the sample and OS interpolated points)
+	long long segs_first, segs_max; // segments per channel of the first contiguous launch and of the following ones
+	long long cap;                  // points per channel the list holds
+	long long segs_cap;             // segments per channel of the largest launch
+};
+ListPlan
+plan_lists (const phaserot* h, int nchan, long long nseg, bool on_device, bool dense)
+{
+	// (8 segments per CTA; device-resident digital-peak input: up to 128 from the
+	// second contiguous launch on - by then the radius is close to final, a launch
+	// leaves a few dozen survivors, and every launch + sweep saved is ~20 us: an hour
+	// of stereo is bootstrap + 2 launches.  The list is sized by the stream, at most
+	// 3.7 GB.  Host input keeps 8, so that little work is left when the last chunk
+	// has landed.)
+	static const SegsKnobs knobs;
+	ListPlan lp;
+	lp.ppseg      = (long long)h->V * 2 * (h->OS > 1 ? h->OS + 1 : 1);
+	lp.segs_first = std::max<long long> (1, ((long long)h->n_sm * knobs.first) / nchan);
+	lp.segs_max   = !on_device ? lp.segs_first : (OS_is_digital (h) ? knobs.mult : 2) * lp.segs_first;
+	// Survivor list, sized by demand.  Normal mode: 1/32 of the points of the
+	// largest launch (pruning leaves 1e-4 .. 1e-5 of them on programme material), at
+	// least 1 M points per channel; a list that overflows flags the pass and
+	// complete_pending() repeats it in dense mode.  Dense mode (and NO_PRUNE, where
+	// every point goes on the list): at most kDenseCap points per channel (4 M .. 48 M), and the
+	// launches are sized to it, so nothing can overflow.
+	// (the list and the wide list: 16 bytes per point and channel; 2 GB between them, 48 M points for stereo)
+	const long long kDenseCap = std::min<long long> (48LL << 20, std::max<long long> (4LL << 20, (2LL << 30) / (16LL * std::max (1, nchan))));
+	if (dense) {
+		const long long fit = std::max<long long> (1, kDenseCap / lp.ppseg);
+		lp.segs_first       = std::min (lp.segs_first, fit);
+		lp.segs_max         = std::min (lp.segs_max, fit);
+		lp.cap              = std::min (std::max (lp.segs_first, lp.segs_max), std::max<long long> (nseg, 1)) * lp.ppseg;
+	} else {
+		const long long full = std::min (std::max (lp.segs_first, lp.segs_max), std::max<long long> (nseg, 1)) * lp.ppseg;
+		// (at least one wave: a stream too short for the bootstrap starts with an unpruned wave that lists every point)
+		const long long wave_pts = std::max<long long> (1, (h->n_sm + nchan - 1) / nchan) * lp.ppseg;
+		lp.cap                   = std::min (full, std::max ({ 1LL << 20, full / 32, wave_pts }));
+	}
+	lp.segs_cap = std::min (std::max (lp.segs_first, lp.segs_max), std::max<long long> (nseg, 1));
+	return lp;
+}
+
 enum class Pass {
 	Fresh,    // a new pass: the pending one is finished first, the device table starts empty, bootstrap included
 	BootOnly, // Fresh, but only the bootstrap wave and its sweep are enqueued (two-phase sharded sweep)
@@ -1000,39 +1048,10 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 	}
 
 	// survivor list: one launch covers at most `segs_max` segments per channel
-	const int       nchan    = c1 - c0;
-	// (8 segments per CTA; device-resident digital-peak input: up to 128 from the
-	// second contiguous launch on - by then the radius is close to final, a launch
-	// leaves a few dozen survivors, and every launch + sweep saved is ~20 us: an hour
-	// of stereo is bootstrap + 2 launches.  The list is sized by the stream, at most
-	// 3.7 GB.  Host input keeps 8, so that little work is left when the last chunk
-	// has landed.)
+	const int       nchan      = c1 - c0;
 	const int       OS         = h->OS;
-	const long long ppseg      = (long long)h->V * 2 * (OS > 1 ? OS + 1 : 1); // points a segment can put on the list (true-peak: the sample and OS interpolated points)
-	static const SegsKnobs knobs;
-	long long       segs_first = std::max<long long> (1, ((long long)h->n_sm * knobs.first) / nchan);
-	long long       segs_max   = !job.on_device ? segs_first : (OS_is_digital (h) ? knobs.mult : 2) * segs_first;
-	// Survivor list, sized by demand.  Normal mode: 1/32 of the points of the
-	// largest launch (pruning leaves 1e-4 .. 1e-5 of them on programme material), at
-	// least 1 M points per channel; a list that overflows flags the pass and
-	// complete_pending() repeats it in dense mode.  Dense mode (and NO_PRUNE, where
-	// every point goes on the list): at most kDenseCap points per channel (4 M .. 48 M), and the
-	// launches are sized to it, so nothing can overflow.
-	// (the list and the wide list: 16 bytes per point and channel; 2 GB between them, 48 M points for stereo)
-	const long long kDenseCap = std::min<long long> (48LL << 20, std::max<long long> (4LL << 20, (2LL << 30) / (16LL * std::max (1, nchan))));
-	long long           cap;
-	if (dense) {
-		const long long fit = std::max<long long> (1, kDenseCap / ppseg);
-		segs_first          = std::min (segs_first, fit);
-		segs_max            = std::min (segs_max, fit);
-		cap                 = std::min (std::max (segs_first, segs_max), std::max<long long> (nseg, 1)) * ppseg;
-	} else {
-		const long long full = std::min (std::max (segs_first, segs_max), std::max<long long> (nseg, 1)) * ppseg;
-		// (at least one wave: a stream too short for the bootstrap starts with an unpruned wave that lists every point)
-		const long long wave_pts = std::max<long long> (1, (h->n_sm + nchan - 1) / nchan) * ppseg;
-		cap                      = std::min (full, std::max ({ 1LL << 20, full / 32, wave_pts }));
-	}
-	const long long segs_cap = std::min (std::max (segs_first, segs_max), std::max<long long> (nseg, 1));
+	const ListPlan  lp         = plan_lists (h, nchan, nseg, job.on_device, dense);
+	const long long segs_first = lp.segs_first, segs_max = lp.segs_max, cap = lp.cap, segs_cap = lp.segs_cap;
 	h->list_stride           = cap;
 	h->list_cap              = cap;
 	rc                       = h->d_list.ensure ((size_t)h->list_stride * h->C * sizeof (float2));
@@ -1232,7 +1251,7 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 			{
 				ProfScope  ps (h, 6);
 				const dim3 grid ((unsigned)(n * (tp.V2 / kTpTile)), (unsigned)nchan);
-				truepeak_kernel<<<grid, 256, 0, h->stream>>> (tp);
+				truepeak_kernel<false><<<grid, 256, 0, h->stream>>> (tp);
 				CK (cudaGetLastError ());
 				++h->stats.kernel_launches;
 			}
@@ -1973,6 +1992,307 @@ flush_analyze (phaserot* h)
 	return finish_pending (h);
 }
 
+/*
+ * phaserot_overs over F frames of interleaved float32 audio on the device: the FFT pass of the sweep with a
+ * fixed filter radius T^2 (1 - 1e-5) (a point whose radius is below T cannot be over T at any angle, up to the
+ * margin threshold_kernel relies on), the survivors counted by overs_kernel, grid index 0 by overs_raw_kernel.
+ * Launches and lists as a device-resident sweep (plan_lists, next_launch_segs); the counters of every launch
+ * are kept, and a (launch, channel) whose list overflowed - low ceilings put most points on it - is re-run
+ * afterwards in pieces the list holds in full.  Synchronous.  counts / excess: host [C][MS] (excess may be null).
+ */
+int
+overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, int ang_end, int ang_stride, int chn, uint64_t* counts, double* excess)
+{
+	std::vector<int> idx;
+	bool             raw = false;
+	int              rc  = angle_schedule (h, ang_start, ang_end, ang_stride, idx, raw);
+	if (rc) return rc;
+	const int       C     = h->C;
+	const int       A     = (int)idx.size ();
+	const int       c0    = chn < 0 ? 0 : chn;
+	const int       c1    = chn < 0 ? C : chn + 1;
+	const int       nchan = c1 - c0;
+	const int       OS    = h->OS;
+	const int       G     = OS > 1 ? OS + 1 : 1; // points per record
+	const long long B     = (F + h->L - 1) / h->L;
+	const long long t_end = (B + 1) * h->L;      // B blocks + the zero flush block, like phaserot_sweep
+	const long long m_end = (t_end + 1) / 2;
+	const long long nseg  = (m_end + h->V - 1) / h->V;
+	const bool      quirk    = !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK);
+	const bool      no_prune = (h->cfg.flags & PHASEROT_FLAG_NO_PRUNE) != 0;
+	const ListPlan  lp       = plan_lists (h, nchan, nseg, true, no_prune);
+	const long long n_lmax = nseg / lp.segs_first + 3; // launches of the schedule (+ 1 counter set for the re-runs)
+
+	// work area: u64 counts [C][A] | u64 excess [C][A] | u64 raw counts [C] | u64 raw excess [C] | u64 evaluated |
+	// (ca, sa) [A] | thr2 [C] | raw peaks [C] (unused) | overflow word (unused) | list counters [n_lmax][C]
+	const size_t n_tab = (size_t)C * A;
+	const size_t n_u64 = 2 * n_tab + 2 * (size_t)C + 1;
+	const size_t bytes = sizeof (unsigned long long) * n_u64 + sizeof (float2) * (size_t)std::max (A, 1) + sizeof (float) * (2 * (size_t)C + 1) +
+	                     sizeof (unsigned) * (size_t)n_lmax * C;
+	rc = h->d_ovw.ensure (bytes);
+	if (rc) return rc;
+	unsigned long long* d_cnt  = (unsigned long long*)h->d_ovw.p;
+	unsigned long long* d_exc  = d_cnt + n_tab;
+	unsigned long long* d_rcnt = d_exc + n_tab;
+	unsigned long long* d_rexc = d_rcnt + C;
+	unsigned long long* d_eval = d_rexc + C;
+	float2*             d_cs   = (float2*)(d_eval + 1);
+	float*              d_thr2 = (float*)(d_cs + std::max (A, 1));
+	unsigned*           d_rawp = (unsigned*)(d_thr2 + C);
+	unsigned*           d_ovf  = d_rawp + C;
+	unsigned*           d_lcnt = d_ovf + 1;
+	CK (cudaMemsetAsync (h->d_ovw.p, 0, bytes, h->stream));
+	{
+		std::vector<float2> cs ((size_t)A);
+		for (int k = 0; k < A; ++k) cs[(size_t)k] = make_float2 (h->lut_c[(size_t)idx[(size_t)k]], h->lut_s[(size_t)idx[(size_t)k]]);
+		// the margin of threshold_kernel; NO_PRUNE: radius 0, every examined point (true-peak: every sample's group) is listed
+		const std::vector<float> thr2 ((size_t)C, no_prune ? 0.f : (T * T) * 0.99999f);
+		CK (cudaMemcpyAsync (d_cs, cs.data (), sizeof (float2) * cs.size (), cudaMemcpyHostToDevice, h->stream));
+		CK (cudaMemcpyAsync (d_thr2, thr2.data (), sizeof (float) * thr2.size (), cudaMemcpyHostToDevice, h->stream));
+	}
+
+	// grid index 0: the raw input (the interpolator reaches 11 frames past the last one)
+	if (raw) {
+		const long long f_end = std::min (F + (OS > 1 ? 11 : 0), t_end - h->L / 2);
+		const long long nb    = std::min<long long> ((f_end + 255) / 256, (long long)h->n_sm * 8);
+		ProfScope       ps (h, 5);
+		overs_raw_kernel<<<dim3 ((unsigned)nb, (unsigned)nchan), 256, 0, h->stream>>> (d_x, F, C, c0, f_end, OS, T, d_rcnt, d_rexc);
+		CK (cudaGetLastError ());
+		++h->stats.kernel_launches;
+	}
+
+	std::vector<unsigned> lcnt;
+	std::vector<long long> l_s0, l_n;
+	if (A > 0) {
+		rc = h->d_ovl.ensure (sizeof (float2) * (size_t)lp.cap * C);
+		if (rc) return rc;
+		const long long tp_stride = (kTpCarry + lp.segs_cap * 2 * h->V + 3) & ~3LL;
+		if (OS > 1) {
+			rc = h->d_ovH.ensure (sizeof (float) * (size_t)tp_stride * C);
+			if (rc) return rc;
+		}
+		ConvParams p;
+		fill_conv_common (h, p);
+		p.inter       = d_x;
+		p.n_frames    = F;
+		p.C           = C;
+		p.m_end       = m_end;
+		p.m_skip      = quirk ? h->Lh / 2 : 0;
+		p.m_zero      = quirk ? h->Lh : 0;
+		p.list        = (float2*)h->d_ovl.p;
+		p.list_stride = lp.cap;
+		p.list_cap    = (unsigned)lp.cap;
+		p.overflow    = d_ovf;
+		p.thr2        = d_thr2;
+		p.rawpeak     = d_rawp;
+		p.thr_mode    = -1;
+		TpParams tp;
+		memset (&tp, 0, sizeof (tp));
+		if (OS > 1) {
+			p.out          = (float2*)h->d_ovH.p;
+			p.out_stride   = tp_stride / 2;
+			p.out_compact  = 1;
+			tp.inter       = d_x;
+			tp.n_frames    = F;
+			tp.C           = C;
+			tp.hist_frames = h->L;
+			tp.H           = (const float*)h->d_ovH.p;
+			tp.h_stride    = tp_stride;
+			tp.seg_stride  = 1;
+			tp.V2          = 2 * h->V;
+			tp.D           = h->L / 2;
+			tp.t_skip      = 2 * p.m_skip;
+			tp.t_zero      = 2 * p.m_zero;
+			tp.t_end       = t_end;
+			tp.os          = OS;
+			tp.list        = p.list;
+			tp.list_stride = p.list_stride;
+			tp.list_cap    = p.list_cap;
+			tp.overflow    = d_ovf;
+			tp.thr2        = d_thr2;
+			tp.rawpeak     = d_rawp;
+		}
+		const SweepCfg sc = pick_sweep_cfg (A);
+		// the Hilbert branch of the segment before s0 -> carry of channels [ch0, ch0 + nch) (zeros at the stream start)
+		auto tp_seed = [&] (long long s0, int ch0, int nch) -> int {
+			if (s0 == 0) {
+				for (int c = ch0; c < ch0 + nch; ++c) CK (cudaMemsetAsync ((float*)h->d_ovH.p + (long long)c * tp_stride, 0, sizeof (float) * kTpCarry, h->stream));
+				return PHASEROT_OK;
+			}
+			p.chan0 = ch0;
+			p.nchan = nch;
+			p.seg0  = s0 - 1;
+			p.nseg  = 1;
+			int r   = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
+			if (r) return r;
+			ProfScope ps (h, 5);
+			tp_carry_kernel<<<nch, 32, 0, h->stream>>> ((float*)h->d_ovH.p, tp_stride, ch0, 2 * h->V);
+			CK (cudaGetLastError ());
+			++h->stats.kernel_launches;
+			return PHASEROT_OK;
+		};
+		// segments [s0, s0 + n) of channels [ch0, ch0 + nch): FFT pass -> list (counters `cnt`) -> overs_kernel
+		auto run_launch = [&] (long long s0, long long n, int ch0, int nch, unsigned* cnt) -> int {
+			p.chan0 = ch0;
+			p.nchan = nch;
+			p.seg0  = s0;
+			p.nseg  = n;
+			p.count = cnt;
+			int r;
+			if (OS > 1) {
+				r = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
+				if (r) return r;
+				tp.chan0 = ch0;
+				tp.seg0  = s0;
+				tp.count = cnt;
+				{
+					ProfScope ps (h, 6);
+					truepeak_kernel<true><<<dim3 ((unsigned)(n * (tp.V2 / kTpTile)), (unsigned)nch), 256, 0, h->stream>>> (tp);
+					CK (cudaGetLastError ());
+				}
+				{
+					ProfScope ps (h, 5);
+					tp_carry_kernel<<<nch, 32, 0, h->stream>>> ((float*)h->d_ovH.p, tp_stride, ch0, n * 2 * h->V);
+					CK (cudaGetLastError ());
+				}
+				h->stats.kernel_launches += 2;
+			} else {
+				r = launch_conv<EPI_POINTS, SRC_INTER> (h, p);
+				if (r) return r;
+			}
+			const long long gx = std::max<long long> (1, (h->n_sm * 8) / std::max<long long> (1, (long long)sc.gy * nch));
+			const dim3      grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)nch);
+			const float2*   lst = (const float2*)h->d_ovl.p;
+			const unsigned  cap = (unsigned)lp.cap;
+			ProfScope       ps (h, 1);
+#define PRK_OVERS(R_, G_) overs_kernel<R_, G_><<<grid, sc.nt, 0, h->stream>>> (lst, lp.cap, cnt, cap, ch0, d_cs, A, T, d_cnt, d_exc, d_eval)
+#define PRK_OVERS_R(G_)                          \
+	switch (sc.R) {                              \
+		case 1: PRK_OVERS (1, G_); break;        \
+		case 2: PRK_OVERS (2, G_); break;        \
+		case 4: PRK_OVERS (4, G_); break;        \
+		default: PRK_OVERS (8, G_); break;       \
+	}
+			if (G == 1) {
+				PRK_OVERS_R (1)
+			} else if (G == 3) {
+				PRK_OVERS_R (3)
+			} else {
+				PRK_OVERS_R (5)
+			}
+#undef PRK_OVERS_R
+#undef PRK_OVERS
+			CK (cudaGetLastError ());
+			++h->stats.kernel_launches;
+			return PHASEROT_OK;
+		};
+
+		// the launches of a device-resident sweep, each with its own list counters
+		if (OS > 1) {
+			rc = tp_seed (0, c0, nchan);
+			if (rc) return rc;
+		}
+		long long seg_done = 0;
+		for (int n_main = 0; seg_done < nseg; ++n_main) {
+			const long long n = std::min (next_launch_segs (n_main, seg_done, nseg, lp.segs_first, lp.segs_max, true), nseg - seg_done);
+			rc                = run_launch (seg_done, n, c0, nchan, d_lcnt + (size_t)n_main * C);
+			if (rc) return rc;
+			l_s0.push_back (seg_done);
+			l_n.push_back (n);
+			seg_done += n;
+		}
+		lcnt.resize (l_s0.size () * C);
+		CK (cudaMemcpyAsync (lcnt.data (), d_lcnt, sizeof (unsigned) * lcnt.size (), cudaMemcpyDeviceToHost, h->stream));
+		CK (cudaStreamSynchronize (h->stream));
+		h->stats.d2h_bytes += sizeof (unsigned) * lcnt.size ();
+
+		// overflowed (launch, channel): overs_kernel skipped it; re-run its segments in pieces that fit the list
+		unsigned*       d_rcnt_l = d_lcnt + (size_t)(n_lmax - 1) * C;
+		const long long fit      = std::max<long long> (1, lp.cap / lp.ppseg);
+		for (size_t k = 0; k < l_s0.size (); ++k) {
+			for (int c = c0; c < c1; ++c) {
+				if (lcnt[k * C + c] <= (unsigned)lp.cap) continue;
+				++h->stats.dense_repeats;
+				for (long long s = l_s0[k]; s < l_s0[k] + l_n[k]; s += fit) {
+					if (OS > 1) {
+						rc = tp_seed (s, c, 1);
+						if (rc) return rc;
+					}
+					CK (cudaMemsetAsync (d_rcnt_l + c, 0, sizeof (unsigned), h->stream));
+					rc = run_launch (s, std::min (fit, l_s0[k] + l_n[k] - s), c, 1, d_rcnt_l);
+					if (rc) return rc;
+				}
+			}
+		}
+	}
+
+	std::vector<unsigned long long> res (n_u64);
+	CK (cudaMemcpyAsync (res.data (), d_cnt, sizeof (unsigned long long) * n_u64, cudaMemcpyDeviceToHost, h->stream));
+	CK (cudaStreamSynchronize (h->stream));
+	prof_resolve (h);
+	h->stats.d2h_bytes += sizeof (unsigned long long) * n_u64;
+	if (A > 0) {
+		h->stats.points_total += (uint64_t)nchan * (uint64_t)(2 * (m_end - (quirk ? h->Lh / 2 : 0))) * (uint64_t)G;
+		h->stats.points_evaluated += res[n_u64 - 1];
+	}
+
+	const size_t MS = (size_t)h->MS;
+	std::fill (counts, counts + (size_t)C * MS, (uint64_t)0);
+	if (excess) std::fill (excess, excess + (size_t)C * MS, 0.0);
+	const double ulp = std::ldexp (1.0, -32);
+	for (int c = c0; c < c1; ++c) {
+		for (int k = 0; k < A; ++k) {
+			const size_t i = (size_t)c * A + k, o = (size_t)c * MS + idx[(size_t)k];
+			counts[o]      = res[i];
+			if (excess) excess[o] = (double)res[n_tab + i] * ulp;
+		}
+		// grid index 0: the raw input; should the schedule also wrap onto index 0, the entry with more overs
+		// (peak[c][0] is the larger of the two peaks)
+		if (raw && res[2 * n_tab + c] >= counts[(size_t)c * MS]) {
+			counts[(size_t)c * MS] = res[2 * n_tab + c];
+			if (excess) excess[(size_t)c * MS] = (double)res[2 * n_tab + C + c] * ulp;
+		}
+	}
+	return PHASEROT_OK;
+}
+
+int
+overs_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t n_frames, float ceiling, int ang_start, int ang_end, int ang_stride, int chn,
+             uint64_t* counts, double* excess)
+{
+	if (!h) {
+		return PHASEROT_E_INVAL;
+	}
+	if (h->plugin) {
+		return PHASEROT_E_STATE;
+	}
+	const char* bad = nullptr;
+	if (!src) bad = "NULL audio";
+	else if (format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) bad = "unknown sample format";
+	else if (n_frames == 0) bad = "n_frames is 0";
+	else if (!(ceiling > 0.f) || !std::isfinite (ceiling)) bad = "the ceiling is not a finite value > 0";
+	else if (!counts) bad = "NULL counts";
+	else if (ang_stride < 1) bad = "ang_stride < 1";
+	else if (chn >= h->C) bad = "chn is not a channel of the handle";
+	if (bad) {
+		snprintf (g_last_error, sizeof (g_last_error), "phaserot_overs: %s", bad);
+		return PHASEROT_E_INVAL;
+	}
+	DevGuard     guard (h->dev);
+	const float* d_x = (const float*)src;
+	if (!dev_in) {
+		// d_inter may still be the source of the pending sweep's dense-mode repeat: complete that sweep first
+		int rc = finish_pending (h);
+		if (rc) return rc;
+		rc = h->d_inter.ensure (sizeof (float) * (size_t)n_frames * h->C);
+		if (rc) return rc;
+		rc = upload_chunks (h, src, format, (long long)n_frames, [] (long long) { return PHASEROT_OK; });
+		if (rc) return rc;
+		d_x = (const float*)h->d_inter.p;
+	}
+	return overs_core (h, d_x, (long long)n_frames, ceiling, ang_start, ang_end, ang_stride, chn, counts, excess);
+}
+
 // Argument checks of the sweep entry points: data may be null for an empty stream only, and every
 // shard of a stream but the last is a whole number of blocks
 int
@@ -2271,7 +2591,7 @@ phaserot_destroy (phaserot_t* h)
 	if (h->copy_stream) cudaStreamSynchronize (h->copy_stream);
 	for (DevBuf* b : { &h->d_G, &h->d_G1, &h->d_scratch, &h->d_tw, &h->d_g, &h->d_plane, &h->d_out, &h->d_list, &h->d_stage[0], &h->d_stage[1], &h->d_io, &h->d_inter, &h->d_hist, &h->d_small,
 	                   &h->d_cs, &h->d_peaks, &h->d_ramp, &h->d_chancs, &h->d_tpH, &h->d_ring, &h->d_slot, &h->d_sec, &h->d_wide,
-	                   &h->d_sect, &h->d_sect_aux, &h->d_sect_rt, &h->d_kx, &h->d_lH, &h->d_lwork, &h->d_lset }) {
+	                   &h->d_sect, &h->d_sect_aux, &h->d_sect_rt, &h->d_kx, &h->d_lH, &h->d_lwork, &h->d_lset, &h->d_ovl, &h->d_ovH, &h->d_ovw }) {
 		b->release ();
 	}
 	for (PinBuf* b : { &h->h_stage[0], &h->h_stage[1], &h->h_res, &h->h_io, &h->h_cs, &h->h_slot }) {
@@ -2782,6 +3102,20 @@ phaserot_loudness_device (phaserot_t* h, const float* d_interleaved, uint64_t n_
                           double* lufs)
 {
 	return loudness_entry (h, d_interleaved, true, PHASEROT_PCM_F32, n_frames, sample_rate, weights, angles, n_sets, lufs);
+}
+
+int
+phaserot_overs (phaserot_t* h, const void* data, int format, uint64_t n_frames, float ceiling, int ang_start, int ang_end, int ang_stride, int chn,
+                uint64_t* counts, double* excess)
+{
+	return overs_entry (h, data, false, format, n_frames, ceiling, ang_start, ang_end, ang_stride, chn, counts, excess);
+}
+
+int
+phaserot_overs_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, float ceiling, int ang_start, int ang_end, int ang_stride, int chn,
+                       uint64_t* counts, double* excess)
+{
+	return overs_entry (h, d_interleaved, true, PHASEROT_PCM_F32, n_frames, ceiling, ang_start, ang_end, ang_stride, chn, counts, excess);
 }
 
 uint32_t

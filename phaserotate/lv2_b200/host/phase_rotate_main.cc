@@ -64,6 +64,8 @@ struct Options {
 	bool         fixed_write = false; // --fixed-write: write loop without the reference's two quirks (cli:985, cli:973)
 	double       sections    = 0;     // --sections SECONDS: one angle per section of the file (0 = one for the whole file)
 	bool         loudness    = false; // --loudness: BS.1770-4 integrated loudness and PLR of the input and of the output
+	bool         overs       = false; // --overs DBFS: samples above the ceiling at the input, the output angle and the best angle
+	double       overs_db    = 0;
 };
 
 // PHASEROT_CLI_TIMING=1: wall-clock breakdown of the process on stderr (file read, CUDA
@@ -176,6 +178,7 @@ parse_options (int argc, char** argv)
 		{ "fixed-write", no_argument, 0, 1003 },
 		{ "sections", required_argument, 0, 1004 },
 		{ "loudness", no_argument, 0, 1005 },
+		{ "overs", required_argument, 0, 1006 },
 		{ 0, 0, 0, 0 },
 	};
 	int c;
@@ -222,6 +225,15 @@ parse_options (int argc, char** argv)
 				break;
 			}
 			case 1005: o.loudness = true; break;
+			case 1006: {
+				char* ep   = nullptr;
+				o.overs    = true;
+				o.overs_db = strtod (optarg, &ep);
+				if (*ep != '\0' || ep == optarg || !std::isfinite (o.overs_db) || o.overs_db < -60 || o.overs_db > 20) {
+					die ("Error: --overs takes a ceiling in dBFS from -60 to 20.\n");
+				}
+				break;
+			}
 			default: die ("Error: unrecognized option. See --help for usage information.\n");
 		}
 	}
@@ -230,6 +242,9 @@ parse_options (int argc, char** argv)
 	}
 	if (o.loudness && (o.angles_arg || o.sections > 0 || o.gpus != 1)) {
 		die ("Error: --loudness cannot be combined with -a, --sections or --gpus.\n");
+	}
+	if (o.overs && (o.sections > 0 || o.gpus != 1)) {
+		die ("Error: --overs cannot be combined with --sections or --gpus.\n");
 	}
 	kSubsample = o.subsample;
 	kMaxSample = 180 * kSubsample;
@@ -745,6 +760,28 @@ main (int argc, char** argv)
 		printf ("Input : %.2f LUFS, PLR %.2f dB\n", lufs[0], to_dB (pk_in) - lufs[0]);
 		printf ("Output: %.2f LUFS, PLR %.2f dB\n", lufs[1], to_dB (pk_out) - lufs[1]);
 		timer.mark ("loudness");
+	}
+
+	if (opt.overs) {
+		// samples above the ceiling at every grid angle (index 0: the input), reported at the input, at the
+		// applied angle (a and a + 180 deg give the same |y|) and at the angle with the fewest
+		const float           T = (float)pow (10.0, opt.overs_db / 20.0);
+		std::vector<uint64_t> n ((size_t)C * kMaxSample, 0);
+		if (F > 0) {
+			check (phaserot_overs (pr, audio, pcm_fmt, F, T, 0, kMaxSample, 1, -1, n.data (), nullptr), "overs failed");
+		}
+		printf ("# Overs -- samples above %.2f %s\n", opt.overs_db, opt.oversample ? "dBTP" : "dBFS");
+		for (int c = 0; c < C; ++c) {
+			const uint64_t* row  = n.data () + (size_t)c * kMaxSample;
+			const int       out  = ((angles[(size_t)c] % kMaxSample) + kMaxSample) % kMaxSample;
+			int             best = 0;
+			for (int a = 1; a < kMaxSample; ++a) {
+				if (row[a] <= row[best]) best = a; // ties: the largest index, like the reference's search
+			}
+			printf ("Channel: %2d Input: %llu Output: %llu Fewest: %llu at %.2f deg\n", c + 1, (unsigned long long)row[0], (unsigned long long)row[out],
+			        (unsigned long long)row[best], best / (float)kSubsample);
+		}
+		timer.mark ("overs");
 	}
 
 	if (outfile) {
