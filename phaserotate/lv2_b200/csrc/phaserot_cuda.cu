@@ -22,6 +22,7 @@
 #include <new>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #ifndef M_PI
@@ -181,20 +182,20 @@ struct SweepJob {
 	bool         on_device   = false;            // src is device memory (float32)
 	int          fmt         = PHASEROT_PCM_F32; // host src: PHASEROT_PCM_*
 	long long    n_frames    = 0;                // frames present in src
-	long long    t_end       = 0;                // the pass examines output samples t in [0, t_end)
+	int          flush       = 0;                // zero blocks after the last (partial) block of src (stream_geom)
 	bool         first_block = false;            // apply the first-block rule (cli:418-419) to t < L
 	const float* hist        = nullptr;          // L frames of history preceding src (interleaved) or null
 	int          ang_start = 0, ang_end = 0, ang_stride = 1, chn = -1;
 };
 
 // The pass over F frames that are a whole stream (first and last) or one shard of it: the last shard ends with
-// one zero flush block (analyze_file, cli:572-586), and the first-block rule applies to the first shard
+// one zero flush block (analyze_file, cli:572-586; every other shard is whole blocks, check_sweep), and the
+// first-block rule applies to the first shard
 SweepJob
-shard_job (int L, const void* src, bool on_device, int fmt, long long F, const float* hist, bool first, bool last, int ang_start, int ang_end,
-           int ang_stride, int chn)
+shard_job (const void* src, bool on_device, int fmt, long long F, const float* hist, bool first, bool last, int ang_start, int ang_end, int ang_stride,
+           int chn)
 {
-	const long long B = (F + L - 1) / L;
-	return { src, on_device, fmt, F, last ? (B + 1) * L : F, first && B > 0, hist, ang_start, ang_end, ang_stride, chn };
+	return { src, on_device, fmt, F, last ? 1 : 0, first && F > 0, hist, ang_start, ang_end, ang_stride, chn };
 }
 
 // d_small: per-channel state of the pending sweep and the render
@@ -439,6 +440,91 @@ fill_conv_common (phaserot* h, ConvParams& p)
 	p.prefetch     = getenv ("PHASEROT_PREFETCH") ? atoi (getenv ("PHASEROT_PREFETCH")) : 0;
 }
 
+// Extent of a pass over F frames followed by `flush_blocks` zero blocks: output samples t < t_end, complex
+// outputs m < m_end in nseg FFT segments; with the first-block rule (cli:418-419) m < m_skip is not examined
+// and the direct branch is zero for m < m_zero.
+struct StreamGeom {
+	long long t_end, m_end, nseg, m_skip, m_zero;
+	// points a pass over nchan channels examines, G per output sample (true-peak: the sample and OS interpolated points)
+	uint64_t points (int nchan, int G) const { return (uint64_t)nchan * (uint64_t)(2 * (m_end - m_skip)) * (uint64_t)G; }
+};
+StreamGeom
+stream_geom (const phaserot* h, long long F, int flush_blocks, bool first_block)
+{
+	StreamGeom g;
+	g.t_end         = ((F + h->L - 1) / h->L + flush_blocks) * h->L;
+	g.m_end         = (g.t_end + 1) / 2;
+	g.nseg          = (g.m_end + h->V - 1) / h->V;
+	const bool rule = first_block && !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK);
+	g.m_skip        = rule ? h->Lh / 2 : 0;
+	g.m_zero        = rule ? h->Lh : 0;
+	return g;
+}
+
+// ConvParams of an analysis pass (EPI_POINTS, EPI_HILBERT, EPI_SECT_POINTS) over F interleaved frames at `inter`
+// (`hist`: frames [-L, 0) or null), channels [c0, c0 + nchan): survivors of the radius thr2 go to `list`, rows of
+// `cap` points counted in `count`
+ConvParams
+analysis_params (phaserot* h, const float* inter, const float* hist, long long F, const StreamGeom& g, int c0, int nchan, float2* list, long long cap,
+                 unsigned* count, unsigned* overflow, const float* thr2, unsigned* rawpeak)
+{
+	ConvParams p;
+	fill_conv_common (h, p);
+	p.inter       = inter;
+	p.hist        = hist;
+	p.n_frames    = F;
+	p.C           = h->C;
+	p.chan0       = c0;
+	p.nchan       = nchan;
+	p.m_end       = g.m_end;
+	p.m_skip      = g.m_skip;
+	p.m_zero      = g.m_zero;
+	p.list        = list;
+	p.list_stride = cap;
+	p.list_cap    = (unsigned)cap;
+	p.count       = count;
+	p.overflow    = overflow;
+	p.thr2        = thr2;
+	p.rawpeak     = rawpeak;
+	return p;
+}
+
+// The true-peak pass over what the analysis pass `p` reads and lists: p's Hilbert branch goes compact to the
+// staging H ([channel][h_stride], kTpCarry carried samples first), and truepeak_kernel reads it from there
+TpParams
+tp_params (const phaserot* h, ConvParams& p, long long t_end, float* H, long long h_stride)
+{
+	p.out         = (float2*)H;
+	p.out_stride  = h_stride / 2;
+	p.out_compact = 1;
+	TpParams tp;
+	memset (&tp, 0, sizeof (tp));
+	tp.inter       = p.inter;
+	tp.hist        = p.hist;
+	tp.n_frames    = p.n_frames;
+	tp.C           = p.C;
+	tp.hist_frames = h->L;
+	tp.H           = H;
+	tp.h_stride    = h_stride;
+	tp.chan0       = p.chan0;
+	tp.seg0        = p.seg0;
+	tp.seg_stride  = p.seg_stride;
+	tp.V2          = 2 * h->V;
+	tp.D           = h->L / 2;
+	tp.t_skip      = 2 * p.m_skip;
+	tp.t_zero      = 2 * p.m_zero;
+	tp.t_end       = t_end;
+	tp.os          = h->OS;
+	tp.list        = p.list;
+	tp.list_stride = p.list_stride;
+	tp.count       = p.count;
+	tp.list_cap    = p.list_cap;
+	tp.overflow    = p.overflow;
+	tp.thr2        = p.thr2;
+	tp.rawpeak     = p.rawpeak;
+	return tp;
+}
+
 // Function attributes are per device (per context): phaserot_create() sets them
 // for every kernel that needs more than the default 48 KB of dynamic shared
 // memory, once per device, under g_create_lock - never on a launch path (an LV2
@@ -523,6 +609,39 @@ int
 launch_conv (phaserot* h, const ConvParams& p)
 {
 	return h->NP == 2 ? launch_conv_np<EPI, SRC, 2> (h, p) : launch_conv_np<EPI, SRC, 1> (h, p);
+}
+
+// true-peak: the last kTpCarry samples of a launch's Hilbert branch (n_samples per channel in the staging H) move
+// to the front of the staging rows of channels [ch0, ch0 + nch), where the next launch's interpolator reads them
+int
+launch_tp_carry (phaserot* h, float* H, long long stride, int ch0, int nch, long long n_samples)
+{
+	ProfScope ps (h, 5);
+	tp_carry_kernel<<<nch, 32, 0, h->stream>>> (H, stride, ch0, n_samples);
+	CK (cudaGetLastError ());
+	++h->stats.kernel_launches;
+	return PHASEROT_OK;
+}
+
+// true-peak: the carry of channels [ch0, ch0 + nch) for a launch from segment s0 on (the interpolator reaches
+// 11 samples back).  At the start of a stream without history it is silence; otherwise one extra segment of
+// `p`'s Hilbert branch ending there seeds it (before the stream start it reads history only: with L frames its
+// last samples lack taps L-16.. of the window edge, which are below 1e-9 (Hann), far inside fp32 rounding of H).
+int
+seed_tp_carry (phaserot* h, ConvParams& p, float* H, long long stride, long long s0, int ch0, int nch)
+{
+	if (s0 == 0 && !p.hist) {
+		for (int c = ch0; c < ch0 + nch; ++c) CK (cudaMemsetAsync (H + (long long)c * stride, 0, sizeof (float) * kTpCarry, h->stream));
+		return PHASEROT_OK;
+	}
+	p.chan0      = ch0;
+	p.nchan      = nch;
+	p.seg0       = s0 - 1;
+	p.seg_stride = 1;
+	p.nseg       = 1;
+	const int rc = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
+	if (rc) return rc;
+	return launch_tp_carry (h, H, stride, ch0, nch, 2 * h->V);
 }
 
 // plane geometry for `m_end` complex outputs per channel
@@ -614,6 +733,23 @@ pick_sweep_cfg (int A)
 	return best;
 }
 
+// Launches a sweep-family kernel (angles in lanes over survivor lists: sweep_kernel, overs_kernel) over `rows`
+// rows of A angles: launch (R, grid, threads), R a std::integral_constant of the angles per thread
+template <class Launch>
+void
+dispatch_sweep (const phaserot* h, int A, int rows, Launch&& launch)
+{
+	const SweepCfg  sc = pick_sweep_cfg (A);
+	const long long gx = std::max<long long> (1, (h->n_sm * 8) / std::max<long long> (1, (long long)sc.gy * rows));
+	const dim3      grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)rows);
+	switch (sc.R) {
+		case 1: launch (std::integral_constant<int, 1> (), grid, sc.nt); break;
+		case 2: launch (std::integral_constant<int, 2> (), grid, sc.nt); break;
+		case 4: launch (std::integral_constant<int, 4> (), grid, sc.nt); break;
+		default: launch (std::integral_constant<int, 8> (), grid, sc.nt); break;
+	}
+}
+
 // Every angle of d_cs over the survivor lists of `rows` rows from row0 on (list, count: [row]), into
 // table [row][A] with a running max.  A bootstrap list is swept even when its count ran past cap (the
 // excess was dropped); any other flagged row is repeated in dense mode, so its full list is skipped.
@@ -622,18 +758,12 @@ launch_sweep (phaserot* h, const float2* lst, long long list_stride, const unsig
               unsigned* table, unsigned long long* n_eval)
 {
 	if (A == 0) return PHASEROT_OK;
-	const SweepCfg  sc = pick_sweep_cfg (A);
-	const long long gx = std::max<long long> (1, (h->n_sm * 8) / std::max<long long> (1, (long long)sc.gy * rows));
-	const dim3      grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)rows);
-	const float2*   cs = (const float2*)h->d_cs.p;
-	const int       so = boot ? 0 : 1;
-	ProfScope       ps (h, 1);
-	switch (sc.R) {
-		case 1: sweep_kernel<1><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
-		case 2: sweep_kernel<2><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
-		case 4: sweep_kernel<4><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
-		default: sweep_kernel<8><<<grid, sc.nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval); break;
-	}
+	const float2* cs = (const float2*)h->d_cs.p;
+	const int     so = boot ? 0 : 1;
+	ProfScope     ps (h, 1);
+	dispatch_sweep (h, A, rows, [&] (auto R, dim3 grid, int nt) {
+		sweep_kernel<decltype (R)::value><<<grid, nt, 0, h->stream>>> (lst, list_stride, count, cap, so, row0, cs, A, table, A, n_eval);
+	});
 	CK (cudaGetLastError ());
 	++h->stats.kernel_launches;
 	return PHASEROT_OK;
@@ -982,6 +1112,26 @@ upload_chunks (phaserot* h, const void* src, int fmt, long long n_frames, Landed
 	return PHASEROT_OK;
 }
 
+// The float32 frames of a synchronous analysis pass on the device (*d_x): device input is read in place and
+// leaves a pending device sweep alone; host input goes to d_inter, which may still be the source of the
+// pending sweep's dense-mode repeat: that sweep is completed first.
+int
+land_input (phaserot* h, const void* src, bool dev_in, int fmt, long long n_frames, const float** d_x)
+{
+	if (dev_in) {
+		*d_x = (const float*)src;
+		return PHASEROT_OK;
+	}
+	int rc = finish_pending (h);
+	if (rc) return rc;
+	rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)n_frames * h->C, 16));
+	if (rc) return rc;
+	rc = upload_chunks (h, src, fmt, n_frames, [] (long long) { return PHASEROT_OK; });
+	if (rc) return rc;
+	*d_x = (const float*)h->d_inter.p;
+	return PHASEROT_OK;
+}
+
 // One analysis pass over a stream (see SweepJob and Pass).
 int
 sweep_core (phaserot* h, SweepJob job, Pass pass)
@@ -1028,9 +1178,9 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 		CK (cudaMemcpyAsync (h->d_slot.p, so, sizeof (int) * (size_t)h->MS, cudaMemcpyHostToDevice, h->stream));
 	}
 
-	const long long m_end = (job.t_end + 1) / 2;
-	const long long nseg  = (m_end + h->V - 1) / h->V;
-	const float*    d_hist = nullptr;
+	const StreamGeom g      = stream_geom (h, job.n_frames, job.flush, job.first_block);
+	const long long  nseg   = g.nseg;
+	const float*     d_hist = nullptr;
 	if (const float* hist = job.hist) {
 		// frames [-L, 0) of the stream, read by the segments that reach before its start
 		cudaPointerAttributes at;
@@ -1064,9 +1214,10 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 		h->tp_stride = (kTpCarry + segs_cap * h->V * 2 + 3) & ~3LL;
 		rc           = h->d_tpH.ensure (sizeof (float) * (size_t)h->tp_stride * h->C);
 		if (rc) return rc;
-		for (int c = c0; c < c1; ++c) { // samples before the stream start are zero
-			CK (cudaMemsetAsync ((float*)h->d_tpH.p + (long long)c * h->tp_stride, 0, sizeof (float) * kTpCarry, h->stream));
-		}
+	}
+	if (!job.on_device) {
+		rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)job.n_frames * h->C, 16));
+		if (rc) return rc;
 	}
 
 	h->pend_idx = idx;
@@ -1075,23 +1226,9 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 	h->pend_c1  = c1;
 	h->pend_A   = A;
 
-	ConvParams p;
-	fill_conv_common (h, p);
-	p.hist     = d_hist;
-	p.n_frames = job.n_frames;
-	p.C        = h->C;
-	p.chan0  = c0;
-	p.nchan  = nchan;
-	p.m_end  = m_end;
-	p.m_skip = (job.first_block && !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK)) ? h->Lh / 2 : 0;
-	p.m_zero = (job.first_block && !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK)) ? h->Lh : 0;
-	p.list        = (float2*)h->d_list.p;
-	p.list_stride = h->list_stride;
-	p.count       = d_count (h);
-	p.list_cap    = (unsigned)h->list_cap;
-	p.overflow    = d_overflow (h);
-	p.thr2        = d_thr2 (h);
-	p.rawpeak     = d_raw (h);
+	const float* d_x = job.on_device ? (const float*)job.src : (const float*)h->d_inter.p;
+	ConvParams   p   = analysis_params (h, d_x, d_hist, job.n_frames, g, c0, nchan, (float2*)h->d_list.p, h->list_cap, d_count (h), d_overflow (h), d_thr2 (h),
+	                                    d_raw (h));
 	const int thr_mode = A == 0 ? 2 : (h->cfg.flags & PHASEROT_FLAG_NO_PRUNE) ? 0 : 1;
 	if (OS > 1) {
 		// true-peak: the radius filter sits in truepeak_kernel and reads thr2 from memory
@@ -1118,42 +1255,12 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 	bool            booted   = thr_mode != 1 || redo; // a repeat starts from the table the first attempt reached
 	int             n_main   = 0; // contiguous launches so far
 
-	TpParams tp;
-	memset (&tp, 0, sizeof (tp));
-	if (OS > 1) {
-		p.out         = (float2*)h->d_tpH.p;
-		p.out_stride  = h->tp_stride / 2;
-		p.out_compact = 1;
-		tp.hist        = d_hist;
-		tp.n_frames    = job.n_frames;
-		tp.C           = h->C;
-		tp.hist_frames = h->L;
-		tp.H           = (const float*)h->d_tpH.p;
-		tp.h_stride    = h->tp_stride;
-		tp.chan0       = c0;
-		tp.V2          = 2 * h->V;
-		tp.D           = h->L / 2;
-		tp.t_skip      = 2 * p.m_skip;
-		tp.t_zero      = 2 * p.m_zero;
-		tp.t_end       = job.t_end;
-		tp.os          = OS;
-		tp.list        = p.list;
-		tp.list_stride = p.list_stride;
-		tp.count       = p.count;
-		tp.list_cap    = p.list_cap;
-		tp.overflow    = p.overflow;
-		tp.thr2        = p.thr2;
-		tp.rawpeak     = p.rawpeak;
-		tp.r2max       = d_r2max (h);
-	}
 	// true-peak: Hilbert branch of the launch -> staging, carry of the last samples to the next launch
-	auto tp_carry = [&] (long long n) -> int {
-		ProfScope ps (h, 5);
-		tp_carry_kernel<<<nchan, 32, 0, h->stream>>> ((float*)h->d_tpH.p, h->tp_stride, c0, n * 2 * h->V);
-		CK (cudaGetLastError ());
-		++h->stats.kernel_launches;
-		return PHASEROT_OK;
-	};
+	TpParams tp {};
+	if (OS > 1) {
+		tp       = tp_params (h, p, g.t_end, (float*)h->d_tpH.p, h->tp_stride);
+		tp.r2max = d_r2max (h);
+	}
 
 	// every angle over the survivors of one launch.  Normal mode: angles in lanes over the
 	// (short) list.  Dense mode: sector thresholds, then one thread per point over the few
@@ -1241,7 +1348,6 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 			p.r2max      = boot ? d_r2max (h) : nullptr;
 			r = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
 			if (r) return r;
-			tp.inter      = p.inter;
 			tp.seg0       = s0;
 			tp.seg_stride = stride;
 			tp.seg_jitter = p.seg_jitter;
@@ -1256,7 +1362,7 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 				++h->stats.kernel_launches;
 			}
 			if (stride == 1) {
-				r = tp_carry (n);
+				r = launch_tp_carry (h, (float*)h->d_tpH.p, h->tp_stride, c0, nchan, n * 2 * h->V);
 				if (r) return r;
 			}
 		} else {
@@ -1285,21 +1391,6 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 		CK (cudaGetLastError ());
 		++h->stats.kernel_launches;
 		return PHASEROT_OK;
-	};
-
-	// true-peak on a continued stream: the interpolator reaches 11 samples back,
-	// so the Hilbert branch just before the stream position 0 is needed once: one
-	// extra segment ending there (it reads history only) seeds the carry.  With L
-	// frames of history its last samples lack taps L-16.. of the window edge,
-	// which are below 1e-9 (Hann), far inside fp32 rounding of H.
-	auto tp_head = [&] () -> int {
-		if (OS <= 1 || !d_hist) return PHASEROT_OK;
-		p.seg0       = -1;
-		p.seg_stride = 1;
-		p.nseg       = 1;
-		const int r  = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
-		if (r) return r;
-		return tp_carry (1);
 	};
 
 	auto process_ready = [&] (bool final) -> int {
@@ -1335,21 +1426,17 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 		return PHASEROT_OK;
 	};
 
-	if (job.on_device) {
-		p.inter      = (const float*)job.src;
-		frames_ready = job.n_frames;
-		rc           = tp_head ();
+	if (OS > 1) {
+		rc = seed_tp_carry (h, p, (float*)h->d_tpH.p, h->tp_stride, 0, c0, nchan);
 		if (rc) return rc;
+	}
+	if (job.on_device) {
+		frames_ready = job.n_frames;
 		rc           = process_ready (true);
 		if (rc) return rc;
 	} else {
 		// H2D in chunks on the copy stream straight into the device copy of the
 		// file; the compute stream starts on a chunk as soon as it has landed
-		rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)job.n_frames * h->C, 16));
-		if (rc) return rc;
-		p.inter = (const float*)h->d_inter.p;
-		rc      = tp_head ();
-		if (rc) return rc;
 		rc = upload_chunks (h, job.src, job.fmt, job.n_frames, [&] (long long f) {
 			frames_ready = f;
 			return process_ready (false);
@@ -1362,11 +1449,11 @@ sweep_core (phaserot* h, SweepJob job, Pass pass)
 		h->pend_again   = 0;
 		h->pend_exposed = false;
 		h->pend_redone  = false;
-		h->pend_points = (uint64_t)nchan * (uint64_t)(2 * (m_end - p.m_skip)) * (uint64_t)(OS > 1 ? OS + 1 : 1);
+		h->pend_points  = g.points (nchan, OS > 1 ? OS + 1 : 1);
 		h->stats.points_total += h->pend_points;
 		// the device-resident form of this pass, should it have to be repeated or resumed
 		h->redo           = job;
-		h->redo.src       = p.inter;
+		h->redo.src       = d_x;
 		h->redo.on_device = true;
 		h->redo.fmt       = PHASEROT_PCM_F32;
 		h->redo.hist      = d_hist;
@@ -1435,14 +1522,12 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 	h->sect_redo_k.clear ();
 	h->sect_redo.clear ();
 
-	const int       A     = (int)idx.size ();
-	const long long R     = n_sect * nchan;
-	const long long B     = (n_frames + h->L - 1) / h->L;
-	const long long t_end = (B + 1) * h->L; // B blocks + the zero flush block, like phaserot_sweep
-	const long long m_end = (t_end + 1) / 2;
-	const long long nseg  = (m_end + h->V - 1) / h->V;
-	const long long sps   = S / (2 * (long long)h->V); // segments per section
-	const long long last_segs = nseg - (n_sect - 1) * sps;
+	const int        A         = (int)idx.size ();
+	const long long  R         = n_sect * nchan;
+	const StreamGeom g         = stream_geom (h, n_frames, 1, true); // like phaserot_sweep
+	const long long  nseg      = g.nseg;
+	const long long  sps       = S / (2 * (long long)h->V); // segments per section
+	const long long  last_segs = nseg - (n_sect - 1) * sps;
 
 	// survivor lists, pooled: 1/32 of the points of a row (the largest one: the last section takes the remainder
 	// and the flush block), at least 8 K points.  Rows only ever receive points of their own section, so a row's
@@ -1450,9 +1535,11 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 	const long long cap = std::max<long long> (8192, 2 * (long long)h->V * std::max (sps, last_segs) / 32);
 	rc = h->d_list.ensure ((size_t)(R * cap) * sizeof (float2));
 	if (rc) return rc;
-	rc = h->d_sect.ensure (sizeof (unsigned) * (size_t)(R * std::max (A, 1) + R));
+	const size_t sect_bytes = sizeof (unsigned) * (size_t)(R * std::max (A, 1) + R);
+	const size_t aux_bytes  = sizeof (unsigned long long) + sizeof (unsigned) * 5 * (size_t)R;
+	rc                      = h->d_sect.ensure (sect_bytes);
 	if (rc) return rc;
-	rc = h->d_sect_aux.ensure (sizeof (unsigned long long) + sizeof (unsigned) * 5 * (size_t)R);
+	rc = h->d_sect_aux.ensure (aux_bytes);
 	if (rc) return rc;
 	unsigned*           table = (unsigned*)h->d_sect.p;
 	unsigned*           rawpk = table + (size_t)R * A;
@@ -1462,42 +1549,22 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 	unsigned*           ovf   = count + R;
 	unsigned*           ovf_b = ovf + R;
 	unsigned*           r2max = ovf_b + R;
-	CK (cudaMemsetAsync (h->d_sect.p, 0, sizeof (unsigned) * (size_t)(R * std::max (A, 1) + R), h->stream));
-	CK (cudaMemsetAsync (h->d_sect_aux.p, 0, sizeof (unsigned long long) + sizeof (unsigned) * 5 * (size_t)R, h->stream));
+	CK (cudaMemsetAsync (h->d_sect.p, 0, sect_bytes, h->stream));
+	CK (cudaMemsetAsync (h->d_sect_aux.p, 0, aux_bytes, h->stream));
 	rc = upload_angle_table (h, idx);
 	if (rc) return rc;
 
-	const float* d_src = src;
-	if (!src_is_device) {
-		// the bootstrap wave samples every section, so the pass starts once the whole stream has landed
-		rc = h->d_inter.ensure (std::max<size_t> (sizeof (float) * (size_t)n_frames * h->C, 16));
-		if (rc) return rc;
-		rc = upload_chunks (h, src, fmt, n_frames, [] (long long) { return PHASEROT_OK; });
-		if (rc) return rc;
-		d_src = (const float*)h->d_inter.p;
-	}
+	// the bootstrap wave samples every section, so the pass starts once the whole stream has landed
+	const float* d_src;
+	rc = land_input (h, src, src_is_device, fmt, n_frames, &d_src);
+	if (rc) return rc;
 
 	const bool no_prune = (h->cfg.flags & PHASEROT_FLAG_NO_PRUNE) != 0;
 	const int  thr_mode = A == 0 ? 2 : no_prune ? 0 : 1;
-	ConvParams p;
-	fill_conv_common (h, p);
-	p.inter       = d_src;
-	p.n_frames    = n_frames;
-	p.C           = h->C;
-	p.chan0       = c0;
-	p.nchan       = nchan;
-	p.m_end       = m_end;
-	p.m_skip      = !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK) ? h->Lh / 2 : 0;
-	p.m_zero      = !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK) ? h->Lh : 0;
-	p.list        = (float2*)h->d_list.p;
-	p.list_stride = cap;
-	p.list_cap    = (unsigned)cap;
-	p.count       = count;
-	p.thr2        = thr2;
-	p.rawpeak     = rawpk;
-	p.r2max       = r2max;
-	p.sect_segs   = sps;
-	p.n_sect      = (int)n_sect;
+	ConvParams p        = analysis_params (h, d_src, nullptr, n_frames, g, c0, nchan, (float2*)h->d_list.p, cap, count, ovf, thr2, rawpk);
+	p.r2max             = r2max;
+	p.sect_segs         = sps;
+	p.n_sect            = (int)n_sect;
 
 	// new radius of every row from its running peaks; zeroes the list counters
 	auto thresholds = [&] () -> int {
@@ -1534,11 +1601,10 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 	p.seg_stride = 1;
 	p.boot_beta  = 0.f;
 	p.overflow   = ovf;
-	static const SegsKnobs knobs;
-	const long long segs_first = std::max<long long> (1, ((long long)h->n_sm * knobs.first) / nchan);
-	long long       seg_done   = 0;
+	const ListPlan lp       = plan_lists (h, nchan, nseg, true, false);
+	long long      seg_done = 0;
 	for (int n_main = 0; seg_done < nseg; ++n_main) {
-		const long long n = std::min (next_launch_segs (n_main, seg_done, nseg, segs_first, knobs.mult * segs_first, true), nseg - seg_done);
+		const long long n = std::min (next_launch_segs (n_main, seg_done, nseg, lp.segs_first, lp.segs_max, true), nseg - seg_done);
 		rc = thresholds ();
 		if (rc) return rc;
 		p.seg0 = seg_done;
@@ -1557,7 +1623,7 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 	CK (cudaMemcpyAsync (&evaluated, n_ev, sizeof (evaluated), cudaMemcpyDeviceToHost, h->stream));
 	CK (cudaStreamSynchronize (h->stream));
 	prof_resolve (h);
-	h->stats.points_total += (uint64_t)nchan * (uint64_t)(2 * (m_end - p.m_skip));
+	h->stats.points_total += g.points (nchan, 1);
 	h->stats.points_evaluated += evaluated;
 	h->sect_n   = n_sect;
 	h->sect_A   = A;
@@ -1577,7 +1643,7 @@ sweep_sections_core (phaserot* h, const float* src, bool src_is_device, int fmt,
 		h->dense_mode       = true;
 		const long long f0  = k * S;
 		const long long F   = std::min (S, n_frames - f0);
-		rc = sweep_core (h, shard_job (h->L, d_src + (size_t)f0 * h->C, true, PHASEROT_PCM_F32, F, k ? d_src + (size_t)(f0 - h->L) * h->C : nullptr, k == 0, k == n_sect - 1,
+		rc = sweep_core (h, shard_job (d_src + (size_t)f0 * h->C, true, PHASEROT_PCM_F32, F, k ? d_src + (size_t)(f0 - h->L) * h->C : nullptr, k == 0, k == n_sect - 1,
 		                               ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 		if (!rc) rc = finish_pending (h);
 		if (!rc) {
@@ -1833,9 +1899,11 @@ loudness_core (phaserot* h, const float* d_x, long long F, double fs, const floa
 	return PHASEROT_OK;
 }
 
+// Argument checks of the synchronous analysis entry points: the handle, the audio, its sample format and length,
+// then the entry's own (`more`: the first of them that fails, or null).  A failed check sets "<entry>: <check>".
+template <class More>
 int
-loudness_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t n_frames, double fs, const float* weights, const int* angles, int n_sets,
-                double* lufs)
+check_analysis (const phaserot* h, const void* src, int format, uint64_t n_frames, const char* entry, More&& more)
 {
 	if (!h) {
 		return PHASEROT_E_INVAL;
@@ -1847,28 +1915,32 @@ loudness_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t 
 	if (!src) bad = "NULL audio";
 	else if (format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) bad = "unknown sample format";
 	else if (n_frames == 0) bad = "n_frames is 0";
-	else if (!(fs >= 8000.0 && fs <= 768000.0)) bad = "sample_rate outside [8000, 768000]";
-	else if (n_sets < 1) bad = "n_sets < 1";
-	else if (!angles || !lufs) bad = "NULL angles or lufs";
-	for (int c = 0; !bad && weights && c < h->C; ++c) {
-		if (!std::isfinite (weights[c]) || weights[c] < 0.f) bad = "a channel weight is negative or not finite";
-	}
+	else bad = more ();
 	if (bad) {
-		snprintf (g_last_error, sizeof (g_last_error), "phaserot_loudness: %s", bad);
+		snprintf (g_last_error, sizeof (g_last_error), "%s: %s", entry, bad);
 		return PHASEROT_E_INVAL;
 	}
+	return PHASEROT_OK;
+}
+
+int
+loudness_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t n_frames, double fs, const float* weights, const int* angles, int n_sets,
+                double* lufs)
+{
+	int rc = check_analysis (h, src, format, n_frames, "phaserot_loudness", [&] () -> const char* {
+		if (!(fs >= 8000.0 && fs <= 768000.0)) return "sample_rate outside [8000, 768000]";
+		if (n_sets < 1) return "n_sets < 1";
+		if (!angles || !lufs) return "NULL angles or lufs";
+		for (int c = 0; weights && c < h->C; ++c) {
+			if (!std::isfinite (weights[c]) || weights[c] < 0.f) return "a channel weight is negative or not finite";
+		}
+		return nullptr;
+	});
+	if (rc) return rc;
 	DevGuard     guard (h->dev);
-	const float* d_x = (const float*)src;
-	if (!dev_in) {
-		// d_inter may still be the source of the pending sweep's dense-mode repeat: complete that sweep first
-		int rc = finish_pending (h);
-		if (rc) return rc;
-		rc = h->d_inter.ensure (sizeof (float) * (size_t)n_frames * h->C);
-		if (rc) return rc;
-		rc = upload_chunks (h, src, format, (long long)n_frames, [] (long long) { return PHASEROT_OK; });
-		if (rc) return rc;
-		d_x = (const float*)h->d_inter.p;
-	}
+	const float* d_x;
+	rc = land_input (h, src, dev_in, format, (long long)n_frames, &d_x);
+	if (rc) return rc;
 	return loudness_core (h, d_x, (long long)n_frames, fs, weights, angles, n_sets, lufs);
 }
 
@@ -1979,7 +2051,7 @@ flush_analyze (phaserot* h)
 		return PHASEROT_OK;
 	}
 	const long long frames = (long long)h->an_blocks * h->L;
-	const SweepJob  job { h->an_buf.data (), false, PHASEROT_PCM_F32, frames, frames, h->an_first != 0, h->hist_valid ? h->hist.data () : nullptr,
+	const SweepJob  job { h->an_buf.data (), false, PHASEROT_PCM_F32, frames, 0, h->an_first != 0, h->hist_valid ? h->hist.data () : nullptr,
                          h->an_start, h->an_end, h->an_stride, h->an_chn };
 	const int rc = sweep_core (h, job, Pass::Fresh);
 	if (rc) return rc;
@@ -2007,21 +2079,18 @@ overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, 
 	bool             raw = false;
 	int              rc  = angle_schedule (h, ang_start, ang_end, ang_stride, idx, raw);
 	if (rc) return rc;
-	const int       C     = h->C;
-	const int       A     = (int)idx.size ();
-	const int       c0    = chn < 0 ? 0 : chn;
-	const int       c1    = chn < 0 ? C : chn + 1;
-	const int       nchan = c1 - c0;
-	const int       OS    = h->OS;
-	const int       G     = OS > 1 ? OS + 1 : 1; // points per record
-	const long long B     = (F + h->L - 1) / h->L;
-	const long long t_end = (B + 1) * h->L;      // B blocks + the zero flush block, like phaserot_sweep
-	const long long m_end = (t_end + 1) / 2;
-	const long long nseg  = (m_end + h->V - 1) / h->V;
-	const bool      quirk    = !(h->cfg.flags & PHASEROT_FLAG_NO_FIRST_BLOCK_QUIRK);
-	const bool      no_prune = (h->cfg.flags & PHASEROT_FLAG_NO_PRUNE) != 0;
-	const ListPlan  lp       = plan_lists (h, nchan, nseg, true, no_prune);
-	const long long n_lmax = nseg / lp.segs_first + 3; // launches of the schedule (+ 1 counter set for the re-runs)
+	const int        C        = h->C;
+	const int        A        = (int)idx.size ();
+	const int        c0       = chn < 0 ? 0 : chn;
+	const int        c1       = chn < 0 ? C : chn + 1;
+	const int        nchan    = c1 - c0;
+	const int        OS       = h->OS;
+	const int        G        = OS > 1 ? OS + 1 : 1;          // points per record
+	const StreamGeom g        = stream_geom (h, F, 1, true); // like phaserot_sweep
+	const long long  nseg     = g.nseg;
+	const bool       no_prune = (h->cfg.flags & PHASEROT_FLAG_NO_PRUNE) != 0;
+	const ListPlan   lp       = plan_lists (h, nchan, nseg, true, no_prune);
+	const long long  n_lmax   = nseg / lp.segs_first + 3; // launches of the schedule (+ 1 counter set for the re-runs)
 
 	// work area: u64 counts [C][A] | u64 excess [C][A] | u64 raw counts [C] | u64 raw excess [C] | u64 evaluated |
 	// (ca, sa) [A] | thr2 [C] | raw peaks [C] (unused) | overflow word (unused) | list counters [n_lmax][C]
@@ -2053,7 +2122,7 @@ overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, 
 
 	// grid index 0: the raw input (the interpolator reaches 11 frames past the last one)
 	if (raw) {
-		const long long f_end = std::min (F + (OS > 1 ? 11 : 0), t_end - h->L / 2);
+		const long long f_end = std::min (F + (OS > 1 ? 11 : 0), g.t_end - h->L / 2);
 		const long long nb    = std::min<long long> ((f_end + 255) / 256, (long long)h->n_sm * 8);
 		ProfScope       ps (h, 5);
 		overs_raw_kernel<<<dim3 ((unsigned)nb, (unsigned)nchan), 256, 0, h->stream>>> (d_x, F, C, c0, f_end, OS, T, d_rcnt, d_rexc);
@@ -2071,66 +2140,11 @@ overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, 
 			rc = h->d_ovH.ensure (sizeof (float) * (size_t)tp_stride * C);
 			if (rc) return rc;
 		}
-		ConvParams p;
-		fill_conv_common (h, p);
-		p.inter       = d_x;
-		p.n_frames    = F;
-		p.C           = C;
-		p.m_end       = m_end;
-		p.m_skip      = quirk ? h->Lh / 2 : 0;
-		p.m_zero      = quirk ? h->Lh : 0;
-		p.list        = (float2*)h->d_ovl.p;
-		p.list_stride = lp.cap;
-		p.list_cap    = (unsigned)lp.cap;
-		p.overflow    = d_ovf;
-		p.thr2        = d_thr2;
-		p.rawpeak     = d_rawp;
-		p.thr_mode    = -1;
-		TpParams tp;
-		memset (&tp, 0, sizeof (tp));
-		if (OS > 1) {
-			p.out          = (float2*)h->d_ovH.p;
-			p.out_stride   = tp_stride / 2;
-			p.out_compact  = 1;
-			tp.inter       = d_x;
-			tp.n_frames    = F;
-			tp.C           = C;
-			tp.hist_frames = h->L;
-			tp.H           = (const float*)h->d_ovH.p;
-			tp.h_stride    = tp_stride;
-			tp.seg_stride  = 1;
-			tp.V2          = 2 * h->V;
-			tp.D           = h->L / 2;
-			tp.t_skip      = 2 * p.m_skip;
-			tp.t_zero      = 2 * p.m_zero;
-			tp.t_end       = t_end;
-			tp.os          = OS;
-			tp.list        = p.list;
-			tp.list_stride = p.list_stride;
-			tp.list_cap    = p.list_cap;
-			tp.overflow    = d_ovf;
-			tp.thr2        = d_thr2;
-			tp.rawpeak     = d_rawp;
-		}
-		const SweepCfg sc = pick_sweep_cfg (A);
-		// the Hilbert branch of the segment before s0 -> carry of channels [ch0, ch0 + nch) (zeros at the stream start)
-		auto tp_seed = [&] (long long s0, int ch0, int nch) -> int {
-			if (s0 == 0) {
-				for (int c = ch0; c < ch0 + nch; ++c) CK (cudaMemsetAsync ((float*)h->d_ovH.p + (long long)c * tp_stride, 0, sizeof (float) * kTpCarry, h->stream));
-				return PHASEROT_OK;
-			}
-			p.chan0 = ch0;
-			p.nchan = nch;
-			p.seg0  = s0 - 1;
-			p.nseg  = 1;
-			int r   = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
-			if (r) return r;
-			ProfScope ps (h, 5);
-			tp_carry_kernel<<<nch, 32, 0, h->stream>>> ((float*)h->d_ovH.p, tp_stride, ch0, 2 * h->V);
-			CK (cudaGetLastError ());
-			++h->stats.kernel_launches;
-			return PHASEROT_OK;
-		};
+		float*     H = (float*)h->d_ovH.p;
+		ConvParams p = analysis_params (h, d_x, nullptr, F, g, c0, nchan, (float2*)h->d_ovl.p, lp.cap, nullptr, d_ovf, d_thr2, d_rawp);
+		p.thr_mode   = -1;
+		TpParams tp {};
+		if (OS > 1) tp = tp_params (h, p, g.t_end, H, tp_stride);
 		// segments [s0, s0 + n) of channels [ch0, ch0 + nch): FFT pass -> list (counters `cnt`) -> overs_kernel
 		auto run_launch = [&] (long long s0, long long n, int ch0, int nch, unsigned* cnt) -> int {
 			p.chan0 = ch0;
@@ -2149,39 +2163,25 @@ overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, 
 					ProfScope ps (h, 6);
 					truepeak_kernel<true><<<dim3 ((unsigned)(n * (tp.V2 / kTpTile)), (unsigned)nch), 256, 0, h->stream>>> (tp);
 					CK (cudaGetLastError ());
+					++h->stats.kernel_launches;
 				}
-				{
-					ProfScope ps (h, 5);
-					tp_carry_kernel<<<nch, 32, 0, h->stream>>> ((float*)h->d_ovH.p, tp_stride, ch0, n * 2 * h->V);
-					CK (cudaGetLastError ());
-				}
-				h->stats.kernel_launches += 2;
+				r = launch_tp_carry (h, H, tp_stride, ch0, nch, n * 2 * h->V);
+				if (r) return r;
 			} else {
 				r = launch_conv<EPI_POINTS, SRC_INTER> (h, p);
 				if (r) return r;
 			}
-			const long long gx = std::max<long long> (1, (h->n_sm * 8) / std::max<long long> (1, (long long)sc.gy * nch));
-			const dim3      grid ((unsigned)gx, (unsigned)sc.gy, (unsigned)nch);
-			const float2*   lst = (const float2*)h->d_ovl.p;
-			const unsigned  cap = (unsigned)lp.cap;
-			ProfScope       ps (h, 1);
-#define PRK_OVERS(R_, G_) overs_kernel<R_, G_><<<grid, sc.nt, 0, h->stream>>> (lst, lp.cap, cnt, cap, ch0, d_cs, A, T, d_cnt, d_exc, d_eval)
-#define PRK_OVERS_R(G_)                          \
-	switch (sc.R) {                              \
-		case 1: PRK_OVERS (1, G_); break;        \
-		case 2: PRK_OVERS (2, G_); break;        \
-		case 4: PRK_OVERS (4, G_); break;        \
-		default: PRK_OVERS (8, G_); break;       \
-	}
-			if (G == 1) {
-				PRK_OVERS_R (1)
-			} else if (G == 3) {
-				PRK_OVERS_R (3)
-			} else {
-				PRK_OVERS_R (5)
-			}
-#undef PRK_OVERS_R
-#undef PRK_OVERS
+			const float2*  lst = (const float2*)h->d_ovl.p;
+			const unsigned cap = (unsigned)lp.cap;
+			ProfScope      ps (h, 1);
+			auto overs = [&] (auto G_) {
+				dispatch_sweep (h, A, nch, [&] (auto R, dim3 grid, int nt) {
+					overs_kernel<decltype (R)::value, decltype (G_)::value><<<grid, nt, 0, h->stream>>> (lst, lp.cap, cnt, cap, ch0, d_cs, A, T, d_cnt, d_exc, d_eval);
+				});
+			};
+			if (G == 1) overs (std::integral_constant<int, 1> ());
+			else if (G == 3) overs (std::integral_constant<int, 3> ());
+			else overs (std::integral_constant<int, 5> ());
 			CK (cudaGetLastError ());
 			++h->stats.kernel_launches;
 			return PHASEROT_OK;
@@ -2189,7 +2189,7 @@ overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, 
 
 		// the launches of a device-resident sweep, each with its own list counters
 		if (OS > 1) {
-			rc = tp_seed (0, c0, nchan);
+			rc = seed_tp_carry (h, p, H, tp_stride, 0, c0, nchan);
 			if (rc) return rc;
 		}
 		long long seg_done = 0;
@@ -2215,7 +2215,7 @@ overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, 
 				++h->stats.dense_repeats;
 				for (long long s = l_s0[k]; s < l_s0[k] + l_n[k]; s += fit) {
 					if (OS > 1) {
-						rc = tp_seed (s, c, 1);
+						rc = seed_tp_carry (h, p, H, tp_stride, s, c, 1);
 						if (rc) return rc;
 					}
 					CK (cudaMemsetAsync (d_rcnt_l + c, 0, sizeof (unsigned), h->stream));
@@ -2232,7 +2232,7 @@ overs_core (phaserot* h, const float* d_x, long long F, float T, int ang_start, 
 	prof_resolve (h);
 	h->stats.d2h_bytes += sizeof (unsigned long long) * n_u64;
 	if (A > 0) {
-		h->stats.points_total += (uint64_t)nchan * (uint64_t)(2 * (m_end - (quirk ? h->Lh / 2 : 0))) * (uint64_t)G;
+		h->stats.points_total += g.points (nchan, G);
 		h->stats.points_evaluated += res[n_u64 - 1];
 	}
 
@@ -2260,36 +2260,18 @@ int
 overs_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t n_frames, float ceiling, int ang_start, int ang_end, int ang_stride, int chn,
              uint64_t* counts, double* excess)
 {
-	if (!h) {
-		return PHASEROT_E_INVAL;
-	}
-	if (h->plugin) {
-		return PHASEROT_E_STATE;
-	}
-	const char* bad = nullptr;
-	if (!src) bad = "NULL audio";
-	else if (format < PHASEROT_PCM_F32 || format > PHASEROT_PCM_S24) bad = "unknown sample format";
-	else if (n_frames == 0) bad = "n_frames is 0";
-	else if (!(ceiling > 0.f) || !std::isfinite (ceiling)) bad = "the ceiling is not a finite value > 0";
-	else if (!counts) bad = "NULL counts";
-	else if (ang_stride < 1) bad = "ang_stride < 1";
-	else if (chn >= h->C) bad = "chn is not a channel of the handle";
-	if (bad) {
-		snprintf (g_last_error, sizeof (g_last_error), "phaserot_overs: %s", bad);
-		return PHASEROT_E_INVAL;
-	}
+	int rc = check_analysis (h, src, format, n_frames, "phaserot_overs", [&] () -> const char* {
+		if (!(ceiling > 0.f) || !std::isfinite (ceiling)) return "the ceiling is not a finite value > 0";
+		if (!counts) return "NULL counts";
+		if (ang_stride < 1) return "ang_stride < 1";
+		if (chn >= h->C) return "chn is not a channel of the handle";
+		return nullptr;
+	});
+	if (rc) return rc;
 	DevGuard     guard (h->dev);
-	const float* d_x = (const float*)src;
-	if (!dev_in) {
-		// d_inter may still be the source of the pending sweep's dense-mode repeat: complete that sweep first
-		int rc = finish_pending (h);
-		if (rc) return rc;
-		rc = h->d_inter.ensure (sizeof (float) * (size_t)n_frames * h->C);
-		if (rc) return rc;
-		rc = upload_chunks (h, src, format, (long long)n_frames, [] (long long) { return PHASEROT_OK; });
-		if (rc) return rc;
-		d_x = (const float*)h->d_inter.p;
-	}
+	const float* d_x;
+	rc = land_input (h, src, dev_in, format, (long long)n_frames, &d_x);
+	if (rc) return rc;
 	return overs_core (h, d_x, (long long)n_frames, ceiling, ang_start, ang_end, ang_stride, chn, counts, excess);
 }
 
@@ -2654,7 +2636,7 @@ phaserot_sweep (phaserot_t* h, const float* interleaved, uint64_t n_frames, int 
 	int rc = check_sweep (h, interleaved, n_frames);
 	if (rc) return rc;
 	DevGuard guard (h->dev);
-	rc = sweep_core (h, shard_job (h->L, interleaved, false, PHASEROT_PCM_F32, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn),
+	rc = sweep_core (h, shard_job (interleaved, false, PHASEROT_PCM_F32, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn),
 	                 Pass::Fresh);
 	if (rc) return rc;
 	return finish_pending (h);
@@ -2669,7 +2651,7 @@ phaserot_sweep_pcm (phaserot_t* h, const void* pcm, int format, uint64_t n_frame
 	int rc = check_sweep (h, pcm, n_frames);
 	if (rc) return rc;
 	DevGuard guard (h->dev);
-	rc = sweep_core (h, shard_job (h->L, pcm, false, format, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
+	rc = sweep_core (h, shard_job (pcm, false, format, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 	if (rc) return rc;
 	return finish_pending (h);
 }
@@ -2680,7 +2662,7 @@ phaserot_sweep_device (phaserot_t* h, const float* d_interleaved, uint64_t n_fra
 	const int rc = check_sweep (h, d_interleaved, n_frames);
 	if (rc) return rc;
 	DevGuard guard (h->dev);
-	return sweep_core (h, shard_job (h->L, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn),
+	return sweep_core (h, shard_job (d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, nullptr, true, true, ang_start, ang_end, ang_stride, chn),
 	                   Pass::Fresh);
 }
 
@@ -2771,7 +2753,7 @@ phaserot_sweep_shard_device (phaserot_t* h, const float* d_interleaved, uint64_t
 	const int rc = check_sweep (h, d_interleaved, n_frames, last != 0);
 	if (rc) return rc;
 	DevGuard guard (h->dev);
-	return sweep_core (h, shard_job (h->L, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn),
+	return sweep_core (h, shard_job (d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn),
 	                   Pass::Fresh);
 }
 
@@ -2782,7 +2764,7 @@ phaserot_sweep_shard_boot_device (phaserot_t* h, const float* d_interleaved, uin
 	const int rc = check_sweep (h, d_interleaved, n_frames, last != 0);
 	if (rc) return rc;
 	DevGuard guard (h->dev);
-	return sweep_core (h, shard_job (h->L, d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn),
+	return sweep_core (h, shard_job (d_interleaved, true, PHASEROT_PCM_F32, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn),
 	                   Pass::BootOnly);
 }
 
@@ -2809,7 +2791,7 @@ phaserot_sweep_shard (phaserot_t* h, const void* data, int format, uint64_t n_fr
 	const int rc = check_sweep (h, data, n_frames, last != 0);
 	if (rc) return rc;
 	DevGuard guard (h->dev);
-	return sweep_core (h, shard_job (h->L, data, false, format, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
+	return sweep_core (h, shard_job (data, false, format, (long long)n_frames, hist, first != 0, last != 0, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 }
 
 int
@@ -2934,7 +2916,7 @@ render_bulk (phaserot* h, const float* src, bool dev_in, uint64_t n_frames, cons
 	angles_to_cs (h, angles, cs);
 	const long long F     = (long long)n_frames;
 	const long long B     = (F + h->L - 1) / h->L;
-	const long long t_end = (B + flush_blocks) * h->L;
+	const long long t_end = stream_geom (h, F, flush_blocks, false).t_end;
 	if (t_end == 0) {
 		return PHASEROT_OK;
 	}
@@ -3049,8 +3031,7 @@ render_sections_bulk (phaserot* h, const float* src, bool dev_in, uint64_t n_fra
 	long long       n_sect;
 	int             rc = check_sections (h, F, (long long)section_frames, h->C, &n_sect);
 	if (rc) return rc;
-	const long long B     = (F + h->L - 1) / h->L;
-	const long long t_end = (B + flush_blocks) * h->L;
+	const long long t_end = stream_geom (h, F, flush_blocks, false).t_end;
 	const size_t    bytes = sizeof (float) * (size_t)t_end * h->C;
 	const float*    d_src = src;
 	if (!dev_in) {
@@ -3573,7 +3554,7 @@ phaserot_group_sweep (phaserot_group_t* g, const void* data, int format, uint64_
 			shard_history (data, format, f0, h->L, h->C, hist);
 		}
 		DevGuard guard (h->dev);
-		int      rc = sweep_core (h, shard_job (h->L, (const char*)data + pcm_bytes (format) * (size_t)f0 * h->C, false, format, nf, i > 0 ? hist.data () : nullptr,
+		int      rc = sweep_core (h, shard_job ((const char*)data + pcm_bytes (format) * (size_t)f0 * h->C, false, format, nf, i > 0 ? hist.data () : nullptr,
 		                                        i == 0, lst, ang_start, ang_end, ang_stride, chn), Pass::Fresh);
 		if (rc == PHASEROT_OK) {
 			rc = complete_pending (h); // a shard whose survivor list overflowed is repeated in dense mode before the tables are combined
