@@ -334,6 +334,41 @@ PHASEROT_API int phaserot_overs_device (phaserot_t* h, const float* d_interleave
                                         int ang_start, int ang_end, int ang_stride, int chn,
                                         uint64_t* counts, double* excess);
 
+/* ---- rank table: the N largest samples at every angle --------------------- */
+
+/* The level that N samples of the rotated output reach, at every angle, from one pass: a limiter or clipper after
+ * the rotation has to act on the samples above it, so the angle where it is lowest is the angle to pick for such a
+ * stage (the sweep's peak is rank 1).
+ *   samples    : exactly those phaserot_overs() examines on the same handle and input (first-block rule
+ *                cli:418-419, the zero flush block, chn, the digital or oversample = 2 / 4 true-peak detector);
+ *                grid index 0 is the raw input under the same detector over the frames of the raw-peak rule
+ *                (cli:413-414)
+ *   value      : v_t(a) = fabsf (fmaf (ca, x_d, sa * H)), the sweep's expression; true-peak: the largest of these
+ *                over the sample's detector points (samples are ranked, not points)
+ *   output     : out[n_channels][180 * subsample][n_rank]; out[c][a][k] is the (k+1)-th largest v_t(a) over the
+ *                examined samples, a multiset (equal values of different samples repeat), so each row is
+ *                non-increasing.  Entries beyond the number of examined samples are 0, and so are the rows outside
+ *                the requested angles and channel.  Should the angle loop reach grid index 0 both as angle 0 (raw
+ *                input) and wrapped, the row is whichever of the two has the larger rank-1 value (ties: the raw
+ *                row), so that out[c][a][0] == peak[c][a] of phaserot_sweep() for every (c, a), index 0 included.
+ * For every ceiling T, min (counts[c][a], n_rank) of phaserot_overs() at T equals the number of k with
+ * out[c][a][k] > T.  A sample whose radius sqrt(x_d^2 + H^2) is below the N-th value of every angle cannot change
+ * any row: the running N-th values are the radius of the sweep's exact pruning, and PHASEROT_FLAG_NO_PRUNE (radius
+ * 0) gives the same table.  The table is a sorted multiset: it does not depend on how the work is split, and
+ * repeated calls and the host and device forms return the same floats.  Material on which most samples stay near
+ * the N-th value (pure tones) keeps most samples listed; the launches whose lists or candidate buffers overflow
+ * are re-run in pieces that fit (phaserot_stats_t.dense_repeats counts them).
+ * 1 <= n_rank <= 256.  `data` and `format` as phaserot_sweep_pcm() / PHASEROT_PCM_F32, with the same widening;
+ * host memory.  Synchronous.  The peak table, section tables and apply() stream state are not changed (the host
+ * form completes a pending device sweep first).  PHASEROT_E_STATE for plugin handles; PHASEROT_E_INVAL with a
+ * phaserot_last_error() text for n_rank out of range, NULL out, n_frames == 0, and the angle and channel arguments
+ * phaserot_sweep() rejects. */
+PHASEROT_API int phaserot_nth_peaks (phaserot_t* h, const void* data, int format, uint64_t n_frames, int n_rank,
+                                     int ang_start, int ang_end, int ang_stride, int chn, float* out);
+/* The same over audio resident in device memory (interleaved float32, n_frames * n_channels). */
+PHASEROT_API int phaserot_nth_peaks_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, int n_rank,
+                                            int ang_start, int ang_end, int ang_stride, int chn, float* out);
+
 /* ---- several GPUs in one process ---------------------------------------- */
 
 /* A group of handles, one per device, that analyses ONE stream: the file is cut

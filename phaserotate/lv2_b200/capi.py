@@ -29,6 +29,7 @@ SYMBOLS = [
     "phaserot_sweep_sections", "phaserot_sweep_sections_device", "phaserot_section_peaks",
     "phaserot_render_sections", "phaserot_render_sections_device",
     "phaserot_loudness", "phaserot_loudness_device", "phaserot_overs", "phaserot_overs_device",
+    "phaserot_nth_peaks", "phaserot_nth_peaks_device",
     "phaserot_group_create", "phaserot_group_destroy", "phaserot_group_size", "phaserot_group_handle", "phaserot_group_sweep",
     "phaserot_group_peaks", "phaserot_group_reset", "phaserot_pending_table", "phaserot_set_profiling", "phaserot_get_kernel_times",
     "phaserot_sync", "phaserot_get_stats", "phaserot_reset_stats",
@@ -115,6 +116,8 @@ def load():
     lib.phaserot_loudness_device.argtypes = [vp, vp, C.c_uint64, C.c_double, vp, vp, C.c_int, vp]
     lib.phaserot_overs.argtypes = [vp, vp, C.c_int, C.c_uint64, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]
     lib.phaserot_overs_device.argtypes = [vp, vp, C.c_uint64, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]
+    lib.phaserot_nth_peaks.argtypes = [vp, vp, C.c_int, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]
+    lib.phaserot_nth_peaks_device.argtypes = [vp, vp, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]
     lib.phaserot_group_create.argtypes = [C.POINTER(vp), C.POINTER(Cfg), vp, C.c_int]
     lib.phaserot_group_destroy.argtypes = [vp]
     lib.phaserot_group_destroy.restype = None
@@ -406,6 +409,29 @@ class Phaserot:
         self._ck(self._lib.phaserot_overs_device(self._h, C.c_void_p(ptr), n_frames, float(ceiling), ang_start, ang_end, ang_stride, chn, _ptr(counts),
                                                  _ptr(excess)), "phaserot_overs_device")
         return counts, excess
+
+    # -- rank table ------------------------------------------------------------
+    def nth_peaks(self, x, n_rank, ang_start=0, ang_end=None, ang_stride=1, chn=-1):
+        """The n_rank largest values of the rotated output at every angle: float32 [C][MS][n_rank], each row non-increasing.
+        x: host array [frames, channels] of float32, int16 or int32 (PCM_S32), or packed 24-bit uint8 bytes."""
+        if ang_end is None:
+            ang_end = self.maxsample
+        x = np.ascontiguousarray(x)
+        fmt = {np.dtype(np.float32): PCM_F32, np.dtype(np.int16): PCM_S16, np.dtype(np.int32): PCM_S32, np.dtype(np.uint8): PCM_S24}[x.dtype]
+        n = x.size // self.n_channels // (3 if fmt == PCM_S24 else 1)
+        out = np.zeros((self.n_channels, self.maxsample, max(int(n_rank), 1)), np.float32)
+        self._ck(self._lib.phaserot_nth_peaks(self._h, _ptr(x), fmt, n, int(n_rank), ang_start, ang_end, ang_stride, chn, _ptr(out)),
+                 "phaserot_nth_peaks")
+        return out
+
+    def nth_peaks_device(self, ptr, n_frames, n_rank, ang_start=0, ang_end=None, ang_stride=1, chn=-1):
+        """The same over interleaved float32 audio in device memory."""
+        if ang_end is None:
+            ang_end = self.maxsample
+        out = np.zeros((self.n_channels, self.maxsample, max(int(n_rank), 1)), np.float32)
+        self._ck(self._lib.phaserot_nth_peaks_device(self._h, C.c_void_p(ptr), n_frames, int(n_rank), ang_start, ang_end, ang_stride, chn, _ptr(out)),
+                 "phaserot_nth_peaks_device")
+        return out
 
     # -- CLI render --------------------------------------------------------
     def apply(self, buf, angles):

@@ -13,6 +13,9 @@
 //    fir_stream_kernel     small-call plugin path: direct-form FIR + rotate, history in a device ring
 //    truepeak_kernel       oversampled true-peak front end of the sweep
 //    overs_kernel          overs table: per-angle count and excess of survivors above a ceiling
+//    nth_kernel            rank table: survivors above an angle's running N-th value -> its candidates
+//    nth_merge_kernel      rank table: sorted top-N row of an angle merged with its candidates
+//
 //
 // Data layout.  A channel's samples x[0..F) are viewed as complex numbers
 // z[n] = x[2n] + i x[2n+1] ("plane", float2, with a zero front pad).  The
@@ -1742,6 +1745,21 @@ __global__ void __launch_bounds__ (256, 4) truepeak_kernel (const TpParams p)
 // (cli:413-414) over frames [0, f_end) - |x[f]| for the digital peak; for os = 2 / 4 the largest of |x[f]|
 // and its interpolated points, formed with the fmaf chain of tp_interp, i.e. the very values truepeak_kernel
 // takes the raw peak of.  Over, count and excess as in overs_kernel.  grid = (frame blocks, channels).
+__device__ __forceinline__ float raw_detector (const float* __restrict__ inter, long long n_frames, int C, int c, long long f, int os)
+{
+	float v = f < n_frames ? fabsf (__ldg (inter + f * C + c)) : 0.f;
+	if (os > 1) {
+		float s[16];
+#pragma unroll
+		for (int k = 0; k < 16; ++k) { // s[12 - k] = x[f - k]
+			const long long g = f + k - 12;
+			s[k]              = (k <= 12 && g >= 0 && g < n_frames) ? __ldg (inter + g * C + c) : 0.f;
+		}
+		v = fmaxf (v, fmaxf (fabsf (tp_interp<0> (s, 0)), fabsf (tp_interp<2> (s, 0))));
+		if (os == 4) v = fmaxf (v, fmaxf (fabsf (tp_interp<1> (s, 0)), fabsf (tp_interp<3> (s, 0))));
+	}
+	return v;
+}
 __global__ void __launch_bounds__ (256) overs_raw_kernel (const float* __restrict__ inter, long long n_frames, int C, int chan0, long long f_end, int os,
                                                            float T, unsigned long long* __restrict__ n_over, unsigned long long* __restrict__ excess)
 {
@@ -1749,17 +1767,7 @@ __global__ void __launch_bounds__ (256) overs_raw_kernel (const float* __restric
 	unsigned           cnt = 0;
 	unsigned long long exc = 0;
 	for (long long f = (long long)blockIdx.x * blockDim.x + threadIdx.x; f < f_end; f += (long long)gridDim.x * blockDim.x) {
-		float v = f < n_frames ? fabsf (__ldg (inter + f * C + c)) : 0.f;
-		if (os > 1) {
-			float s[16];
-#pragma unroll
-			for (int k = 0; k < 16; ++k) { // s[12 - k] = x[f - k]
-				const long long g = f + k - 12;
-				s[k]              = (k <= 12 && g >= 0 && g < n_frames) ? __ldg (inter + g * C + c) : 0.f;
-			}
-			v = fmaxf (v, fmaxf (fabsf (tp_interp<0> (s, 0)), fabsf (tp_interp<2> (s, 0))));
-			if (os == 4) v = fmaxf (v, fmaxf (fabsf (tp_interp<1> (s, 0)), fabsf (tp_interp<3> (s, 0))));
-		}
+		const float v = raw_detector (inter, n_frames, C, c, f, os);
 		if (v > T) {
 			++cnt;
 			exc += (unsigned long long)(((double)v - (double)T) * 4294967296.0);
@@ -1772,6 +1780,256 @@ __global__ void __launch_bounds__ (256) overs_raw_kernel (const float* __restric
 	if ((threadIdx.x & 31) == 0 && cnt) {
 		atomicAdd (n_over + c, (unsigned long long)cnt);
 		atomicAdd (excess + c, exc);
+	}
+}
+
+// ---------------------------------------------------------------------------
+// Rank table (phaserot_nth_peaks): the N largest values of every angle.  Slot (c, a) of a channel's A1 = A + 1
+// slots (the swept angles, then grid index 0 from the raw input) has a row of N floats, non-increasing, zero
+// where fewer samples were merged, a bucket of K candidate floats with its counter, and kth[c][a]: the float
+// bits of the value a sample has to exceed to change the row.
+// ---------------------------------------------------------------------------
+
+// The overs_kernel layout over the records [rec0, rec0 + rec_max) of a survivor list: each lane appends the
+// records whose value v (as in overs_kernel) exceeds kth of its angle to that angle's bucket.  A bucket that runs
+// over sets cand_ovf[c]; nth_merge_kernel then drops all of the channel's candidates.  A channel whose count
+// exceeds skip_above is skipped (its list overflowed; the launch is re-run in pieces).
+template <int R, int G>
+__global__ void __launch_bounds__ (256) nth_kernel (const float2* __restrict__ list, long long list_stride, const unsigned* __restrict__ count,
+                                                     unsigned cap, unsigned skip_above, unsigned rec0, unsigned rec_max, int chan0,
+                                                     const float2* __restrict__ cs, int A, int A1, const unsigned* __restrict__ kth,
+                                                     float* __restrict__ cand, unsigned* __restrict__ cand_cnt, unsigned K, unsigned* __restrict__ cand_ovf,
+                                                     unsigned long long* __restrict__ n_eval)
+{
+	__shared__ __align__ (16) float2 tile[kOversTile * G];
+	const int c = chan0 + blockIdx.z;
+	if (count[c] > skip_above) return;
+	const unsigned n_all = min (count[c], cap) / G; // records on the list (a bootstrap list may have dropped some)
+	if (n_all <= rec0) return;
+	const unsigned n        = min (n_all - rec0, rec_max);
+	const unsigned tile_rec = min ((unsigned)kOversTile, max (32u, (n + gridDim.x - 1) / gridDim.x));
+	if (blockIdx.x * tile_rec >= n) return;
+	const float2* pts = list + (long long)c * list_stride + (long long)rec0 * G;
+	const int     a0  = blockIdx.y * (blockDim.x * R) + threadIdx.x;
+
+	float ca[R], sa[R], kt[R];
+#pragma unroll
+	for (int r = 0; r < R; ++r) {
+		const int    a = a0 + r * blockDim.x;
+		const float2 v = a < A ? cs[a] : make_float2 (0.f, 0.f);
+		ca[r]          = v.x;
+		sa[r]          = v.y;
+		kt[r]          = a < A ? __uint_as_float (kth[(long long)c * A1 + a]) : __int_as_float (0x7f800000);
+	}
+
+	for (unsigned base = blockIdx.x * tile_rec; base < n; base += gridDim.x * tile_rec) {
+		const unsigned nr = min (tile_rec, n - base);
+		// a bucket of the channel ran over (an empty row takes every record): the rest would be dropped anyway
+		if (__syncthreads_or (threadIdx.x == 0 && *(volatile const unsigned*)(cand_ovf + c))) break;
+		for (unsigned i = threadIdx.x; i < nr * G; i += blockDim.x) tile[i] = pts[(size_t)base * G + i];
+		__syncthreads ();
+#pragma unroll 2
+		for (unsigned i = 0; i < nr; ++i) {
+			float2 q[G];
+#pragma unroll
+			for (int g = 0; g < G; ++g) q[g] = tile[i * G + g]; // broadcast
+#pragma unroll
+			for (int r = 0; r < R; ++r) {
+				float v = 0.f;
+#pragma unroll
+				for (int g = 0; g < G; ++g) v = fmaxf (v, fabsf (fmaf (ca[r], q[g].x, sa[r] * q[g].y)));
+				if (v > kt[r]) {
+					const long long slot = (long long)c * A1 + a0 + r * (int)blockDim.x;
+					const unsigned  pos  = atomicAdd (cand_cnt + slot, 1u);
+					if (pos < K) cand[slot * K + pos] = v;
+					else cand_ovf[c] = 1u;
+				}
+			}
+		}
+		if (n_eval && blockIdx.y == 0 && threadIdx.x == 0) atomicAdd (n_eval, (unsigned long long)nr * G);
+	}
+}
+
+// 512 floats in shared memory into non-increasing order (bitonic network, 256 threads)
+constexpr int kNthSort = 512;
+__device__ __forceinline__ void nth_sort512 (float* s, int tid)
+{
+	for (int k = 2; k <= kNthSort; k <<= 1) {
+		for (int j = k >> 1; j > 0; j >>= 1) {
+			const int   i = 2 * tid - (tid & (j - 1)), l = i + j;
+			const float x = s[i], y = s[l];
+			if ((i & k) == 0 ? x < y : x > y) {
+				s[i] = y;
+				s[l] = x;
+			}
+			__syncthreads ();
+		}
+	}
+}
+
+// One CTA of 256 threads per (slot a0 + blockIdx.x, channel) with candidates: those above the row's N-th value
+// are compacted behind the row in shared memory and sorted in with it whenever another 256 might not fit (N <=
+// 256); then kth = bits of the N-th value.  lower_bound: the candidates were a subset of the samples (bootstrap
+// wave), whose N-th value bounds the final one from below only - kth is the float below it, so that a sample
+// equal to it still enters the row (the caller clears the rows).  A channel with cand_ovf set keeps its rows and
+// drops its candidates.  The bucket counters are cleared.
+__global__ void __launch_bounds__ (256) nth_merge_kernel (float* __restrict__ rows, unsigned* __restrict__ kth, const float* __restrict__ cand,
+                                                           unsigned* __restrict__ cand_cnt, unsigned K, int A1, int a0, int N, int chan0,
+                                                           const unsigned* __restrict__ cand_ovf, int lower_bound)
+{
+	__shared__ float    s[kNthSort];
+	__shared__ unsigned wsum[8];
+	const int       c    = chan0 + blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	const long long slot = (long long)c * A1 + a0 + blockIdx.x;
+	const unsigned  n    = cand_cnt[slot];
+	if (n == 0) return;
+	if (cand_ovf[c]) {
+		if (tid == 0) cand_cnt[slot] = 0; // (a thread that reads the cleared counter returns as well)
+		return;
+	}
+	float* row = rows + slot * N;
+	for (int j = tid; j < N; j += blockDim.x) s[j] = row[j];
+	const float* cd   = cand + slot * K;
+	int          fill = N;
+	__syncthreads ();
+	for (unsigned b = 0; b < n; b += blockDim.x) {
+		const float    v   = b + tid < n ? cd[b + tid] : 0.f;
+		const bool     in  = v > s[N - 1];
+		const unsigned bal = __ballot_sync (0xffffffffu, in);
+		if (lane == 0) wsum[warp] = __popc (bal);
+		__syncthreads ();
+		int off = fill, tot = 0;
+		for (int w = 0; w < 8; ++w) {
+			off += w < warp ? (int)wsum[w] : 0;
+			tot += (int)wsum[w];
+		}
+		if (in) s[off + __popc (bal & lanemask_lt ())] = v;
+		fill += tot;
+		__syncthreads ();
+		if (fill > N && (fill > kNthSort - 256 || b + blockDim.x >= n)) {
+			for (int j = fill + tid; j < kNthSort; j += blockDim.x) s[j] = 0.f;
+			__syncthreads ();
+			nth_sort512 (s, tid);
+			fill = N;
+		}
+	}
+	for (int j = tid; j < N; j += blockDim.x) row[j] = s[j];
+	if (tid == 0) {
+		const unsigned nb = __float_as_uint (s[N - 1]);
+		kth[slot]         = lower_bound ? (nb ? nb - 1 : 0u) : max (kth[slot], nb);
+		cand_cnt[slot]    = 0;
+	}
+}
+
+// Grid index 0 of the rank table: the N largest raw_detector values of frames [0, f_end) (overs_raw_kernel's),
+// selected exactly by radix on their bits (non-negative floats order as unsigned integers).  kth of slot A first
+// takes a lower bound from block maxima (nth_raw_max_kernel); only the values above it take part.  Three digit
+// passes, bits [shift, hi) of 30..20, 19..10, 9..0, each a histogram of the values whose higher bits match the
+// prefix so far (nth_raw_hist_kernel) and the choice of the digit (nth_raw_pick_kernel), give the bits of the N-th
+// value and how many values lie above it; nth_raw_collect_kernel puts those into the bucket of slot A, the last
+// pick fills it up to N with the N-th value.  A channel with fewer than N values takes 0 for the missing ones.
+// sel[c] = { prefix, rank still to place, values above the prefix, bucket fill }.  grid = (frame blocks, channels).
+constexpr int kNthDigits = 2048;
+
+// maxima of the frames [b f_end / M, (b + 1) f_end / M), b < M = gridDim.x, into the bucket of slot A: they are
+// values of M distinct samples, so their N-th largest bounds the N-th value from below (nth_merge_kernel with
+// lower_bound; M >= N)
+__global__ void __launch_bounds__ (256) nth_raw_max_kernel (const float* __restrict__ inter, long long n_frames, int C, int chan0, long long f_end, int os,
+                                                             int A1, int A, float* __restrict__ cand, unsigned* __restrict__ cand_cnt, unsigned K)
+{
+	__shared__ float red[8];
+	const int       c  = chan0 + blockIdx.y;
+	const long long f0 = f_end * blockIdx.x / gridDim.x, f1 = f_end * (blockIdx.x + 1) / gridDim.x;
+	float           m  = 0.f;
+	for (long long f = f0 + threadIdx.x; f < f1; f += blockDim.x) m = fmaxf (m, raw_detector (inter, n_frames, C, c, f, os));
+	for (int o = 16; o; o >>= 1) m = fmaxf (m, __shfl_xor_sync (0xffffffffu, m, o));
+	if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
+	__syncthreads ();
+	if (threadIdx.x == 0) {
+		for (int w = 1; w < 8; ++w) m = fmaxf (m, red[w]);
+		const long long slot           = (long long)c * A1 + A;
+		cand[slot * K + blockIdx.x]    = m;
+		if (blockIdx.x == 0) cand_cnt[slot] = gridDim.x;
+	}
+}
+
+__global__ void __launch_bounds__ (256) nth_raw_hist_kernel (const float* __restrict__ inter, long long n_frames, int C, int chan0, long long f_end, int os,
+                                                              int shift, int hi, const unsigned* __restrict__ sel, const unsigned* __restrict__ kth, int A1,
+                                                              int A, unsigned* __restrict__ hist)
+{
+	__shared__ unsigned hs[kNthDigits];
+	for (int i = threadIdx.x; i < kNthDigits; i += blockDim.x) hs[i] = 0;
+	__syncthreads ();
+	const int      c      = chan0 + blockIdx.y;
+	const unsigned prefix = sel[4 * c] >> hi, mask = (1u << (hi - shift)) - 1u, lb = kth[(long long)c * A1 + A];
+	for (long long f = (long long)blockIdx.x * blockDim.x + threadIdx.x; f < f_end; f += (long long)gridDim.x * blockDim.x) {
+		const unsigned u = __float_as_uint (raw_detector (inter, n_frames, C, c, f, os));
+		if (u > lb && (u >> hi) == prefix) atomicAdd (hs + ((u >> shift) & mask), 1u);
+	}
+	__syncthreads ();
+	for (int i = threadIdx.x; i < kNthDigits; i += blockDim.x) {
+		if (hs[i]) atomicAdd (hist + (long long)c * kNthDigits + i, hs[i]);
+	}
+}
+
+// one CTA of 256 threads per channel: the largest digit d with fewer than `rank` values above it (0 when the
+// channel has fewer values than that); clears the histogram.  last: the bucket of slot A is filled up to N.
+__global__ void __launch_bounds__ (256) nth_raw_pick_kernel (unsigned* __restrict__ sel, unsigned* __restrict__ hist, int chan0, int shift, int last, int N,
+                                                              int A1, int A, float* __restrict__ cand, unsigned* __restrict__ cand_cnt, unsigned K)
+{
+	__shared__ unsigned wt[8], pick[2];
+	const int c = chan0 + blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+	unsigned* hc   = hist + (long long)c * kNthDigits;
+	const unsigned prefix0 = sel[4 * c], rank = sel[4 * c + 1], above0 = sel[4 * c + 2];
+	// thread t owns digits 2047 - 8 t - j, j < 8: thread 0 the largest
+	unsigned b[8], sum = 0;
+#pragma unroll
+	for (int j = 0; j < 8; ++j) {
+		b[j] = hc[kNthDigits - 1 - 8 * tid - j];
+		sum += b[j];
+		hc[kNthDigits - 1 - 8 * tid - j] = 0;
+	}
+	unsigned inc = sum;
+	for (int o = 1; o < 32; o <<= 1) {
+		const unsigned t = __shfl_up_sync (0xffffffffu, inc, o);
+		if (lane >= o) inc += t;
+	}
+	if (lane == 31) wt[warp] = inc;
+	__syncthreads ();
+	unsigned above = inc - sum; // values in the digits above this thread's
+	for (int w = 0; w < warp; ++w) above += wt[w];
+#pragma unroll
+	for (int j = 0; j < 8; ++j) {
+		const int d = kNthDigits - 1 - 8 * tid - j;
+		if (above < rank && (above + b[j] >= rank || d == 0)) {
+			pick[0] = (unsigned)d;
+			pick[1] = above;
+		}
+		above += b[j];
+	}
+	__syncthreads ();
+	const unsigned prefix = prefix0 | (pick[0] << shift), n_above = above0 + pick[1];
+	if (tid == 0) {
+		sel[4 * c]     = prefix;
+		sel[4 * c + 1] = rank - pick[1];
+		sel[4 * c + 2] = n_above;
+	}
+	if (last) {
+		float* bucket = cand + ((long long)c * A1 + A) * K;
+		for (int j = (int)n_above + tid; j < N; j += blockDim.x) bucket[j] = __uint_as_float (prefix);
+		if (tid == 0) cand_cnt[(long long)c * A1 + A] = (unsigned)N;
+	}
+}
+
+__global__ void __launch_bounds__ (256) nth_raw_collect_kernel (const float* __restrict__ inter, long long n_frames, int C, int chan0, long long f_end, int os,
+                                                                 unsigned* __restrict__ sel, int A1, int A, float* __restrict__ cand, unsigned K)
+{
+	const int      c      = chan0 + blockIdx.y;
+	const unsigned vn     = sel[4 * c];
+	float*         bucket = cand + ((long long)c * A1 + A) * K;
+	for (long long f = (long long)blockIdx.x * blockDim.x + threadIdx.x; f < f_end; f += (long long)gridDim.x * blockDim.x) {
+		const float v = raw_detector (inter, n_frames, C, c, f, os);
+		if (__float_as_uint (v) > vn) bucket[atomicAdd (sel + 4 * c + 3, 1u)] = v; // fewer than N values
 	}
 }
 

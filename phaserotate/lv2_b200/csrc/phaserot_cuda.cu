@@ -269,8 +269,11 @@ struct phaserot {
 	DevBuf d_kx, d_lH, d_lwork, d_lset;
 
 	// overs table (phaserot_overs): survivor list | true-peak staging of the Hilbert branch | tables, angle table,
-	// radii and the list counters of every launch; its own buffers, so that a pending device sweep is not disturbed
+	// radii and the list counters of every launch; its own buffers, so that a pending device sweep is not disturbed.
+	// The rank table (phaserot_nth_peaks) shares the list and the staging.
 	DevBuf d_ovl, d_ovH, d_ovw;
+	// rank table: rows, thresholds, counters, radix selection state | candidate buckets
+	DevBuf d_nthw, d_nthc;
 
 	// pending (asynchronous) sweep result
 	bool             pending = false;
@@ -2275,6 +2278,293 @@ overs_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t n_f
 	return overs_core (h, d_x, (long long)n_frames, ceiling, ang_start, ang_end, ang_stride, chn, counts, excess);
 }
 
+/*
+ * phaserot_nth_peaks over F frames of interleaved float32 audio on the device.  kth[c][a] starts at 0 and
+ * follows the N-th value of the row; threshold_kernel turns it into the filter radius (min_a kth)^2 (1 - 1e-5)
+ * of the FFT pass (a sample below it is at or below kth at every angle, and so cannot change a row), and
+ * nth_kernel / nth_merge_kernel turn each launch's survivors into candidates and merge them.  Launches and lists
+ * as a device-resident sweep, including its bootstrap wave, whose rows are a subset's: they only seed kth from
+ * below and are cleared.  After every launch the host reads the list counters and bucket flags.  Every sample
+ * enters a row exactly once: a channel whose buckets ran over had all of the launch's candidates dropped and
+ * takes its list again in chunks of K records, which one bucket holds in full; a channel whose list overflowed
+ * was skipped by nth_kernel, and its segments are re-run at the end in pieces the list holds.  Grid index 0:
+ * exact radix selection over the raw input values above a lower bound from block maxima.  Synchronous.  out: host
+ * [C][MS][N].
+ */
+constexpr int kMaxRank = 256; // largest n_rank of phaserot_nth_peaks: a row and 256 candidates fill one sort of kNthSort
+
+int
+nth_core (phaserot* h, const float* d_x, long long F, int N, int ang_start, int ang_end, int ang_stride, int chn, float* out)
+{
+	std::vector<int> idx;
+	bool             raw = false;
+	int              rc  = angle_schedule (h, ang_start, ang_end, ang_stride, idx, raw);
+	if (rc) return rc;
+	const int        C        = h->C;
+	const int        A        = (int)idx.size ();
+	const int        A1       = A + 1; // slot A: grid index 0 from the raw input
+	const int        c0       = chn < 0 ? 0 : chn;
+	const int        c1       = chn < 0 ? C : chn + 1;
+	const int        nchan    = c1 - c0;
+	const int        OS       = h->OS;
+	const int        G        = OS > 1 ? OS + 1 : 1;          // points per record
+	const StreamGeom g        = stream_geom (h, F, 1, true); // like phaserot_sweep
+	const long long  nseg     = g.nseg;
+	const bool       no_prune = (h->cfg.flags & PHASEROT_FLAG_NO_PRUNE) != 0;
+	const ListPlan   lp       = plan_lists (h, nchan, nseg, true, no_prune);
+	// candidate floats per slot: 8 K, fewer on grids so fine or wide that the buckets would pass 512 MB
+	const unsigned K = (unsigned)std::min<long long> (8192, std::max<long long> (kNthSort, (128LL << 20) / ((long long)C * A1)));
+
+	// work area: u64 evaluated | (ca, sa) [A] | rows [C][A1][N] | kth [C][A1] | bucket counters [C][A1] |
+	// histograms [C][kNthDigits] | selection state [C][4] | list counters [C] | bucket flags [C] | thr2 [C] |
+	// raw peaks [C] (unused) | r2max [C] | list overflow word (unused)
+	const size_t n_slot = (size_t)C * A1;
+	const size_t bytes  = sizeof (unsigned long long) + sizeof (float2) * (size_t)std::max (A, 1) + sizeof (float) * n_slot * N +
+	                     sizeof (unsigned) * (2 * n_slot + (size_t)C * (kNthDigits + 4 + 5) + 1);
+	rc = h->d_nthw.ensure (bytes);
+	if (rc) return rc;
+	rc = h->d_nthc.ensure (sizeof (float) * n_slot * K);
+	if (rc) return rc;
+	unsigned long long* d_eval  = (unsigned long long*)h->d_nthw.p;
+	float2*             d_cs    = (float2*)(d_eval + 1);
+	float*              d_rows  = (float*)(d_cs + std::max (A, 1));
+	unsigned*           d_kth   = (unsigned*)(d_rows + n_slot * N);
+	unsigned*           d_ccnt  = d_kth + n_slot;
+	unsigned*           d_hist  = d_ccnt + n_slot;
+	unsigned*           d_sel   = d_hist + (size_t)C * kNthDigits;
+	unsigned*           d_lcnt  = d_sel + 4 * (size_t)C;
+	unsigned*           d_covf  = d_lcnt + C;
+	float*              d_thr2  = (float*)(d_covf + C);
+	unsigned*           d_rawp  = (unsigned*)(d_thr2 + C);
+	unsigned*           d_r2max = d_rawp + C;
+	unsigned*           d_lovf  = d_r2max + C;
+	float*              d_cand  = (float*)h->d_nthc.p;
+	CK (cudaMemsetAsync (h->d_nthw.p, 0, bytes, h->stream));
+	{
+		std::vector<float2> cs ((size_t)A);
+		for (int k = 0; k < A; ++k) cs[(size_t)k] = make_float2 (h->lut_c[(size_t)idx[(size_t)k]], h->lut_s[(size_t)idx[(size_t)k]]);
+		std::vector<unsigned> sel ((size_t)4 * C, 0u); // the raw selection looks for rank N
+		for (int c = 0; c < C; ++c) sel[(size_t)4 * c + 1] = (unsigned)N;
+		CK (cudaMemcpyAsync (d_cs, cs.data (), sizeof (float2) * cs.size (), cudaMemcpyHostToDevice, h->stream));
+		CK (cudaMemcpyAsync (d_sel, sel.data (), sizeof (unsigned) * sel.size (), cudaMemcpyHostToDevice, h->stream));
+	}
+
+	if (A > 0) {
+		rc = h->d_ovl.ensure (sizeof (float2) * (size_t)lp.cap * C);
+		if (rc) return rc;
+		const long long tp_stride = (kTpCarry + lp.segs_cap * 2 * h->V + 3) & ~3LL;
+		if (OS > 1) {
+			rc = h->d_ovH.ensure (sizeof (float) * (size_t)tp_stride * C);
+			if (rc) return rc;
+		}
+		float*         H   = (float*)h->d_ovH.p;
+		const float2*  lst = (const float2*)h->d_ovl.p;
+		const unsigned cap = (unsigned)lp.cap;
+		ConvParams     p   = analysis_params (h, d_x, nullptr, F, g, c0, nchan, (float2*)h->d_ovl.p, lp.cap, d_lcnt, d_lovf, d_thr2, d_rawp);
+		p.thr_mode         = -1;
+		TpParams tp {};
+		if (OS > 1) tp = tp_params (h, p, g.t_end, H, tp_stride);
+
+		// records [r0, r0 + n_rec) of the lists of channels [ch0, ch0 + nch) (list capacity lcap) -> candidates -> rows
+		auto candidates = [&] (int ch0, int nch, unsigned lcap, unsigned skip_above, unsigned r0, unsigned n_rec, bool boot) -> int {
+			{
+				ProfScope ps (h, 1);
+				auto nth = [&] (auto G_) {
+					dispatch_sweep (h, A, nch, [&] (auto R, dim3 grid, int nt) {
+						nth_kernel<decltype (R)::value, decltype (G_)::value><<<grid, nt, 0, h->stream>>> (lst, lp.cap, d_lcnt, lcap, skip_above, r0, n_rec, ch0, d_cs, A, A1,
+						                                                                                    d_kth, d_cand, d_ccnt, K, d_covf, d_eval);
+					});
+				};
+				if (G == 1) nth (std::integral_constant<int, 1> ());
+				else if (G == 3) nth (std::integral_constant<int, 3> ());
+				else nth (std::integral_constant<int, 5> ());
+				CK (cudaGetLastError ());
+			}
+			{
+				ProfScope ps (h, 5);
+				nth_merge_kernel<<<dim3 ((unsigned)A, (unsigned)nch), 256, 0, h->stream>>> (d_rows, d_kth, d_cand, d_ccnt, K, A1, 0, N, ch0, d_covf, boot ? 1 : 0);
+				CK (cudaGetLastError ());
+			}
+			h->stats.kernel_launches += 2;
+			return PHASEROT_OK;
+		};
+
+		// segments s0 + i stride, i < n, of channels [ch0, ch0 + nch): radius, FFT pass, candidates; then on the host
+		// the bucket re-runs, and the channels whose list overflowed (not for the bootstrap, whose list may drop
+		// points) to `overflowed`
+		std::vector<unsigned> st ((size_t)2 * C);
+		auto run_launch = [&] (long long s0, long long stride, long long n, int ch0, int nch, bool boot, std::vector<int>& overflowed) -> int {
+			{
+				ProfScope ps (h, 5);
+				threshold_kernel<<<nch, 256, 0, h->stream>>> (d_kth, A1, A, ch0, d_thr2, d_lcnt, 1, no_prune ? 0 : 1);
+				CK (cudaGetLastError ());
+				++h->stats.kernel_launches;
+			}
+			p.chan0      = ch0;
+			p.nchan      = nch;
+			p.seg0       = s0;
+			p.seg_stride = stride;
+			p.nseg       = n;
+			p.seg_jitter = boot && stride > 1;
+			// the bootstrap wave: any subset of its samples is valid, what does not fit kBootCap points is dropped
+			const unsigned lcap = boot ? (unsigned)std::min<long long> (lp.cap, kBootCap) : cap;
+			int            r;
+			if (OS > 1) {
+				p.r2max = boot ? d_r2max : nullptr;
+				r       = launch_conv<EPI_HILBERT, SRC_INTER> (h, p);
+				if (r) return r;
+				tp.chan0      = ch0;
+				tp.seg0       = s0;
+				tp.seg_stride = stride;
+				tp.seg_jitter = p.seg_jitter;
+				tp.boot_beta  = boot ? kBootBeta : 0.f;
+				tp.r2max      = d_r2max;
+				tp.list_cap   = lcap;
+				{
+					ProfScope ps (h, 6);
+					truepeak_kernel<true><<<dim3 ((unsigned)(n * (tp.V2 / kTpTile)), (unsigned)nch), 256, 0, h->stream>>> (tp);
+					CK (cudaGetLastError ());
+					++h->stats.kernel_launches;
+				}
+				if (stride == 1) {
+					r = launch_tp_carry (h, H, tp_stride, ch0, nch, n * 2 * h->V);
+					if (r) return r;
+				}
+			} else {
+				p.boot_beta = boot ? kBootBeta : 0.f;
+				p.r2max     = d_r2max;
+				p.list_cap  = lcap;
+				r           = launch_conv<EPI_POINTS, SRC_INTER> (h, p);
+				if (r) return r;
+			}
+			const unsigned skip_above = boot ? ~0u : cap;
+			r                         = candidates (ch0, nch, lcap, skip_above, 0, ~0u, boot);
+			if (r) return r;
+			CK (cudaMemcpyAsync (st.data (), d_lcnt, sizeof (unsigned) * 2 * C, cudaMemcpyDeviceToHost, h->stream)); // list counters | bucket flags
+			CK (cudaStreamSynchronize (h->stream));
+			h->stats.d2h_bytes += sizeof (unsigned) * 2 * C;
+			for (int c = ch0; c < ch0 + nch; ++c) {
+				if (st[(size_t)c] > skip_above) {
+					overflowed.push_back (c);
+				} else if (st[(size_t)C + c]) {
+					++h->stats.dense_repeats;
+					CK (cudaMemsetAsync (d_covf + c, 0, sizeof (unsigned), h->stream));
+					const unsigned n_rec = std::min (st[(size_t)c], lcap) / (unsigned)G;
+					for (unsigned r0 = 0; r0 < n_rec; r0 += K) {
+						r = candidates (c, 1, lcap, skip_above, r0, K, boot);
+						if (r) return r;
+					}
+				}
+			}
+			return PHASEROT_OK;
+		};
+
+		std::vector<int> overflowed;
+		const long long  wave = std::max<long long> (1, (h->n_sm + nchan - 1) / nchan); // segments per channel in one wave
+		if (!no_prune && nseg >= 2 * wave) {
+			// the sweep's bootstrap wave: kth from below, then empty rows
+			rc = run_launch (0, nseg / wave, wave, c0, nchan, true, overflowed);
+			if (rc) return rc;
+			CK (cudaMemsetAsync (d_rows, 0, sizeof (float) * n_slot * N, h->stream));
+		}
+		if (OS > 1) {
+			rc = seed_tp_carry (h, p, H, tp_stride, 0, c0, nchan);
+			if (rc) return rc;
+		}
+		std::vector<long long> l_s0, l_n;
+		std::vector<int>       l_k; // launch of each overflowed channel
+		long long              seg_done = 0;
+		for (int n_main = 0; seg_done < nseg; ++n_main) {
+			const long long n = std::min (next_launch_segs (n_main, seg_done, nseg, lp.segs_first, lp.segs_max, true), nseg - seg_done);
+			rc                = run_launch (seg_done, 1, n, c0, nchan, false, overflowed);
+			if (rc) return rc;
+			l_s0.push_back (seg_done);
+			l_n.push_back (n);
+			l_k.resize (overflowed.size (), n_main);
+			seg_done += n;
+		}
+		// overflowed (launch, channel): re-run its segments in pieces that fit the list
+		const long long fit = std::max<long long> (1, lp.cap / lp.ppseg);
+		for (size_t i = 0; i < overflowed.size (); ++i) {
+			const int c = overflowed[i], k = l_k[i];
+			++h->stats.dense_repeats;
+			for (long long s = l_s0[(size_t)k]; s < l_s0[(size_t)k] + l_n[(size_t)k]; s += fit) {
+				if (OS > 1) {
+					rc = seed_tp_carry (h, p, H, tp_stride, s, c, 1);
+					if (rc) return rc;
+				}
+				std::vector<int> none;
+				rc = run_launch (s, 1, std::min (fit, l_s0[(size_t)k] + l_n[(size_t)k] - s), c, 1, false, none);
+				if (rc) return rc;
+			}
+		}
+	}
+
+	// grid index 0: radix selection over the raw input (the interpolator reaches 11 frames past the last one)
+	static_assert (kMaxRank <= kNthSort, "the raw lower bound needs at least N block maxima (K >= kNthSort)");
+	if (raw) {
+		const long long f_end = std::min (F + (OS > 1 ? 11 : 0), g.t_end - h->L / 2);
+		const dim3      grid ((unsigned)std::min<long long> ((f_end + 255) / 256, (long long)h->n_sm * 8), (unsigned)nchan);
+		ProfScope       ps (h, 5);
+		// the lower bound from kNthSort .. 4096 block maxima (at least N), then the rows cleared of them
+		nth_raw_max_kernel<<<dim3 (std::min (K, 4096u), (unsigned)nchan), 256, 0, h->stream>>> (d_x, F, C, c0, f_end, OS, A1, A, d_cand, d_ccnt, K);
+		nth_merge_kernel<<<dim3 (1, (unsigned)nchan), 256, 0, h->stream>>> (d_rows, d_kth, d_cand, d_ccnt, K, A1, A, N, c0, d_covf, 1);
+		CK (cudaMemset2DAsync (d_rows + ((size_t)c0 * A1 + A) * N, sizeof (float) * A1 * N, 0, sizeof (float) * N, (size_t)nchan, h->stream));
+		const int shift[3] = { 20, 10, 0 }, hi[3] = { 31, 20, 10 };
+		for (int k = 0; k < 3; ++k) {
+			nth_raw_hist_kernel<<<grid, 256, 0, h->stream>>> (d_x, F, C, c0, f_end, OS, shift[k], hi[k], d_sel, d_kth, A1, A, d_hist);
+			nth_raw_pick_kernel<<<nchan, 256, 0, h->stream>>> (d_sel, d_hist, c0, shift[k], k == 2, N, A1, A, d_cand, d_ccnt, K);
+		}
+		nth_raw_collect_kernel<<<grid, 256, 0, h->stream>>> (d_x, F, C, c0, f_end, OS, d_sel, A1, A, d_cand, K);
+		nth_merge_kernel<<<dim3 (1, (unsigned)nchan), 256, 0, h->stream>>> (d_rows, d_kth, d_cand, d_ccnt, K, A1, A, N, c0, d_covf, 0);
+		CK (cudaGetLastError ());
+		h->stats.kernel_launches += 10;
+	}
+
+	std::vector<float> rows (n_slot * N);
+	unsigned long long n_eval = 0;
+	CK (cudaMemcpyAsync (rows.data (), d_rows, sizeof (float) * rows.size (), cudaMemcpyDeviceToHost, h->stream));
+	CK (cudaMemcpyAsync (&n_eval, d_eval, sizeof (n_eval), cudaMemcpyDeviceToHost, h->stream));
+	CK (cudaStreamSynchronize (h->stream));
+	prof_resolve (h);
+	h->stats.d2h_bytes += sizeof (float) * rows.size () + sizeof (n_eval);
+	if (A > 0) {
+		h->stats.points_total += g.points (nchan, G);
+		h->stats.points_evaluated += n_eval;
+	}
+
+	const size_t MS = (size_t)h->MS, n = (size_t)N;
+	std::fill (out, out + (size_t)C * MS * n, 0.f);
+	for (int c = c0; c < c1; ++c) {
+		const float* rw = rows.data () + (size_t)c * A1 * n;
+		float*       oc = out + (size_t)c * MS * n;
+		for (int k = 0; k < A; ++k) std::copy (rw + (size_t)k * n, rw + (size_t)(k + 1) * n, oc + (size_t)idx[(size_t)k] * n);
+		// grid index 0: the raw input; should the schedule also wrap onto index 0, the row with the larger rank-1
+		// value (peak[c][0] is the larger of the two peaks; ties: the raw row)
+		if (raw && rw[(size_t)A * n] >= oc[0]) std::copy (rw + (size_t)A * n, rw + (size_t)A1 * n, oc);
+	}
+	return PHASEROT_OK;
+}
+
+int
+nth_entry (phaserot* h, const void* src, bool dev_in, int format, uint64_t n_frames, int n_rank, int ang_start, int ang_end, int ang_stride, int chn,
+           float* out)
+{
+	int rc = check_analysis (h, src, format, n_frames, "phaserot_nth_peaks", [&] () -> const char* {
+		if (n_rank < 1 || n_rank > kMaxRank) return "n_rank is not in 1 .. 256";
+		if (!out) return "NULL out";
+		if (ang_stride < 1) return "ang_stride < 1";
+		if (chn >= h->C) return "chn is not a channel of the handle";
+		return nullptr;
+	});
+	if (rc) return rc;
+	DevGuard     guard (h->dev);
+	const float* d_x;
+	rc = land_input (h, src, dev_in, format, (long long)n_frames, &d_x);
+	if (rc) return rc;
+	return nth_core (h, d_x, (long long)n_frames, n_rank, ang_start, ang_end, ang_stride, chn, out);
+}
+
 // Argument checks of the sweep entry points: data may be null for an empty stream only, and every
 // shard of a stream but the last is a whole number of blocks
 int
@@ -2573,7 +2863,8 @@ phaserot_destroy (phaserot_t* h)
 	if (h->copy_stream) cudaStreamSynchronize (h->copy_stream);
 	for (DevBuf* b : { &h->d_G, &h->d_G1, &h->d_scratch, &h->d_tw, &h->d_g, &h->d_plane, &h->d_out, &h->d_list, &h->d_stage[0], &h->d_stage[1], &h->d_io, &h->d_inter, &h->d_hist, &h->d_small,
 	                   &h->d_cs, &h->d_peaks, &h->d_ramp, &h->d_chancs, &h->d_tpH, &h->d_ring, &h->d_slot, &h->d_sec, &h->d_wide,
-	                   &h->d_sect, &h->d_sect_aux, &h->d_sect_rt, &h->d_kx, &h->d_lH, &h->d_lwork, &h->d_lset, &h->d_ovl, &h->d_ovH, &h->d_ovw }) {
+	                   &h->d_sect, &h->d_sect_aux, &h->d_sect_rt, &h->d_kx, &h->d_lH, &h->d_lwork, &h->d_lset, &h->d_ovl, &h->d_ovH, &h->d_ovw,
+	                   &h->d_nthw, &h->d_nthc }) {
 		b->release ();
 	}
 	for (PinBuf* b : { &h->h_stage[0], &h->h_stage[1], &h->h_res, &h->h_io, &h->h_cs, &h->h_slot }) {
@@ -3097,6 +3388,20 @@ phaserot_overs_device (phaserot_t* h, const float* d_interleaved, uint64_t n_fra
                        uint64_t* counts, double* excess)
 {
 	return overs_entry (h, d_interleaved, true, PHASEROT_PCM_F32, n_frames, ceiling, ang_start, ang_end, ang_stride, chn, counts, excess);
+}
+
+PHASEROT_API int
+phaserot_nth_peaks (phaserot_t* h, const void* data, int format, uint64_t n_frames, int n_rank, int ang_start, int ang_end, int ang_stride, int chn,
+                    float* out)
+{
+	return nth_entry (h, data, false, format, n_frames, n_rank, ang_start, ang_end, ang_stride, chn, out);
+}
+
+PHASEROT_API int
+phaserot_nth_peaks_device (phaserot_t* h, const float* d_interleaved, uint64_t n_frames, int n_rank, int ang_start, int ang_end, int ang_stride, int chn,
+                           float* out)
+{
+	return nth_entry (h, d_interleaved, true, PHASEROT_PCM_F32, n_frames, n_rank, ang_start, ang_end, ang_stride, chn, out);
 }
 
 uint32_t

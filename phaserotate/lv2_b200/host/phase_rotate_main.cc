@@ -66,6 +66,7 @@ struct Options {
 	bool         loudness    = false; // --loudness: BS.1770-4 integrated loudness and PLR of the input and of the output
 	bool         overs       = false; // --overs DBFS: samples above the ceiling at the input, the output angle and the best angle
 	double       overs_db    = 0;
+	int          nth_peak    = 0;     // --nth-peak N: minimise the level of the N-th largest sample instead of the peak (0: off)
 };
 
 // PHASEROT_CLI_TIMING=1: wall-clock breakdown of the process on stderr (file read, CUDA
@@ -179,6 +180,7 @@ parse_options (int argc, char** argv)
 		{ "sections", required_argument, 0, 1004 },
 		{ "loudness", no_argument, 0, 1005 },
 		{ "overs", required_argument, 0, 1006 },
+		{ "nth-peak", required_argument, 0, 1007 },
 		{ 0, 0, 0, 0 },
 	};
 	int c;
@@ -234,6 +236,15 @@ parse_options (int argc, char** argv)
 				}
 				break;
 			}
+			case 1007: {
+				char*      ep = nullptr;
+				const long n  = strtol (optarg, &ep, 10);
+				if (*ep != '\0' || ep == optarg || n < 1 || n > 256) {
+					die ("Error: --nth-peak takes a rank of 1 .. 256.\n");
+				}
+				o.nth_peak = (int)n;
+				break;
+			}
 			default: die ("Error: unrecognized option. See --help for usage information.\n");
 		}
 	}
@@ -245,6 +256,10 @@ parse_options (int argc, char** argv)
 	}
 	if (o.overs && (o.sections > 0 || o.gpus != 1)) {
 		die ("Error: --overs cannot be combined with --sections or --gpus.\n");
+	}
+	if (o.nth_peak && (o.angles_arg || o.sections > 0 || o.gpus != 1 || o.loudness)) {
+		// (--loudness: its PLR lines are defined on the rank-1 peaks)
+		die ("Error: --nth-peak cannot be combined with -a, --sections, --gpus or --loudness.\n");
 	}
 	kSubsample = o.subsample;
 	kMaxSample = 180 * kSubsample;
@@ -717,23 +732,38 @@ main (int argc, char** argv)
 		if (opt.verbose > 1) {
 			fprintf (vfd, "Analyzing using %d process threads, stride = %d\n", C, stride);
 		}
-		// one pass, every grid index (index 0 = raw peak, cli:413-414)
-		if (grp) {
-			check (phaserot_group_sweep (grp, audio, pcm_fmt, F, 0, kMaxSample, 1, -1), "analysis failed");
-		} else if (pcm_fmt) {
-			check (phaserot_sweep_pcm (pr, audio, pcm_fmt, F, 0, kMaxSample, 1, -1), "analysis failed");
-		} else {
-			check (phaserot_sweep (pr, audio, F, 0, kMaxSample, 1, -1), "analysis failed");
-		}
 		PeakTable tab;
 		tab.channels = C;
 		tab.t.resize ((size_t)C * kMaxSample);
-		check (phaserot_peaks (pr, tab.t.data ()), "analysis failed");
+		if (opt.nth_peak) {
+			// --nth-peak N: one pass, the N largest samples at every grid index (index 0 = the input); the search
+			// and the report run on the rank-N levels as they would on the peaks (rank 1 is the peak table)
+			const size_t       N = (size_t)opt.nth_peak;
+			std::vector<float> ranks (tab.t.size () * N, 0.f);
+			if (F > 0) {
+				check (phaserot_nth_peaks (pr, audio, pcm_fmt, F, opt.nth_peak, 0, kMaxSample, 1, -1, ranks.data ()), "analysis failed");
+			}
+			for (size_t i = 0; i < tab.t.size (); ++i) tab.t[i] = ranks[i * N + N - 1];
+		} else {
+			// one pass, every grid index (index 0 = raw peak, cli:413-414)
+			if (grp) {
+				check (phaserot_group_sweep (grp, audio, pcm_fmt, F, 0, kMaxSample, 1, -1), "analysis failed");
+			} else if (pcm_fmt) {
+				check (phaserot_sweep_pcm (pr, audio, pcm_fmt, F, 0, kMaxSample, 1, -1), "analysis failed");
+			} else {
+				check (phaserot_sweep (pr, audio, F, 0, kMaxSample, 1, -1), "analysis failed");
+			}
+			check (phaserot_peaks (pr, tab.t.data ()), "analysis failed");
+		}
 		timer.mark ("analysis (upload + sweep)");
 		res    = find_min_angles (tab, opt, vfd);
 		angles = res.angle;
 		if (!outfile || opt.verbose) { // report (cli:931-947)
-			fprintf (vfd, "# Result -- Minimize digital peak\n");
+			if (opt.nth_peak > 1) {
+				fprintf (vfd, "# Result -- Minimize digital peak, rank %d\n", opt.nth_peak);
+			} else {
+				fprintf (vfd, "# Result -- Minimize digital peak\n");
+			}
 			report_channels (res, vfd);
 		}
 	}
